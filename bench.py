@@ -2,7 +2,7 @@
 """bench.py -- VIGOR pairs/sec of the CCVPE hot path on N B200s (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload W] [--batch B] [--scaling weak|strong]
-                    [--precision bf16|fp32] [--impl ours|reference]
+                    [--precision bf16|fp32] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of `CVM_VIGOR.forward` + pose decode over one batch of synthetic VIGOR-shaped pairs
 (3x320x640 panorama + 3x512x512 aerial, random-init weights).  Workload = BASELINE.json configs[1]: batch 64 bf16 per
@@ -27,6 +27,7 @@ oracle port that the tests pin bit-equal to it) and prints the same line with "i
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import statistics
@@ -111,6 +112,7 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", "-i", str(self.gpu_index), "--query-gpu=" + self.QUERY,
                                           "--format=csv,noheader,nounits", "-lms", "100"],
                                          stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)             # the sampler never outlives a run that stops early
             self.thread = threading.Thread(target=self._pump, daemon=True)
             self.thread.start()
         except Exception:
@@ -293,6 +295,30 @@ def run_reference_arm(args):
 # ---------------------------------------------------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------------------------------------------------
+OUT_NAMES = ["logits", "heatmap", "ori", "scores1", "scores2", "scores3", "scores4", "scores5", "scores6"]
+#: --dump-outputs stores an array of up to this many elements whole and a sample of this many elements of a larger one, so
+#: one step's 9 outputs and 5 pose fields stay well under 64 MB
+DUMP_MAX_ELEMS = 1 << 20
+
+
+def host_outputs(out, pose):
+    """What one step hands its caller -- the 9 forward outputs and the decoded poses (`pose_<field>`) -- as host float32
+    (floating-point tensors) or float64 (integer tensors, exact) arrays.  A larger array becomes the elements at a fixed,
+    seeded set of sorted flat indices, the same set in every run with the same arguments."""
+    import numpy as np
+
+    arrays = dict(zip(OUT_NAMES, out), **{"pose_" + k: v for k, v in pose.items()})
+    host = {}
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        dtype = torch.float32 if t.is_floating_point() and t.dtype != torch.float64 else torch.float64
+        host[name] = t.to(dtype).cpu().numpy()
+    return host
+
+
 def run_ours(args):
     from ccvpe_b200 import cabi, models
     from ccvpe_b200.decoder import OpTimer
@@ -355,7 +381,7 @@ def run_ours(args):
 
     def step_resident():
         out = model(grd_d, sat_d)
-        return model.decode_pose(out[1], out[2])
+        return out, model.decode_pose(out[1], out[2])
 
     copy_stream = torch.cuda.Stream(device=dev)
     # e2e: two preallocated device input slots (no allocator traffic inside the timed region): the H2D copy of step i+1
@@ -454,13 +480,15 @@ def run_ours(args):
             torch.cuda.profiler.start()
         ev0.record()
         for _ in range(args.steps):
-            step_resident()
+            last = step_resident()
         ev1.record()
         if ncu_range:
             torch.cuda.synchronize()
             torch.cuda.profiler.stop()
         barrier()
         sampler.window(w0, time.time())
+        # copied now: in CUDA-graph mode the outputs are the graph's static buffers, which every later forward overwrites
+        dumped = host_outputs(*last) if args.dump_outputs and rank == 0 else None
         launches = cabi.launch_count()
         ms_total = ev0.elapsed_time(ev1)
         if use_graph:
@@ -646,6 +674,11 @@ def run_ours(args):
                     ideal = max(r["flops"] / pt, r["bytes"] / ph)
                     f.write("%-64s %9.4f %10.2f %10.1f %9.3f\n" % (tag, r["ms"] / args.steps, r["flops"] / sec / 1e12,
                                                                    r["bytes"] / sec / 1e9, ideal / sec))
+        if dumped is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if dist is not None:
         dist.destroy_process_group()
 
@@ -670,7 +703,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-cuda-graph", action="store_true", help="launch every kernel eagerly in the timed regions")
     ap.add_argument("--layers", default=None, help="write a per-layer timing table to this file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step computed (rank 0) as DIR/<name>.npy, to compare two builds output "
+                         "for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload == "train" or args.impl == "reference"):
+        ap.error("--dump-outputs covers the inference workloads of --impl ours")
     if args.workload == "train":
         import bench_train
         bench_train.main(args)

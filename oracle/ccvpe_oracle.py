@@ -13,8 +13,8 @@ PARITY PINNING: the reference ships no tests or golden vectors for this path (SU
 oracle is pinned against outputs of the reference itself executed in the authoring container:
 `oracle/make_golden.py` imports the unmodified reference (via `oracle/ref_shim.py`), runs it on seeded
 weights/inputs and commits digests + samples of all nine outputs to `tests/golden/*.npz`;
-`tests/test_oracle_golden.py` checks this file against those fixtures everywhere, and
-`tests/test_oracle_vs_reference.py` checks it against the live reference wherever /root/reference exists.
+`tests/test_oracle_golden.py` checks this file against those fixtures, and its losses against values stored in
+`tests/golden/oracle_losses.npz`.
 
 The op ORDER deliberately mirrors the reference (roll -> window -> norm -> mul -> sum -> cat per orientation)
 so that timing this file on host cores is a fair stand-in for the reference's CPU forward.

@@ -1,6 +1,6 @@
-"""TEST INFRASTRUCTURE -- generates tests/golden/*.npz by running the UNMODIFIED reference in this container.
+"""TEST INFRASTRUCTURE -- generates the model fixtures tests/golden/<config>.npz by running the UNMODIFIED reference.
 
-    python oracle/make_golden.py            # needs /root/reference (not present on the GPU box)
+    CCVPE_REFERENCE_ROOT=<checkout of tudelft-iv/CCVPE> python oracle/make_golden.py
 
 For every configuration of BASELINE.json (class x ground shape x ori prior) the reference model is built
 via `oracle/ref_shim.py`, its weights are overwritten by `ccvpe_b200.synthetic.fill_deterministic(seed)`, it is

@@ -1,10 +1,8 @@
-"""TEST INFRASTRUCTURE ONLY -- imports the unmodified reference from /root/reference.
+"""TEST INFRASTRUCTURE ONLY -- imports an unmodified checkout of the reference from $CCVPE_REFERENCE_ROOT.
 
-This module exists solely so that `oracle/make_golden.py` and the container-side
-`tests/test_oracle_vs_reference.py` can execute the real reference (tudelft-iv/CCVPE,
-GPL-3, read-only at /root/reference) to pin the oracle restatement in
-`oracle/ccvpe_oracle.py`.  `/root/reference` does not exist on the GPU box, so nothing that
-runs there (`-m gpu` tests, smoke(), bench.py) may import this file.
+This module exists solely so that `oracle/make_golden.py` can execute the real reference (tudelft-iv/CCVPE, GPL-3,
+not part of this repository) to pin the oracle restatement in `oracle/ccvpe_oracle.py`.  The tests, smoke() and
+bench.py never need the reference checkout.
 
 Two shims, no edits to the reference (SURVEY.md section 8(c)):
   * models.py:8-9 import IPython / matplotlib which are not installed -> empty stub modules.
@@ -14,11 +12,11 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("CCVPE_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("CCVPE_REFERENCE_ROOT", "")
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_ROOT, "models.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(REFERENCE_ROOT, "models.py"))
 
 
 def load_reference_models():
