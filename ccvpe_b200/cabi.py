@@ -25,7 +25,7 @@ EXPORTED_SYMBOLS = (
     "ccvpe_pose_scratch_bytes", "ccvpe_pose_decode", "ccvpe_bias_silu_nhwc", "ccvpe_dwconv_bias_silu_nhwc",
     "ccvpe_pointwise_silu_nhwc", "ccvpe_stem_conv_silu_nhwc", "ccvpe_se_gate_scale", "ccvpe_mbconv_project_nhwc",
     "ccvpe_wrap_columns_nhwc",
-    "ccvpe_ingest_u8", "ccvpe_stem_conv_silu_u8_nhwc",
+    "ccvpe_ingest_u8", "ccvpe_resize_u8", "ccvpe_stem_conv_silu_u8_nhwc",
     # training step (config 5)
     "ccvpe_wgrad_workspace_elems", "ccvpe_wgrad", "ccvpe_wgrad_plan", "ccvpe_colsum_workspace_elems", "ccvpe_colsum",
     "ccvpe_relu_bwd", "ccvpe_scale_rows", "ccvpe_planar_to_cl", "ccvpe_cl_to_planar", "ccvpe_ori_normalize_bwd",
@@ -153,6 +153,9 @@ def load() -> C.CDLL:
     lib.ccvpe_ingest_u8.restype = C.c_int
     lib.ccvpe_ingest_u8.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                     C.POINTER(C.c_float), C.POINTER(C.c_float), C.c_void_p, C.c_void_p]
+    lib.ccvpe_resize_u8.restype = C.c_int
+    lib.ccvpe_resize_u8.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                    C.c_void_p]
     lib.ccvpe_wgrad_workspace_elems.restype = C.c_int64
     lib.ccvpe_wgrad_workspace_elems.argtypes = [C.POINTER(WgradDesc)]
     lib.ccvpe_wgrad.restype = C.c_int
@@ -713,3 +716,22 @@ def ingest_u8(img: torch.Tensor, out: torch.Tensor, shift: Optional[torch.Tensor
     s = (C.c_float * 3)(*[float(v) for v in std])
     _check(load().ccvpe_ingest_u8(_ptr(img), 1 if nhwc else 0, B, H, W, out.shape[3], _ptr(shift), m, s, _ptr(out), _stream()),
            "ccvpe_ingest_u8")
+
+
+def resize_u8(img: torch.Tensor, out: torch.Tensor):
+    """img: uint8 [B,3,H,W] (NCHW) or [B,H,W,3] (NHWC), contiguous; out: uint8 [B,3,h,w] contiguous.  Writes Pillow's
+    bilinear resize of each image to out (bit-identical to transforms.Resize((h, w)) on the image as a PIL image)."""
+    if img.dtype != torch.uint8 or not img.is_contiguous() or img.dim() != 4:
+        raise CcvpeError("resize_u8: img must be a contiguous uint8 [B,3,H,W] or [B,H,W,3] tensor")
+    nhwc = img.shape[1] != 3
+    if nhwc and img.shape[3] != 3:
+        raise CcvpeError("resize_u8: neither dim 1 nor dim 3 of img %s has 3 channels" % (tuple(img.shape),))
+    B = img.shape[0]
+    H, W = (img.shape[1], img.shape[2]) if nhwc else (img.shape[2], img.shape[3])
+    if out.dtype != torch.uint8 or not out.is_contiguous() or out.dim() != 4 or tuple(out.shape[:2]) != (B, 3):
+        raise CcvpeError("resize_u8: out must be a contiguous uint8 [B,3,h,w] tensor")
+    h, w = out.shape[2], out.shape[3]
+    if min(B, H, W, h, w) <= 0:
+        raise CcvpeError("resize_u8: empty image: %s -> %s" % (tuple(img.shape), tuple(out.shape)))
+    _require_cuda(img, out)
+    _check(load().ccvpe_resize_u8(_ptr(img), 1 if nhwc else 0, B, H, W, h, w, _ptr(out), _stream()), "ccvpe_resize_u8")

@@ -5,7 +5,7 @@
 //       dst[b, c, h, w] = (src[b, c, h, (w - shift_b) mod W] / 255 - mean[c]) / std[c]            w < crop_w
 // The host ships 1 byte per sample instead of 4 (the fp32 images were what bounded 8-GPU end-to-end throughput).  The
 // arithmetic is the reference's, operation for operation (IEEE fp32 divide, subtract, divide), so the result is
-// bit-identical to torchvision's transforms on the same uint8 pixels.  Resizing stays with the image decoder on the host.
+// bit-identical to torchvision's transforms on the same uint8 pixels.  The Resize before it is resize.cu.
 #include "common.cuh"
 
 namespace ccvpe {

@@ -9,7 +9,8 @@ called, and there is no PyTorch fallback for the decoder.
 Extras over the reference (all optional, defaults reproduce the reference's fp32 behaviour):
   * `set_precision("bf16")`  -- encoders in bf16 channels-last, decoder kernels on tcgen05 tensor cores;
   * `decode_pose(heatmap, ori)` -- the scripts' NumPy argmax/orientation decode as a CUDA kernel;
-  * `localize(grd, sat)`     -- forward + decode in one call, returns only the small pose tensors.
+  * `localize(grd, sat)`     -- forward + decode in one call, returns only the small pose tensors;
+  * `resize_u8(img, size)`   -- the reference's bilinear `transforms.Resize` of native-size uint8 images, on the device.
 """
 from __future__ import annotations
 
@@ -295,9 +296,33 @@ class _CVMBase(nn.Module):
             cabi.ingest_u8(img_u8, out, shift)
         return out
 
-    def localize_u8(self, grd_u8, sat_u8, shift=None, crop_w=None):
-        """uint8 images in, poses out: normalise (/ roll / crop) + forward + pose decode, all on the device.  Without a roll or
-        crop the bf16 plan reads the uint8 images straight from the stem kernel (no fp32 image is ever materialised)."""
+    @staticmethod
+    def resize_u8(img_u8, size, out=None):
+        """The reference's transforms.Resize(size) (bilinear) on the GPU: uint8 [B,3,H,W] / [B,H,W,3] -> uint8 [B,3,h,w]
+        with size = (h, w), bit-identical to `transforms.Resize(size)` on each image as a PIL image (Pillow's 8-bit
+        fixed-point resampler), so everything downstream (`ingest`, `forward` on uint8 images) sees the reference's pixels.
+        One call resizes images of one input size: batches whose native sizes differ (KITTI's vary by drive) are grouped by
+        size by the caller.  `forward` never resizes; feed it the output of this."""
+        h, w = (int(v) for v in size)
+        if h <= 0 or w <= 0:
+            raise cabi.CcvpeError("resize_u8: size must be two positive ints (h, w), got %r" % (size,))
+        if out is None:
+            out = torch.empty((img_u8.shape[0], 3, h, w), dtype=torch.uint8, device=img_u8.device)
+        elif tuple(out.shape[2:]) != (h, w):
+            raise cabi.CcvpeError("resize_u8: out is %s but size is %r" % (tuple(out.shape), (h, w)))
+        with cabi.device_of(img_u8):
+            cabi.resize_u8(img_u8, out)
+        return out
+
+    def localize_u8(self, grd_u8, sat_u8, shift=None, crop_w=None, grd_size=None, sat_size=None):
+        """uint8 images in, poses out: (resize +) normalise (/ roll / crop) + forward + pose decode, all on the device.
+        grd_size / sat_size: (h, w) to resize the native-resolution images to first (`resize_u8`), as the reference's
+        Resize does before its roll and crop; None if the images are already at model resolution.  Without a roll or crop
+        the bf16 plan reads the uint8 images straight from the stem kernel (no fp32 image is ever materialised)."""
+        if grd_size is not None:
+            grd_u8 = self.resize_u8(grd_u8, grd_size)
+        if sat_size is not None:
+            sat_u8 = self.resize_u8(sat_u8, sat_size)
         if shift is None and crop_w is None:
             return self.localize(grd_u8, sat_u8)
         return self.localize(self.ingest(grd_u8, shift, crop_w), sat_u8)

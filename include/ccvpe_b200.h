@@ -248,6 +248,16 @@ int ccvpe_mbconv_project_nhwc(const void* d, const void* wg, const void* residua
 int ccvpe_ingest_u8(const uint8_t* src, int nhwc, int B, int H, int W, int crop_w, const int32_t* shift,
                     const float* mean_host, const float* std_host, float* dst, void* stream);
 
+/* f4  Resize before ingest -- reference transforms.Resize([out_h, out_w]) on each image as a PIL image (train_VIGOR.py:55-70),
+ * i.e. Pillow's Image.resize((out_w, out_h), BILINEAR) in 8 bits per channel: per axis, integer weights (2^22 fixed point)
+ * from Pillow's double-precision coefficient tables, horizontal pass first into a uint8 intermediate, then the vertical pass.
+ * Bit-identical to Pillow for any ratio in either direction (downscales by up to 1000x per axis; a factor so large that
+ * one output pixel's coefficient tables and uint8 intermediate column do not fit in shared memory is refused with
+ * CCVPE_ERR_BAD_ARGUMENT).  src: uint8 image batch, NCHW [B,3,H,W] (nhwc == 0) or NHWC [B,H,W,3] (nhwc != 0);
+ * dst: uint8 NCHW [B,3,out_h,out_w] (the layout ccvpe_ingest_u8 and ccvpe_stem_conv_silu_u8_nhwc read), not overlapping src.
+ * One launch; the coefficients are computed on the device: no workspace, no allocation, no synchronisation. */
+int ccvpe_resize_u8(const uint8_t* src, int nhwc, int B, int H, int W, int out_h, int out_w, uint8_t* dst, void* stream);
+
 /* =================================================================================================================
  * Training step (BASELINE.json configs[4]; reference train_VIGOR.py:120-150, losses.py:4-29): backward kernels.
  * The data gradient of every convolution is a `ccvpe_igemm` call on re-laid-out weights (a 3x3 pad-1 conv's is a 3x3 pad-1
