@@ -31,6 +31,7 @@ EXPORTED_SYMBOLS = (
     "ccvpe_relu_bwd", "ccvpe_scale_rows", "ccvpe_planar_to_cl", "ccvpe_cl_to_planar", "ccvpe_ori_normalize_bwd",
     "ccvpe_match_bwd_scratch_elems", "ccvpe_match_level_bwd", "ccvpe_loss_workspace_elems", "ccvpe_infonce_loss",
     "ccvpe_cross_entropy_loss", "ccvpe_orientation_loss", "ccvpe_grd_descriptors_bwd",
+    "ccvpe_gt_pyramid", "ccvpe_infonce_loss_binned", "ccvpe_orientation_loss_const",
 )
 
 
@@ -196,6 +197,14 @@ def load() -> C.CDLL:
     lib.ccvpe_orientation_loss.restype = C.c_int
     lib.ccvpe_orientation_loss.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p,
                                            C.c_void_p, C.c_void_p]
+    lib.ccvpe_gt_pyramid.restype = C.c_int
+    lib.ccvpe_gt_pyramid.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
+    lib.ccvpe_infonce_loss_binned.restype = C.c_int
+    lib.ccvpe_infonce_loss_binned.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int64, C.c_float,
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.ccvpe_orientation_loss_const.restype = C.c_int
+    lib.ccvpe_orientation_loss_const.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p,
+                                                 C.c_void_p, C.c_void_p, C.c_void_p]
     lib.ccvpe_grd_descriptors_bwd.restype = C.c_int
     lib.ccvpe_grd_descriptors_bwd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                               C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int,
@@ -671,6 +680,69 @@ def orientation_loss(ori: torch.Tensor, gt_ori: torch.Tensor, gt: torch.Tensor, 
     ws = torch.empty(2048, dtype=torch.float32, device=ori.device)
     _check(load().ccvpe_orientation_loss(_ptr(ori), _ptr(gt_ori), _ptr(gt), B, HW, _ptr(loss), _ptr(d_ori), _ptr(ws),
                                          _stream()), "ccvpe_orientation_loss")
+
+
+#: max_pool2d kernel sizes of the label pyramid, in the order of the six score volumes a model returns (scores1..6)
+GT_PYRAMID_KS = (64, 32, 16, 8, 4, 2)
+
+
+def _require_f32(name: str, t: torch.Tensor, shape):
+    """fp32, contiguous and `shape` (None entries match any size)."""
+    if not isinstance(t, torch.Tensor) or t.dtype != torch.float32:
+        raise CcvpeError("%s must be a float32 tensor, got %s" % (name, getattr(t, "dtype", type(t).__name__)))
+    if t.dim() != len(shape) or any(want is not None and got != want for got, want in zip(t.shape, shape)):
+        raise CcvpeError("%s must have shape %s, got %s" % (name, tuple("*" if v is None else v for v in shape),
+                                                           tuple(t.shape)))
+    if not t.is_contiguous():
+        raise CcvpeError("%s must be contiguous" % name)
+
+
+def gt_pyramid_elems(B: int, H: int, W: int) -> int:
+    return sum(B * (H // k) * (W // k) for k in GT_PYRAMID_KS)
+
+
+def gt_pyramid(gt: torch.Tensor, out: torch.Tensor):
+    """gt: fp32 [B, 1, H, W] contiguous, H and W multiples of 64; out: fp32 [gt_pyramid_elems(B, H, W)].  Writes
+    max_pool2d(gt, k, stride=k) for k in GT_PYRAMID_KS, each [B, 1, H/k, W/k], one after the other."""
+    _require_f32("gt", gt, (None, 1, None, None))
+    B, _, H, W = gt.shape
+    if B <= 0 or H <= 0 or W <= 0 or H % 64 or W % 64:
+        raise CcvpeError("gt_pyramid: H and W must be positive multiples of 64, got gt %s" % (tuple(gt.shape),))
+    _require_f32("out", out, (gt_pyramid_elems(B, H, W),))
+    _require_cuda(gt, out)
+    _check(load().ccvpe_gt_pyramid(_ptr(gt), B, H, W, _ptr(out), _stream()), "ccvpe_gt_pyramid")
+
+
+def infonce_loss_binned(scores: torch.Tensor, pooled: torch.Tensor, bin_w: torch.Tensor, temperature: float,
+                        loss: torch.Tensor, d_scores: torch.Tensor):
+    """infonce_loss on the labels pooled[b, 0] * bin_w[b, r] without materialising them: scores fp32 [B, R, h, w],
+    pooled fp32 [B, 1, h, w], bin_w fp32 [B, R], loss fp32 [], d_scores fp32 [B, R, h, w]; all contiguous."""
+    _require_f32("scores", scores, (None, None, None, None))
+    B, R, h, w = scores.shape
+    _require_f32("gt_pooled", pooled, (B, 1, h, w))
+    _require_f32("bin_weights", bin_w, (B, R))
+    _require_f32("loss", loss, ())
+    _require_f32("d_scores", d_scores, (B, R, h, w))
+    _require_cuda(scores, pooled, bin_w, loss, d_scores)
+    _check(load().ccvpe_infonce_loss_binned(_ptr(scores), _ptr(pooled), _ptr(bin_w), B, R, h * w, C.c_float(temperature),
+                                            _ptr(loss), _ptr(d_scores), _ptr(_loss_ws(B, scores.device)), _stream()),
+           "ccvpe_infonce_loss_binned")
+
+
+def orientation_loss_const(ori: torch.Tensor, ori_vec: torch.Tensor, gt: torch.Tensor, loss: torch.Tensor,
+                           d_ori: torch.Tensor):
+    """orientation_loss with the target field ori_vec[b] at every pixel: ori fp32 [B, 2, H, W], ori_vec fp32 [B, 2],
+    gt fp32 [B, 1, H, W], loss fp32 [], d_ori fp32 [B, 2, H, W]; all contiguous."""
+    _require_f32("ori", ori, (None, 2, None, None))
+    B, _, H, W = ori.shape
+    _require_f32("ori_vec", ori_vec, (B, 2))
+    _require_f32("gt", gt, (B, 1, H, W))
+    _require_f32("loss", loss, ())
+    _require_f32("d_ori", d_ori, (B, 2, H, W))
+    _require_cuda(ori, ori_vec, gt, loss, d_ori)
+    ws = torch.empty(2048, dtype=torch.float32, device=ori.device)
+    _check(load().ccvpe_orientation_loss_const(_ptr(ori), _ptr(ori_vec), _ptr(gt), B, H * W, _ptr(loss), _ptr(d_ori),
+                                               _ptr(ws), _stream()), "ccvpe_orientation_loss_const")
 
 
 def grd_descriptors_bwd(feat: torch.Tensor, heads, dgs, dfeat: torch.Tensor, dw1, db1, dw2, db2):

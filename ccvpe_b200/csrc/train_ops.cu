@@ -904,9 +904,32 @@ __device__ __forceinline__ float block_sum_256(float v, float* red) {
   return r;   // valid in thread 0
 }
 
+// How the InfoNCE kernels fetch label j of row b (j = flat index into the row of n = R * hw labels).
+//   DenseLabels:  lab [B, n], the max-pooled orientation-binned map as stored.
+//   BinnedLabels: the rank-1 form of the same map, pooled [B, hw] (the pooled location map) times w [B, R] (the pair's bin
+//                 weights).  __fmul_rn is the correctly rounded product that the dense map's `gt * w` stores (max-pooling
+//                 commutes with it: rounding is monotone and w >= 0), and it keeps nvcc from contracting it into the
+//                 `w += l` / fmaf that follow, so both give the same label bits.
+struct DenseLabels {
+  const float* lab;
+  int64_t n;
+  __device__ __forceinline__ float operator()(int b, int64_t j) const { return lab[b * n + j]; }
+};
+struct BinnedLabels {
+  const float* pooled;
+  const float* w;
+  int R;
+  uint32_t hw;                                     // R * hw < 2^31 (checked by the launcher)
+  __device__ __forceinline__ float operator()(int b, int64_t j) const {
+    const uint32_t r = (uint32_t)j / hw, p = (uint32_t)j - r * hw;
+    return __fmul_rn(pooled[(int64_t)b * hw + p], w[b * R + r]);
+  }
+};
+
 // infoNCE (losses.py:4-20): per (row b, chunk): sum exp(s / tau), sum w, sum w * s / tau       (w = label if label > 1e-2)
+template <typename Labels>
 __global__ void __launch_bounds__(LS_THREADS)
-infonce_partial_kernel(const float* __restrict__ s, const float* __restrict__ lab, int64_t n, int chunks, float inv_tau,
+infonce_partial_kernel(const float* __restrict__ s, const Labels lab, int64_t n, int chunks, float inv_tau,
                        float* __restrict__ part) {
   __shared__ float red[LS_THREADS / 32];
   const int b = blockIdx.y, ch = blockIdx.x;
@@ -915,7 +938,7 @@ infonce_partial_kernel(const float* __restrict__ s, const float* __restrict__ la
   float e = 0.f, w = 0.f, ws = 0.f;
   for (int64_t j = lo + threadIdx.x; j < hi; j += LS_THREADS) {
     const float v = s[b * n + j] * inv_tau;
-    const float l = lab[b * n + j];
+    const float l = lab(b, j);
     e += __expf(v);
     if (l > 1e-2f) {
       w += l;
@@ -950,13 +973,14 @@ __global__ void infonce_finalize_kernel(const float* __restrict__ part, int B, i
 }
 
 // d loss / d s[b, j] = -(1 / W) * ( w_j / tau - (sum_b w) * exp(s_j / tau) / (tau * sum_b exp) )
-__global__ void infonce_grad_kernel(const float* __restrict__ s, const float* __restrict__ lab, int64_t n, int B,
+template <typename Labels>
+__global__ void infonce_grad_kernel(const float* __restrict__ s, const Labels lab, int64_t n, int B,
                                     float inv_tau, const float* __restrict__ stats, float* __restrict__ ds) {
   const float W = stats[2 * B];
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < (int64_t)B * n; i += (int64_t)gridDim.x * blockDim.x) {
     const int b = (int)(i / n);
     const float v = s[i] * inv_tau;
-    const float l = lab[i];
+    const float l = lab(b, i - b * n);
     const float w = l > 1e-2f ? l : 0.f;
     ds[i] = -(w - stats[b * 2 + 1] * __expf(v) / stats[b * 2]) * inv_tau / W;
   }
@@ -1029,9 +1053,23 @@ __global__ void ce_grad_kernel(const float* __restrict__ lg, const float* __rest
   }
 }
 
+// How ori_loss_kernel fetches the target (c = 0: cos, 1: sin) of pair b at pixel r.
+//   DenseOrientation: gt_ori planar [B, 2, HW], the orientation field as stored.
+//   ConstOrientation: v [B, 2], one unit vector per pair (the field is constant over the map).
+struct DenseOrientation {
+  const float* gt_ori;
+  int64_t HW;
+  __device__ __forceinline__ float operator()(int64_t b, int c, int64_t r) const { return gt_ori[(b * 2 + c) * HW + r]; }
+};
+struct ConstOrientation {
+  const float* v;
+  __device__ __forceinline__ float operator()(int64_t b, int c, int64_t) const { return v[b * 2 + c]; }
+};
+
 // orientation loss (losses.py:28-29): sum_p gt[p] * ((go0 - o0)^2 + (go1 - o1)^2) / B; partial per block
+template <typename Target>
 __global__ void __launch_bounds__(LS_THREADS)
-ori_loss_kernel(const float* __restrict__ ori, const float* __restrict__ gt_ori, const float* __restrict__ gt, int64_t HW,
+ori_loss_kernel(const float* __restrict__ ori, const Target gt_ori, const float* __restrict__ gt, int64_t HW,
                 int B, float* __restrict__ part, float* __restrict__ d_ori) {
   __shared__ float red[LS_THREADS / 32];
   const float invB = 1.f / (float)B;
@@ -1039,8 +1077,8 @@ ori_loss_kernel(const float* __restrict__ ori, const float* __restrict__ gt_ori,
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < (int64_t)B * HW; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t b = i / HW, r = i - b * HW;
     const float w = gt[i];
-    const float e0 = gt_ori[(b * 2) * HW + r] - ori[(b * 2) * HW + r];
-    const float e1 = gt_ori[(b * 2 + 1) * HW + r] - ori[(b * 2 + 1) * HW + r];
+    const float e0 = gt_ori(b, 0, r) - ori[(b * 2) * HW + r];
+    const float e1 = gt_ori(b, 1, r) - ori[(b * 2 + 1) * HW + r];
     acc = fmaf(w, e0 * e0 + e1 * e1, acc);
     d_ori[(b * 2) * HW + r] = -2.f * w * e0 * invB;
     d_ori[(b * 2 + 1) * HW + r] = -2.f * w * e1 * invB;
@@ -1069,22 +1107,55 @@ inline int loss_chunks(int B, int64_t n) {
 
 extern "C" int64_t ccvpe_loss_workspace_elems(int B) { return (int64_t)B * ccvpe::LS_MAX_CHUNKS * 4 + 4 * B + 2048; }
 
+namespace ccvpe {
+
+template <typename Labels>
+static int infonce_launch(const float* scores, const Labels lab, int B, int64_t n, float temperature, float* loss,
+                          float* d_scores, float* workspace, cudaStream_t st) {
+  const int chunks = loss_chunks(B, n);
+  float* part = workspace;
+  float* stats = workspace + (int64_t)B * LS_MAX_CHUNKS * 4;
+  infonce_partial_kernel<<<dim3(chunks, B), LS_THREADS, 0, st>>>(scores, lab, n, chunks, 1.f / temperature, part);
+  CCVPE_LAUNCH_CHECK("infonce_partial_kernel");
+  infonce_finalize_kernel<<<1, 32, 0, st>>>(part, B, chunks, stats, loss);
+  CCVPE_LAUNCH_CHECK("infonce_finalize_kernel");
+  infonce_grad_kernel<<<ew_blocks((int64_t)B * n), 256, 0, st>>>(scores, lab, n, B, 1.f / temperature, stats, d_scores);
+  CCVPE_LAUNCH_CHECK("infonce_grad_kernel");
+  return CCVPE_OK;
+}
+
+template <typename Target>
+static int ori_loss_launch(const float* ori, const Target gt_ori, const float* gt, int B, int64_t HW, float* loss,
+                           float* d_ori, float* workspace, cudaStream_t st) {
+  int blocks = ew_blocks((int64_t)B * HW);
+  if (blocks > 1024) blocks = 1024;
+  ori_loss_kernel<<<blocks, LS_THREADS, 0, st>>>(ori, gt_ori, gt, HW, B, workspace, d_ori);
+  CCVPE_LAUNCH_CHECK("ori_loss_kernel");
+  sum_scale_kernel<<<1, 32, 0, st>>>(workspace, blocks, 1.f / (float)B, loss);
+  CCVPE_LAUNCH_CHECK("sum_scale_kernel");
+  return CCVPE_OK;
+}
+
+}  // namespace ccvpe
+
 extern "C" int ccvpe_infonce_loss(const float* scores, const float* labels, int B, int64_t n, float temperature, float* loss,
                                   float* d_scores, float* workspace, void* stream) {
   using namespace ccvpe;
   CCVPE_REQUIRE(scores && labels && loss && d_scores && workspace && B > 0 && n > 0 && temperature > 0.f,
                 "ccvpe_infonce_loss: bad argument");
-  cudaStream_t st = (cudaStream_t)stream;
-  const int chunks = loss_chunks(B, n);
-  float* part = workspace;
-  float* stats = workspace + (int64_t)B * LS_MAX_CHUNKS * 4;
-  infonce_partial_kernel<<<dim3(chunks, B), LS_THREADS, 0, st>>>(scores, labels, n, chunks, 1.f / temperature, part);
-  CCVPE_LAUNCH_CHECK("infonce_partial_kernel");
-  infonce_finalize_kernel<<<1, 32, 0, st>>>(part, B, chunks, stats, loss);
-  CCVPE_LAUNCH_CHECK("infonce_finalize_kernel");
-  infonce_grad_kernel<<<ew_blocks((int64_t)B * n), 256, 0, st>>>(scores, labels, n, B, 1.f / temperature, stats, d_scores);
-  CCVPE_LAUNCH_CHECK("infonce_grad_kernel");
-  return CCVPE_OK;
+  return infonce_launch(scores, DenseLabels{labels, n}, B, n, temperature, loss, d_scores, workspace, (cudaStream_t)stream);
+}
+
+extern "C" int ccvpe_infonce_loss_binned(const float* scores, const float* pooled, const float* bin_w, int B, int R,
+                                         int64_t HW, float temperature, float* loss, float* d_scores, float* workspace,
+                                         void* stream) {
+  using namespace ccvpe;
+  CCVPE_REQUIRE(scores && pooled && bin_w && loss && d_scores && workspace && B > 0 && R > 0 && HW > 0 &&
+                    (int64_t)R * HW <= INT32_MAX && temperature > 0.f,
+                "ccvpe_infonce_loss_binned: bad argument (B=%d, R=%d, HW=%lld)", B, R, (long long)HW);
+  const int64_t n = (int64_t)R * HW;
+  return infonce_launch(scores, BinnedLabels{pooled, bin_w, R, (uint32_t)HW}, B, n, temperature, loss, d_scores, workspace,
+                        (cudaStream_t)stream);
 }
 
 extern "C" int ccvpe_cross_entropy_loss(const float* logits, const float* labels, int B, int64_t n, float* loss,
@@ -1108,13 +1179,79 @@ extern "C" int ccvpe_orientation_loss(const float* ori, const float* gt_ori, con
                                       float* d_ori, float* workspace, void* stream) {
   using namespace ccvpe;
   CCVPE_REQUIRE(ori && gt_ori && gt && loss && d_ori && workspace && B > 0 && HW > 0, "ccvpe_orientation_loss: bad argument");
-  cudaStream_t st = (cudaStream_t)stream;
-  int blocks = ew_blocks((int64_t)B * HW);
-  if (blocks > 1024) blocks = 1024;
-  ori_loss_kernel<<<blocks, LS_THREADS, 0, st>>>(ori, gt_ori, gt, HW, B, workspace, d_ori);
-  CCVPE_LAUNCH_CHECK("ori_loss_kernel");
-  sum_scale_kernel<<<1, 32, 0, st>>>(workspace, blocks, 1.f / (float)B, loss);
-  CCVPE_LAUNCH_CHECK("sum_scale_kernel");
+  return ori_loss_launch(ori, DenseOrientation{gt_ori, HW}, gt, B, HW, loss, d_ori, workspace, (cudaStream_t)stream);
+}
+
+extern "C" int ccvpe_orientation_loss_const(const float* ori, const float* ori_vec, const float* gt, int B, int64_t HW,
+                                            float* loss, float* d_ori, float* workspace, void* stream) {
+  using namespace ccvpe;
+  CCVPE_REQUIRE(ori && ori_vec && gt && loss && d_ori && workspace && B > 0 && HW > 0,
+                "ccvpe_orientation_loss_const: bad argument");
+  return ori_loss_launch(ori, ConstOrientation{ori_vec}, gt, B, HW, loss, d_ori, workspace, (cudaStream_t)stream);
+}
+
+// ====================================================================================================================
+// Label pyramid of the InfoNCE terms (reference train_VIGOR.py:128-133, max_pool2d(gt, k, stride=k) for k = 64 ... 2) in one
+// pass: each CTA loads one 64x64 tile of gt [B, H, W] with float4 loads and halves it 2x2 by 2x2 in shared memory, writing
+// every level on the way.  Level l (k = 64 >> l) is [B, H/k, W/k] at element offset B * sum_{m<l} (H / k_m) * (W / k_m) of
+// `out`.  The max propagates NaN like max_pool2d: any NaN in a window gives NaN.
+// ====================================================================================================================
+namespace ccvpe {
+
+constexpr int PYR_TILE = 64, PYR_THREADS = 256, PYR_LEVELS = 6;
+
+__device__ __forceinline__ float max_nan(float a, float b) { return (a > b || a != a) ? a : b; }
+
+__host__ __device__ __forceinline__ int64_t pyr_level_offset(int l, int B, int H, int W) {
+  int64_t off = 0;
+  for (int m = 0; m < l; ++m) off += (int64_t)B * (H >> (PYR_LEVELS - m)) * (W >> (PYR_LEVELS - m));
+  return off;
+}
+
+__global__ void __launch_bounds__(PYR_THREADS) gt_pyramid_kernel(const float* __restrict__ gt, int H, int W,
+                                                                 float* __restrict__ out) {
+  __shared__ float4 tile4[PYR_TILE * PYR_TILE / 4];
+  __shared__ float halved[PYR_TILE * PYR_TILE / 4];
+  float* tile = reinterpret_cast<float*>(tile4);
+  const int tx = blockIdx.x, ty = blockIdx.y, b = blockIdx.z, B = gridDim.z;
+  const float* src = gt + ((int64_t)b * H + (int64_t)ty * PYR_TILE) * W + (int64_t)tx * PYR_TILE;
+#pragma unroll
+  for (int i = 0; i < PYR_TILE * PYR_TILE / 4 / PYR_THREADS; ++i) {
+    const int q = threadIdx.x + i * PYR_THREADS, row = q / (PYR_TILE / 4), c4 = q % (PYR_TILE / 4);
+    tile4[q] = __ldg(reinterpret_cast<const float4*>(src + (int64_t)row * W) + c4);
+  }
+  __syncthreads();
+  // level l = 5 .. 0 (k = 2 .. 64): this tile's n x n map (n = 64 / k) is reduced from the 2n x 2n one, ping-ponging
+  // tile <-> halved
+  float* cur = tile;
+  float* nxt = halved;
+  for (int l = PYR_LEVELS - 1; l >= 0; --l) {
+    const int n = 1 << l, Hl = H >> (PYR_LEVELS - l), Wl = W >> (PYR_LEVELS - l);
+    float* dst = out + pyr_level_offset(l, B, H, W) + ((int64_t)b * Hl + (int64_t)ty * n) * Wl + (int64_t)tx * n;
+    for (int q = threadIdx.x; q < n * n; q += PYR_THREADS) {
+      const int y = q >> l, x = q & (n - 1);
+      const float* c = cur + (2 * y) * (2 * n) + 2 * x;
+      const float m = max_nan(max_nan(c[0], c[1]), max_nan(c[2 * n], c[2 * n + 1]));
+      nxt[q] = m;
+      dst[(int64_t)y * Wl + x] = m;
+    }
+    __syncthreads();
+    float* t = cur;
+    cur = nxt;
+    nxt = t;
+  }
+}
+
+}  // namespace ccvpe
+
+extern "C" int ccvpe_gt_pyramid(const float* gt, int B, int H, int W, float* out, void* stream) {
+  using namespace ccvpe;
+  CCVPE_REQUIRE(gt && out && B > 0 && H > 0 && W > 0 && H % PYR_TILE == 0 && W % PYR_TILE == 0 && B <= 65535 &&
+                    H / PYR_TILE <= 65535 && ((uintptr_t)gt & 15) == 0,
+                "ccvpe_gt_pyramid: bad argument (B=%d, H=%d, W=%d: H and W must be positive multiples of %d, gt 16-byte "
+                "aligned)", B, H, W, PYR_TILE);
+  gt_pyramid_kernel<<<dim3(W / PYR_TILE, H / PYR_TILE, B), PYR_THREADS, 0, (cudaStream_t)stream>>>(gt, H, W, out);
+  CCVPE_LAUNCH_CHECK("gt_pyramid_kernel");
   return CCVPE_OK;
 }
 

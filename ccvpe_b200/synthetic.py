@@ -9,11 +9,12 @@ which makes end-to-end argmax comparisons meaningless -- SURVEY.md section 7.3-4
 """
 from __future__ import annotations
 
-import math
 import zlib
 from typing import Dict
 
 import torch
+
+from .losses import orientation_labels
 
 #: input shapes (H, W) of the ground image per dataset family; aerial is always 512x512
 GROUND_SHAPES = {"vigor": (320, 640), "vigor_fov180": (320, 320), "vigor_fov108": (320, 192),
@@ -67,27 +68,29 @@ def synthetic_pair(batch: int, ground_hw, seed: int = 0, dtype=torch.float32):
     return grd, sat
 
 
-def synthetic_ground_truth(batch: int, seed: int = 0, size: int = 512, n_bins: int = 20):
-    """Synthetic training ground truth with the statistics of the reference dataset (reference datasets.py:142-166): a sigma-4 Gaussian at a random
-    pixel, the same Gaussian split over two adjacent orientation bins, and a constant unit-vector orientation field."""
+def synthetic_labels(batch: int, seed: int = 0, size: int = 512):
+    """Compact synthetic training labels with the statistics of the reference dataset (reference datasets.py:142-166):
+    gt [B, 1, size, size], a sigma-4 Gaussian at a random pixel, and each pair's orientation in degrees, a float64 [B]
+    tensor in [0, 360).  `losses.orientation_labels(angles)` turns the angles into the bin weights and unit vectors that
+    `losses.training_loss_from_labels` reads; `synthetic_ground_truth` expands the same draws into the dense maps."""
     g = torch.Generator().manual_seed(20_000 + seed)
     ys = torch.arange(size, dtype=torch.float32).view(size, 1)
     xs = torch.arange(size, dtype=torch.float32).view(1, size)
     gt = torch.zeros(batch, 1, size, size)
-    gt_with_ori = torch.zeros(batch, n_bins, size, size)
-    gt_orientation = torch.zeros(batch, 2, size, size)
+    angles = torch.zeros(batch, dtype=torch.float64)
     for b in range(batch):
         cy, cx = (torch.rand(2, generator=g) * (size - 64) + 32).tolist()
-        blob = torch.exp(-((ys - cy) ** 2 + (xs - cx) ** 2) / (2.0 * 4.0 ** 2))
-        gt[b, 0] = blob
-        angle = float(torch.rand(1, generator=g)) * 360.0
-        index, ratio = int(angle // 18), (angle % 18) / 18
-        if index == 0:
-            gt_with_ori[b, 0] = blob * (1 - ratio)
-            gt_with_ori[b, n_bins - 1] = blob * ratio
-        else:
-            gt_with_ori[b, n_bins - index] = blob * (1 - ratio)
-            gt_with_ori[b, n_bins - index - 1] = blob * ratio
-        gt_orientation[b, 0] = math.cos(math.radians(angle))
-        gt_orientation[b, 1] = math.sin(math.radians(angle))
+        gt[b, 0] = torch.exp(-((ys - cy) ** 2 + (xs - cx) ** 2) / (2.0 * 4.0 ** 2))
+        angles[b] = float(torch.rand(1, generator=g)) * 360.0
+    return gt, angles
+
+
+def synthetic_ground_truth(batch: int, seed: int = 0, size: int = 512, n_bins: int = 20):
+    """Synthetic training ground truth with the statistics of the reference dataset (reference datasets.py:142-166): a sigma-4 Gaussian at a random
+    pixel, the same Gaussian split over two adjacent orientation bins, and a constant unit-vector orientation field.
+    The dense form of `synthetic_labels` (same draws for the same seed)."""
+    gt, angles = synthetic_labels(batch, seed, size)
+    bin_weights, ori_vec = orientation_labels(angles, n_bins)
+    gt_with_ori = gt * bin_weights[:, :, None, None]
+    gt_orientation = ori_vec[:, :, None, None].expand(batch, 2, size, size).contiguous()
     return gt, gt_with_ori, gt_orientation

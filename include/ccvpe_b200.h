@@ -338,6 +338,21 @@ int ccvpe_cross_entropy_loss(const float* logits, const float* labels, int B, in
 int ccvpe_orientation_loss(const float* ori, const float* gt_ori, const float* gt, int B, int64_t HW, float* loss,
                            float* d_ori, float* workspace, void* stream);
 
+/* The same losses from compact labels.  A pair's orientation-binned map is rank 1, gt_with_ori[b, r] = gt[b] * bin_w[b, r],
+ * and its orientation field is one unit vector, gt_ori[b, :, p] = ori_vec[b, :]; these read the factors instead of the maps
+ * and give the same loss and gradient bits as the calls above fed the materialised maps.
+ *   label pyramid: gt [B, H, W] (16-byte aligned; H, W multiples of 64, else CCVPE_ERR_BAD_ARGUMENT) -> out, the six
+ *     max_pool2d(gt, k, stride=k) maps, k = 64, 32, 16, 8, 4, 2 in this order; level l (k = 64 >> l) is [B, H/k, W/k] at
+ *     element offset B * sum_{m<l} (H >> (6-m)) * (W >> (6-m)) (one 64x64 tile per CTA, read once).  NaN propagates.
+ *   infoNCE: scores [B, R, HW] of one level, pooled [B, HW] its label pyramid level, bin_w [B, R] (>= 0); the labels are
+ *     the correctly rounded products pooled[b, p] * bin_w[b, r].  R * HW < 2^31.  d_scores [B, R, HW].
+ *   orientation: ori planar [B, 2, HW], ori_vec [B, 2], gt [B, HW]; d_ori [B, 2, HW]. */
+int ccvpe_gt_pyramid(const float* gt, int B, int H, int W, float* out, void* stream);
+int ccvpe_infonce_loss_binned(const float* scores, const float* pooled, const float* bin_w, int B, int R, int64_t HW,
+                              float temperature, float* loss, float* d_scores, float* workspace, void* stream);
+int ccvpe_orientation_loss_const(const float* ori, const float* ori_vec, const float* gt, int B, int64_t HW,
+                                 float* loss, float* d_ori, float* workspace, void* stream);
+
 /* Backward of the ground descriptor heads (models.py:57-97, 152-157); arguments as ccvpe_grd_descriptors plus the incoming
  * dg[l] fp32 [B, W*c[l]].  Outputs: dfeat fp32 [B, K, H, W] contiguous (NCHW), dw1[l] [c, K], db1[l] [c], dw2[l] [H],
  * db2[l] [1].  scratch: fp32, >= 2*n_heads*B*K*W elements. */
