@@ -16,7 +16,7 @@ OBJ_DIR = os.path.join(PKG_DIR, "build")
 INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include")
 LIB_PATH = os.path.join(PKG_DIR, "libccvpe_b200.so")
 SOURCES = ["runtime.cu", "descriptors.cu", "match.cu", "pointwise.cu", "igemm_simt.cu", "igemm_tcgen05.cu",
-           "conv_ring_tcgen05.cu", "match_tcgen05.cu", "project_tcgen05.cu", "stem_tcgen05.cu", "encoder_ops.cu", "ingest.cu", "resize.cu", "train_ops.cu", "wgrad_tcgen05.cu"]
+           "conv_ring_tcgen05.cu", "match_tcgen05.cu", "project_tcgen05.cu", "stem_tcgen05.cu", "encoder_ops.cu", "ingest.cu", "resize.cu", "affine.cu", "train_ops.cu", "wgrad_tcgen05.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 
 

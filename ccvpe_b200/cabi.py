@@ -6,6 +6,7 @@ to own device memory and the stream; every pointer handed to the library is `ten
 from __future__ import annotations
 
 import ctypes as C
+import numbers
 import os
 from typing import Optional, Sequence
 
@@ -25,7 +26,7 @@ EXPORTED_SYMBOLS = (
     "ccvpe_pose_scratch_bytes", "ccvpe_pose_decode", "ccvpe_bias_silu_nhwc", "ccvpe_dwconv_bias_silu_nhwc",
     "ccvpe_pointwise_silu_nhwc", "ccvpe_stem_conv_silu_nhwc", "ccvpe_se_gate_scale", "ccvpe_mbconv_project_nhwc",
     "ccvpe_wrap_columns_nhwc",
-    "ccvpe_ingest_u8", "ccvpe_resize_u8", "ccvpe_stem_conv_silu_u8_nhwc",
+    "ccvpe_ingest_u8", "ccvpe_resize_u8", "ccvpe_affine_u8", "ccvpe_stem_conv_silu_u8_nhwc",
     # training step (config 5)
     "ccvpe_wgrad_workspace_elems", "ccvpe_wgrad", "ccvpe_wgrad_plan", "ccvpe_colsum_workspace_elems", "ccvpe_colsum",
     "ccvpe_relu_bwd", "ccvpe_scale_rows", "ccvpe_planar_to_cl", "ccvpe_cl_to_planar", "ccvpe_ori_normalize_bwd",
@@ -157,6 +158,9 @@ def load() -> C.CDLL:
     lib.ccvpe_resize_u8.restype = C.c_int
     lib.ccvpe_resize_u8.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                     C.c_void_p]
+    lib.ccvpe_affine_u8.restype = C.c_int
+    lib.ccvpe_affine_u8.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                    C.c_int, C.POINTER(C.c_uint8), C.c_void_p, C.c_void_p]
     lib.ccvpe_wgrad_workspace_elems.restype = C.c_int64
     lib.ccvpe_wgrad_workspace_elems.argtypes = [C.POINTER(WgradDesc)]
     lib.ccvpe_wgrad.restype = C.c_int
@@ -807,3 +811,48 @@ def resize_u8(img: torch.Tensor, out: torch.Tensor):
         raise CcvpeError("resize_u8: empty image: %s -> %s" % (tuple(img.shape), tuple(out.shape)))
     _require_cuda(img, out)
     _check(load().ccvpe_resize_u8(_ptr(img), 1 if nhwc else 0, B, H, W, h, w, _ptr(out), _stream()), "ccvpe_resize_u8")
+
+
+#: the resampling filters `affine_u8` accepts: Pillow's BILINEAR (`PIL.Image.Resampling.BILINEAR == 2`), the only one
+#: whose affine arithmetic is reproduced exactly
+AFFINE_RESAMPLE = ("bilinear", 2)
+
+
+def _is_int(v) -> bool:
+    return isinstance(v, numbers.Integral) and not isinstance(v, bool)
+
+
+def affine_u8(img: torch.Tensor, matrices: torch.Tensor, out: torch.Tensor, offset: Sequence[int] = (0, 0),
+              fill: Sequence[int] = (0, 0, 0), resample="bilinear"):
+    """img: uint8 [B,3,H,W] (NCHW) or [B,H,W,3] (NHWC), contiguous; matrices: float64 [B,6] contiguous, on img's device;
+    out: uint8 [B,3,h,w] contiguous.  Writes pixel (x + left, y + top) of Pillow's bilinear affine transform of each image
+    (`Image.transform(size, AFFINE, matrices[b], BILINEAR, fillcolor=fill)`, bit-identical) to out[b, :, y, x], with
+    offset = (left, top)."""
+    if isinstance(resample, bool) or resample not in AFFINE_RESAMPLE:
+        raise CcvpeError("affine_u8: resample=%r: only bilinear (PIL.Image.BILINEAR) is supported; Pillow's NEAREST and "
+                         "BICUBIC affine resamplers are not reproduced" % (resample,))
+    if img.dtype != torch.uint8 or not img.is_contiguous() or img.dim() != 4:
+        raise CcvpeError("affine_u8: img must be a contiguous uint8 [B,3,H,W] or [B,H,W,3] tensor")
+    nhwc = img.shape[1] != 3
+    if nhwc and img.shape[3] != 3:
+        raise CcvpeError("affine_u8: neither dim 1 nor dim 3 of img %s has 3 channels" % (tuple(img.shape),))
+    B = img.shape[0]
+    H, W = (img.shape[1], img.shape[2]) if nhwc else (img.shape[2], img.shape[3])
+    if matrices.dtype != torch.float64 or not matrices.is_contiguous() or tuple(matrices.shape) != (B, 6):
+        raise CcvpeError("affine_u8: matrices must be a contiguous float64 [%d, 6] tensor, got %s %s"
+                         % (B, matrices.dtype, tuple(matrices.shape)))
+    if out.dtype != torch.uint8 or not out.is_contiguous() or out.dim() != 4 or tuple(out.shape[:2]) != (B, 3):
+        raise CcvpeError("affine_u8: out must be a contiguous uint8 [B,3,h,w] tensor")
+    h, w = out.shape[2], out.shape[3]
+    if min(B, H, W, h, w) <= 0:
+        raise CcvpeError("affine_u8: empty image: %s -> %s" % (tuple(img.shape), tuple(out.shape)))
+    offset, fill = tuple(offset), tuple(fill)
+    if len(offset) != 2 or not all(_is_int(v) and 0 <= v < 2 ** 31 for v in offset):
+        raise CcvpeError("affine_u8: offset must be two non-negative ints (left, top), got %r" % (offset,))
+    if len(fill) != 3 or not all(_is_int(v) and 0 <= v <= 255 for v in fill):
+        raise CcvpeError("affine_u8: fill must be three ints in 0..255 (R, G, B), got %r" % (fill,))
+    offset, fill = [int(v) for v in offset], [int(v) for v in fill]
+    _require_cuda(img, matrices, out)
+    f = (C.c_uint8 * 3)(*fill)
+    _check(load().ccvpe_affine_u8(_ptr(img), 1 if nhwc else 0, B, H, W, _ptr(matrices), h, w, offset[0], offset[1], f,
+                                  _ptr(out), _stream()), "ccvpe_affine_u8")

@@ -10,11 +10,15 @@ Extras over the reference (all optional, defaults reproduce the reference's fp32
   * `set_precision("bf16")`  -- encoders in bf16 channels-last, decoder kernels on tcgen05 tensor cores;
   * `decode_pose(heatmap, ori)` -- the scripts' NumPy argmax/orientation decode as a CUDA kernel;
   * `localize(grd, sat)`     -- forward + decode in one call, returns only the small pose tensors;
-  * `resize_u8(img, size)`   -- the reference's bilinear `transforms.Resize` of native-size uint8 images, on the device.
+  * `resize_u8(img, size)`   -- the reference's bilinear `transforms.Resize` of native-size uint8 images, on the device;
+  * `affine_u8(img, matrices, size)`, `rotate_u8(img, angles)` -- Pillow's bilinear affine transform / rotation (+ crop) of
+    uint8 images, on the device (augmentation).
 """
 from __future__ import annotations
 
+import contextlib
 import copy
+import math
 from typing import Optional
 
 import torch
@@ -25,6 +29,33 @@ from .decoder import Fork, PostEncoderPipeline, decode_pose
 from .efficientnet import EfficientNetB0
 from .fast_encoder import FastEncoder
 from .specs import KITTI, OXFORD, SKIP_BLOCKS, SKIP_CHANNELS, VIGOR, VariantSpec
+
+
+def rotate_matrix(angle, size, center=None, translate=None):
+    """The AFFINE data `Image.rotate(angle, resample, expand=False, center, translate)` hands to `Image.transform` for an
+    image of size = (W, H), in Pillow's own float arithmetic (PIL/Image.py), as a list of 6 floats.  Where Pillow takes a
+    copy / transpose fast path instead (angle % 360 in {0, 180}, or {90, 270} on a square image, with neither center nor
+    translate given) this returns the exact matrix whose bilinear transform equals that copy / transpose."""
+    W, H = size
+    angle = angle % 360.0
+    if not (center or translate):
+        if angle == 0:
+            return [1.0, 0.0, 0.0, 0.0, 1.0, 0.0]
+        if angle == 180:
+            return [-1.0, 0.0, float(W), 0.0, -1.0, float(H)]
+        if angle in (90, 270) and W == H:
+            return [0.0, -1.0, float(W), 1.0, 0.0, 0.0] if angle == 90 else [0.0, 1.0, 0.0, -1.0, 0.0, float(H)]
+    post_trans = (0, 0) if translate is None else translate
+    if center is None:
+        center = (W / 2, H / 2)
+    angle = -math.radians(angle)
+    m = [round(math.cos(angle), 15), round(math.sin(angle), 15), 0.0,
+         round(-math.sin(angle), 15), round(math.cos(angle), 15), 0.0]
+    x, y = -center[0] - post_trans[0], -center[1] - post_trans[1]
+    m[2], m[5] = m[0] * x + m[1] * y + m[2], m[3] * x + m[4] * y + m[5]
+    m[2] += center[0]
+    m[5] += center[1]
+    return [float(v) for v in m]
 
 
 class _Permute(nn.Module):
@@ -313,6 +344,51 @@ class _CVMBase(nn.Module):
         with cabi.device_of(img_u8):
             cabi.resize_u8(img_u8, out)
         return out
+
+    @staticmethod
+    def affine_u8(img_u8, matrices, size, offset=(0, 0), fill=(0, 0, 0), out=None, resample="bilinear"):
+        """Pillow's bilinear affine transform on the GPU, one matrix per image: uint8 [B,3,H,W] / [B,H,W,3] -> uint8
+        [B,3,h,w] with size = (h, w).  `matrices`: float64 [B,6] on the images' device, each the `data` of
+        `Image.transform(.., AFFINE, data, ..)` (output pixel centre -> input coordinate); it is read when the kernel runs,
+        so a captured CUDA graph replays with whatever the tensor holds then.  `offset` = (left, top): out[b, :, y, x] is
+        pixel (x + left, y + top) of the transform, so the result is bit-identical to
+        `Image.transform((left + w, top + h), AFFINE, data, BILINEAR, fillcolor=fill).crop((left, top, left + w, top + h))`
+        on each image as a PIL image.  Only bilinear resampling is provided (see INTEGRATION.md)."""
+        h, w = (int(v) for v in size)
+        if h <= 0 or w <= 0:
+            raise cabi.CcvpeError("affine_u8: size must be two positive ints (h, w), got %r" % (size,))
+        if out is None:
+            out = torch.empty((img_u8.shape[0], 3, h, w), dtype=torch.uint8, device=img_u8.device)
+        elif tuple(out.shape[2:]) != (h, w):
+            raise cabi.CcvpeError("affine_u8: out is %s but size is %r" % (tuple(out.shape), (h, w)))
+        # a CPU tensor reaches the binding, which refuses it with a CcvpeError
+        with cabi.device_of(img_u8) if img_u8.is_cuda else contextlib.nullcontext():
+            cabi.affine_u8(img_u8, matrices, out, offset, fill, resample)
+        return out
+
+    @staticmethod
+    def rotate_u8(img_u8, angles, center=None, translate=None, fill=(0, 0, 0), size=None, offset=(0, 0),
+                  resample="bilinear", expand=False):
+        """Pillow's `Image.rotate(angle, BILINEAR, expand=False, center, translate, fillcolor=fill)` of each image on the GPU,
+        bit-identical: uint8 [B,3,H,W] / [B,H,W,3] -> uint8 [B,3,h,w].  `angles`: one angle in degrees (counter-clockwise)
+        or one per image; `center` / `translate`: as Pillow's, shared by all images.  size = (h, w) and offset = (left,
+        top) fuse a crop: the result is `.crop((left, top, left + w, top + h))` of the rotated image (size None: the input
+        size).  The [B,6] matrices are built on the host (`rotate_matrix`) and copied to the device; a CUDA-graph caller
+        builds them itself and calls `affine_u8`."""
+        if expand:
+            raise cabi.CcvpeError("rotate_u8: expand=True is not supported; the output size is the input size or `size`")
+        if img_u8.dim() != 4:
+            raise cabi.CcvpeError("rotate_u8: img must be a uint8 [B,3,H,W] or [B,H,W,3] tensor")
+        B = img_u8.shape[0]
+        H, W = (img_u8.shape[2], img_u8.shape[3]) if img_u8.shape[1] == 3 else (img_u8.shape[1], img_u8.shape[2])
+        angles = torch.as_tensor(angles, dtype=torch.float64).flatten().tolist()
+        if len(angles) == 1:
+            angles = angles * B
+        if len(angles) != B:
+            raise cabi.CcvpeError("rotate_u8: %d angles for %d images" % (len(angles), B))
+        mats = torch.tensor([rotate_matrix(a, (W, H), center, translate) for a in angles], dtype=torch.float64)
+        return _CVMBase.affine_u8(img_u8, mats.to(img_u8.device), (H, W) if size is None else size, offset, fill,
+                                  resample=resample)
 
     def localize_u8(self, grd_u8, sat_u8, shift=None, crop_w=None, grd_size=None, sat_size=None):
         """uint8 images in, poses out: (resize +) normalise (/ roll / crop) + forward + pose decode, all on the device.

@@ -258,6 +258,18 @@ int ccvpe_ingest_u8(const uint8_t* src, int nhwc, int B, int H, int W, int crop_
  * One launch; the coefficients are computed on the device: no workspace, no allocation, no synchronisation. */
 int ccvpe_resize_u8(const uint8_t* src, int nhwc, int B, int H, int W, int out_h, int out_w, uint8_t* dst, void* stream);
 
+/* f4  Geometric augmentation (rotation, shift, scale, shear, crop) -- Pillow's Image.transform(size, AFFINE, a, BILINEAR,
+ * fillcolor) in 8 bits per channel, bit-identical; Image.rotate(angle, BILINEAR, center, translate, fillcolor) is such a
+ * transform of the matrix it builds.  matrices: DEVICE float64 [B][6], one `a` per image, mapping output pixel centres to
+ * input coordinates (read at run time: a captured launch can be replayed with the matrices rewritten in place).
+ * dst[b, :, y, x] is pixel (x + left, y + top) of image b's transform, so with left, top >= 0 the output equals
+ * Image.transform((left + out_w, top + out_h), ...).crop((left, top, left + out_w, top + out_h)).  Pixels whose source
+ * coordinate falls outside the image take fill_host[0..2] (HOST uint8[3], RGB).  src: uint8 NCHW [B,3,H,W] (nhwc == 0)
+ * or NHWC [B,H,W,3] (nhwc != 0); dst: uint8 NCHW [B,3,out_h,out_w], not overlapping src.  One launch: no workspace, no
+ * allocation, no synchronisation.  Pillow's NEAREST and BICUBIC affine resamplers are not provided. */
+int ccvpe_affine_u8(const uint8_t* src, int nhwc, int B, int H, int W, const double* matrices, int out_h, int out_w,
+                    int left, int top, const uint8_t* fill_host, uint8_t* dst, void* stream);
+
 /* =================================================================================================================
  * Training step (BASELINE.json configs[4]; reference train_VIGOR.py:120-150, losses.py:4-29): backward kernels.
  * The data gradient of every convolution is a `ccvpe_igemm` call on re-laid-out weights (a 3x3 pad-1 conv's is a 3x3 pad-1
