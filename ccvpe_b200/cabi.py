@@ -6,6 +6,7 @@ to own device memory and the stream; every pointer handed to the library is `ten
 from __future__ import annotations
 
 import ctypes as C
+import math
 import numbers
 import os
 from typing import Optional, Sequence
@@ -32,7 +33,7 @@ EXPORTED_SYMBOLS = (
     "ccvpe_relu_bwd", "ccvpe_scale_rows", "ccvpe_planar_to_cl", "ccvpe_cl_to_planar", "ccvpe_ori_normalize_bwd",
     "ccvpe_match_bwd_scratch_elems", "ccvpe_match_level_bwd", "ccvpe_loss_workspace_elems", "ccvpe_infonce_loss",
     "ccvpe_cross_entropy_loss", "ccvpe_orientation_loss", "ccvpe_grd_descriptors_bwd",
-    "ccvpe_gt_pyramid", "ccvpe_infonce_loss_binned", "ccvpe_orientation_loss_const",
+    "ccvpe_gt_pyramid", "ccvpe_infonce_loss_binned", "ccvpe_orientation_loss_const", "ccvpe_pose_labels",
 )
 
 
@@ -209,6 +210,9 @@ def load() -> C.CDLL:
     lib.ccvpe_orientation_loss_const.restype = C.c_int
     lib.ccvpe_orientation_loss_const.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p,
                                                  C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.ccvpe_pose_labels.restype = C.c_int
+    lib.ccvpe_pose_labels.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_double, C.c_int, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_void_p]
     lib.ccvpe_grd_descriptors_bwd.restype = C.c_int
     lib.ccvpe_grd_descriptors_bwd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                               C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int,
@@ -747,6 +751,45 @@ def orientation_loss_const(ori: torch.Tensor, ori_vec: torch.Tensor, gt: torch.T
     ws = torch.empty(2048, dtype=torch.float32, device=ori.device)
     _check(load().ccvpe_orientation_loss_const(_ptr(ori), _ptr(ori_vec), _ptr(gt), B, H * W, _ptr(loss), _ptr(d_ori),
                                                _ptr(ws), _stream()), "ccvpe_orientation_loss_const")
+
+
+#: the bin counts `pose_labels` accepts: from 10 every bin index of VIGOR's 18-degree rule is a valid tensor index (up to
+#: 10 from the end); up to 32 one warp writes a pair's weights
+POSE_LABEL_BINS = (10, 32)
+
+
+def check_pose_label_args(H, W, sigma, n_bins):
+    """Raises CcvpeError unless H and W are positive multiples of 64, sigma is a positive finite number and n_bins is an int
+    in POSE_LABEL_BINS."""
+    if not (_is_int(H) and _is_int(W) and H > 0 and W > 0 and H % 64 == 0 and W % 64 == 0):
+        raise CcvpeError("pose_labels: H and W must be positive multiples of 64, got %r x %r" % (H, W))
+    if not (isinstance(sigma, numbers.Real) and not isinstance(sigma, bool) and math.isfinite(sigma) and sigma > 0):
+        raise CcvpeError("pose_labels: sigma must be a positive finite number, got %r" % (sigma,))
+    if not (_is_int(n_bins) and POSE_LABEL_BINS[0] <= n_bins <= POSE_LABEL_BINS[1]):
+        raise CcvpeError("pose_labels: n_bins must be an int in [%d, %d], got %r" % (*POSE_LABEL_BINS, n_bins))
+
+
+def pose_labels(poses: torch.Tensor, sigma: float, n_bins: int, gt: torch.Tensor, pyramid: torch.Tensor,
+                bin_weights: torch.Tensor, ori_vec: torch.Tensor):
+    """The compact labels of a batch of poses in one launch.  poses: float64 [B, 3] contiguous, rows (row, col, angle_deg),
+    read when the kernel runs; gt: fp32 [B, 1, H, W] (H, W multiples of 64), the sigma Gaussian at (row, col) evaluated in
+    float64; pyramid: fp32 [gt_pyramid_elems(B, H, W)], as `gt_pyramid` writes it; bin_weights fp32 [B, n_bins] and
+    ori_vec fp32 [B, 2], as `losses.orientation_labels` builds them (NaN for an angle outside [0, 360)).  All contiguous,
+    on the current device."""
+    if not isinstance(poses, torch.Tensor) or poses.dtype != torch.float64 or poses.dim() != 2 or poses.shape[1] != 3 \
+            or poses.shape[0] == 0 or not poses.is_contiguous():
+        raise CcvpeError("pose_labels: poses must be a contiguous float64 [B, 3] tensor, got %s %s"
+                         % (getattr(poses, "dtype", type(poses).__name__), tuple(getattr(poses, "shape", ()))))
+    B = poses.shape[0]
+    _require_f32("gt", gt, (B, 1, None, None))
+    H, W = gt.shape[2], gt.shape[3]
+    check_pose_label_args(H, W, sigma, n_bins)
+    _require_f32("pyramid", pyramid, (gt_pyramid_elems(B, H, W),))
+    _require_f32("bin_weights", bin_weights, (B, n_bins))
+    _require_f32("ori_vec", ori_vec, (B, 2))
+    _require_cuda(poses, gt, pyramid, bin_weights, ori_vec)
+    _check(load().ccvpe_pose_labels(_ptr(poses), B, H, W, float(sigma), n_bins, _ptr(gt), _ptr(pyramid), _ptr(bin_weights),
+                                    _ptr(ori_vec), _stream()), "ccvpe_pose_labels")
 
 
 def grd_descriptors_bwd(feat: torch.Tensor, heads, dgs, dfeat: torch.Tensor, dw1, db1, dw2, db2):

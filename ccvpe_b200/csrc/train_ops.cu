@@ -1195,10 +1195,13 @@ extern "C" int ccvpe_orientation_loss_const(const float* ori, const float* ori_v
 // pass: each CTA loads one 64x64 tile of gt [B, H, W] with float4 loads and halves it 2x2 by 2x2 in shared memory, writing
 // every level on the way.  Level l (k = 64 >> l) is [B, H/k, W/k] at element offset B * sum_{m<l} (H / k_m) * (W / k_m) of
 // `out`.  The max propagates NaN like max_pool2d: any NaN in a window gives NaN.
+// The kernel is templated on how it obtains its tile: LoadedTile reads gt; PoseTile evaluates the location label of the
+// pair's pose into it (and stores it to gt), so the labels of a pose batch are built by the same launch (see below).
 // ====================================================================================================================
 namespace ccvpe {
 
 constexpr int PYR_TILE = 64, PYR_THREADS = 256, PYR_LEVELS = 6;
+constexpr int PYR_TILE_VECS = PYR_TILE * PYR_TILE / 4 / PYR_THREADS;   // float4s of the tile per thread
 
 __device__ __forceinline__ float max_nan(float a, float b) { return (a > b || a != a) ? a : b; }
 
@@ -1208,18 +1211,115 @@ __host__ __device__ __forceinline__ int64_t pyr_level_offset(int l, int B, int H
   return off;
 }
 
-__global__ void __launch_bounds__(PYR_THREADS) gt_pyramid_kernel(const float* __restrict__ gt, int H, int W,
+// Thread t fills float4 q = t + i * PYR_THREADS of the tile: tile row q / 16, columns 4 * (q % 16) ... + 3.
+struct LoadedTile {
+  const float* gt;
+  __device__ __forceinline__ void operator()(float4* tile4, int b, int ty, int tx, int H, int W) const {
+    const float* src = gt + ((int64_t)b * H + (int64_t)ty * PYR_TILE) * W + (int64_t)tx * PYR_TILE;
+#pragma unroll
+    for (int i = 0; i < PYR_TILE_VECS; ++i) {
+      const int q = threadIdx.x + i * PYR_THREADS, row = q / (PYR_TILE / 4), c4 = q % (PYR_TILE / 4);
+      tile4[q] = __ldg(reinterpret_cast<const float4*>(src + (int64_t)row * W) + c4);
+    }
+  }
+};
+
+// Labels of a pose (row, col, angle_deg), as the host builds them in NumPy float64 / Python float arithmetic:
+//   gt[i, j] = float32(exp(-(((i - row)^2 + (j - col)^2) / (2 * sigma^2))))
+//   bin weights and orientation vector: losses.orientation_labels (VIGOR's 18-degree rule).
+// Every double operation of the formulas is an explicit _rn intrinsic, so nvcc cannot contract them into DFMAs.
+constexpr double kPoseLabelZeroArg = 120.0;   // exp(-q) < 2^-150 for q > 104: float32(exp(-q)) is +0, exp is skipped
+constexpr double kDegToRad = 3.14159265358979323846 / 180.0;   // CPython's math.radians factor (Py_MATH_PI / 180.0)
+
+// CPython's float_divmod (Objects/floatobject.c) of vx by wx: floor division and remainder with the sign of wx.
+__device__ __forceinline__ void py_divmod(double vx, double wx, double& floordiv, double& mod) {
+  mod = fmod(vx, wx);
+  double div = __ddiv_rn(__dsub_rn(vx, mod), wx);
+  if (mod != 0.0) {
+    if ((wx < 0.0) != (mod < 0.0)) {
+      mod = __dadd_rn(mod, wx);
+      div = __dsub_rn(div, 1.0);
+    }
+  } else {
+    mod = copysign(0.0, wx);
+  }
+  if (div != 0.0) {
+    floordiv = floor(div);
+    if (__dsub_rn(div, floordiv) > 0.5) floordiv = __dadd_rn(floordiv, 1.0);
+  } else {
+    floordiv = copysign(0.0, __ddiv_rn(vx, wx));
+  }
+}
+
+// losses.orientation_labels of one angle, by warp 0 (lane r writes bin r; n_bins <= 32):
+//   index = int(angle // 18), ratio = (angle % 18) / 18; bins (lo, hi) = (0, n_bins - 1) if index == 0 else
+//   (n_bins - index, n_bins - index - 1), negative bins counting from the end; w[lo] = 1 - ratio, then w[hi] = ratio;
+//   v = (cos, sin)(angle * pi / 180).  An angle outside [0, 360) or non-finite gives NaN weights and vector.
+__device__ __forceinline__ void pose_orientation_labels(double angle, int n_bins, float* __restrict__ w,
+                                                        float* __restrict__ v) {
+  const int lane = threadIdx.x;
+  if (!(angle >= 0.0 && angle < 360.0)) {
+    if (lane < n_bins) w[lane] = __int_as_float(0x7fffffff);
+    if (lane < 2) v[lane] = __int_as_float(0x7fffffff);
+    return;
+  }
+  double floordiv, mod;
+  py_divmod(angle, 18.0, floordiv, mod);
+  const int index = (int)floordiv;   // 0 ... 19
+  const double ratio = __ddiv_rn(mod, 18.0);
+  int lo = index == 0 ? 0 : n_bins - index, hi = index == 0 ? n_bins - 1 : n_bins - index - 1;
+  if (lo < 0) lo += n_bins;          // >= n_bins - 19 >= -9
+  if (hi < 0) hi += n_bins;          // >= n_bins - 20 >= -10
+  if (lane < n_bins)
+    w[lane] = lane == hi ? __double2float_rn(ratio) : lane == lo ? __double2float_rn(__dsub_rn(1.0, ratio)) : 0.f;
+  if (lane < 2) {
+    const double rad = __dmul_rn(angle, kDegToRad);
+    v[lane] = __double2float_rn(lane == 0 ? cos(rad) : sin(rad));
+  }
+}
+
+struct PoseTile {
+  const double* poses;   // [B, 3]: row, col, angle_deg
+  double sigma;
+  int n_bins;
+  float* gt;             // [B, H, W]
+  float* bin_w;          // [B, n_bins]
+  float* ori_vec;        // [B, 2]
+  __device__ __forceinline__ void operator()(float4* tile4, int b, int ty, int tx, int H, int W) const {
+    const double row = __ldg(poses + 3 * (int64_t)b), col = __ldg(poses + 3 * (int64_t)b + 1);
+    const double denom = __dmul_rn(2.0, __dmul_rn(sigma, sigma));
+    const double zero_above = __dmul_rn(kPoseLabelZeroArg, denom);   // s > zero_above: s / denom > 119.99, label +0
+    float* dst = gt + ((int64_t)b * H + (int64_t)ty * PYR_TILE) * W + (int64_t)tx * PYR_TILE;
+#pragma unroll
+    for (int i = 0; i < PYR_TILE_VECS; ++i) {
+      const int q = threadIdx.x + i * PYR_THREADS, r = q / (PYR_TILE / 4), c4 = q % (PYR_TILE / 4);
+      const double dy = __dsub_rn((double)(ty * PYR_TILE + r), row);
+      const double dy2 = __dmul_rn(dy, dy);
+      float g[4];
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const double dx = __dsub_rn((double)(tx * PYR_TILE + 4 * c4 + k), col);
+        const double s = __dadd_rn(dy2, __dmul_rn(dx, dx));
+        // written so that a NaN s (a non-finite centre) takes the exp path and gives NaN
+        g[k] = s > zero_above ? 0.f : __double2float_rn(exp(-__ddiv_rn(s, denom)));
+      }
+      const float4 t = make_float4(g[0], g[1], g[2], g[3]);
+      tile4[q] = t;
+      reinterpret_cast<float4*>(dst + (int64_t)r * W)[c4] = t;
+    }
+    if (tx == 0 && ty == 0 && threadIdx.x < 32)
+      pose_orientation_labels(__ldg(poses + 3 * (int64_t)b + 2), n_bins, bin_w + (int64_t)b * n_bins, ori_vec + 2 * (int64_t)b);
+  }
+};
+
+template <typename Tile>
+__global__ void __launch_bounds__(PYR_THREADS) gt_pyramid_kernel(const Tile fill_tile, int H, int W,
                                                                  float* __restrict__ out) {
   __shared__ float4 tile4[PYR_TILE * PYR_TILE / 4];
   __shared__ float halved[PYR_TILE * PYR_TILE / 4];
   float* tile = reinterpret_cast<float*>(tile4);
   const int tx = blockIdx.x, ty = blockIdx.y, b = blockIdx.z, B = gridDim.z;
-  const float* src = gt + ((int64_t)b * H + (int64_t)ty * PYR_TILE) * W + (int64_t)tx * PYR_TILE;
-#pragma unroll
-  for (int i = 0; i < PYR_TILE * PYR_TILE / 4 / PYR_THREADS; ++i) {
-    const int q = threadIdx.x + i * PYR_THREADS, row = q / (PYR_TILE / 4), c4 = q % (PYR_TILE / 4);
-    tile4[q] = __ldg(reinterpret_cast<const float4*>(src + (int64_t)row * W) + c4);
-  }
+  fill_tile(tile4, b, ty, tx, H, W);
   __syncthreads();
   // level l = 5 .. 0 (k = 2 .. 64): this tile's n x n map (n = 64 / k) is reduced from the 2n x 2n one, ping-ponging
   // tile <-> halved
@@ -1250,7 +1350,26 @@ extern "C" int ccvpe_gt_pyramid(const float* gt, int B, int H, int W, float* out
                     H / PYR_TILE <= 65535 && ((uintptr_t)gt & 15) == 0,
                 "ccvpe_gt_pyramid: bad argument (B=%d, H=%d, W=%d: H and W must be positive multiples of %d, gt 16-byte "
                 "aligned)", B, H, W, PYR_TILE);
-  gt_pyramid_kernel<<<dim3(W / PYR_TILE, H / PYR_TILE, B), PYR_THREADS, 0, (cudaStream_t)stream>>>(gt, H, W, out);
+  gt_pyramid_kernel<<<dim3(W / PYR_TILE, H / PYR_TILE, B), PYR_THREADS, 0, (cudaStream_t)stream>>>(LoadedTile{gt}, H, W,
+                                                                                                    out);
+  CCVPE_LAUNCH_CHECK("gt_pyramid_kernel");
+  return CCVPE_OK;
+}
+
+extern "C" int ccvpe_pose_labels(const double* poses, int B, int H, int W, double sigma, int n_bins, float* gt,
+                                 float* pyramid, float* bin_weights, float* ori_vec, void* stream) {
+  using namespace ccvpe;
+  CCVPE_REQUIRE(poses && gt && pyramid && bin_weights && ori_vec, "ccvpe_pose_labels: null pointer");
+  CCVPE_REQUIRE(B > 0 && H > 0 && W > 0 && H % PYR_TILE == 0 && W % PYR_TILE == 0 && B <= 65535 && H / PYR_TILE <= 65535,
+                "ccvpe_pose_labels: bad argument (B=%d, H=%d, W=%d: H and W must be positive multiples of %d)", B, H, W,
+                PYR_TILE);
+  CCVPE_REQUIRE(((uintptr_t)poses & 7) == 0 && ((uintptr_t)gt & 15) == 0 && ((uintptr_t)pyramid & 3) == 0 &&
+                    ((uintptr_t)bin_weights & 3) == 0 && ((uintptr_t)ori_vec & 3) == 0,
+                "ccvpe_pose_labels: misaligned pointer (poses 8-byte, gt 16-byte, the float outputs 4-byte aligned)");
+  CCVPE_REQUIRE(sigma > 0.0 && sigma <= DBL_MAX, "ccvpe_pose_labels: sigma must be positive and finite, got %g", sigma);
+  CCVPE_REQUIRE(n_bins >= 10 && n_bins <= 32, "ccvpe_pose_labels: n_bins must be in [10, 32], got %d", n_bins);
+  gt_pyramid_kernel<<<dim3(W / PYR_TILE, H / PYR_TILE, B), PYR_THREADS, 0, (cudaStream_t)stream>>>(
+      PoseTile{poses, sigma, n_bins, gt, bin_weights, ori_vec}, H, W, pyramid);
   CCVPE_LAUNCH_CHECK("gt_pyramid_kernel");
   return CCVPE_OK;
 }

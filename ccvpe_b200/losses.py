@@ -187,6 +187,11 @@ def gt_pyramid(gt):
     out = torch.empty(cabi.gt_pyramid_elems(B, H, W), dtype=torch.float32, device=g.device)
     with cabi.device_of(g):
         cabi.gt_pyramid(g, out)
+    return _pyramid_levels(out, B, H, W)
+
+
+def _pyramid_levels(out, B, H, W):
+    """The six [B, 1, H/k, W/k] levels of a label-pyramid buffer, as views."""
     levels, off = [], 0
     for k in cabi.GT_PYRAMID_KS:
         n = B * (H // k) * (W // k)
@@ -207,22 +212,70 @@ def orientation_loss_const(ori, ori_vec, gt):
     return _OrientationConst.apply(ori, ori_vec, gt)
 
 
+def _require_bins(outputs, n_bins, caller, source):
+    for level, scores in enumerate(outputs[3:9], start=1):
+        if scores.dim() != 4 or scores.shape[1] != n_bins:
+            raise cabi.CcvpeError("%s: score volume %d has shape %s, but %s has %d bins "
+                                  "(each level needs one weight per orientation channel)"
+                                  % (caller, level, tuple(scores.shape), source, n_bins))
+
+
+def _compact_label_loss(outputs, gt, levels, bin_weights, ori_vec, weight_infoNCE, weight_ori):
+    """`training_loss` on compact labels whose six pooled levels are given."""
+    logits_flattened, _heatmap, ori = outputs[0], outputs[1], outputs[2]
+    gt_flattened = torch.flatten(gt, start_dim=1)
+    gt_flattened = gt_flattened / torch.sum(gt_flattened, dim=1, keepdim=True)
+    loss_ori = orientation_loss_const(ori, ori_vec, gt)
+    nce = 0
+    for scores, gt_b in zip(outputs[3:9], levels):
+        nce = nce + infoNCELoss_binned(scores, gt_b, bin_weights)
+    loss_ce = cross_entropy_loss(logits_flattened, gt_flattened)
+    return loss_ce + weight_infoNCE * nce / 6 + weight_ori * loss_ori
+
+
 def training_loss_from_labels(outputs, gt, bin_weights, ori_vec, weight_infoNCE=1e4, weight_ori=1e1):
     """`training_loss` on compact labels: gt [B, 1, H, W], bin_weights [B, R], ori_vec [B, 2] (device tensors; see
     `orientation_labels`).  Same value and gradients as training_loss(outputs, gt, gt * bin_weights[:, :, None, None],
     ori_vec[:, :, None, None].expand(B, 2, H, W)); one label-pyramid launch replaces the six max-pools.  Every score volume
     must have bin_weights.shape[1] orientation channels."""
-    logits_flattened, _heatmap, ori = outputs[0], outputs[1], outputs[2]
-    for level, scores in enumerate(outputs[3:9], start=1):
-        if scores.dim() != 4 or scores.shape[1] != bin_weights.shape[1]:
-            raise cabi.CcvpeError("training_loss_from_labels: score volume %d has shape %s, but bin_weights has %d bins "
-                                  "(each level needs one weight per orientation channel)"
-                                  % (level, tuple(scores.shape), bin_weights.shape[1]))
-    gt_flattened = torch.flatten(gt, start_dim=1)
-    gt_flattened = gt_flattened / torch.sum(gt_flattened, dim=1, keepdim=True)
-    loss_ori = orientation_loss_const(ori, ori_vec, gt)
-    nce = 0
-    for scores, gt_b in zip(outputs[3:9], gt_pyramid(gt)):
-        nce = nce + infoNCELoss_binned(scores, gt_b, bin_weights)
-    loss_ce = cross_entropy_loss(logits_flattened, gt_flattened)
-    return loss_ce + weight_infoNCE * nce / 6 + weight_ori * loss_ori
+    _require_bins(outputs, bin_weights.shape[1], "training_loss_from_labels", "bin_weights")
+    return _compact_label_loss(outputs, gt, gt_pyramid(gt), bin_weights, ori_vec, weight_infoNCE, weight_ori)
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# Labels from poses.  A pair's labels are fully determined by its pose (row, col, angle): the location map is a Gaussian
+# at (row, col) and the orientation labels follow from the angle, so a batch can carry a float64 [B, 3] tensor and build
+# everything on the device, in one launch that also writes the label pyramid.
+# ------------------------------------------------------------------------------------------------------------------
+def labels_from_poses(poses, size=(512, 512), sigma=4.0, n_bins=20):
+    """The compact labels of poses float64 [B, 3] (device tensor; rows (row, col, angle_deg), as the reference dataset
+    draws them): returns (gt, bin_weights, ori_vec, levels), all on the poses' device.
+      gt [B, 1, H, W], size = (H, W) multiples of 64: gt[b, 0, i, j] = exp(-((i - row)^2 + (j - col)^2) / (2 sigma^2)),
+        bit-identical to NumPy float64 rounded once to float32;
+      bin_weights [B, n_bins], ori_vec [B, 2]: bit-identical to `orientation_labels(poses[:, 2], n_bins)`
+        (10 <= n_bins <= 32); an angle outside [0, 360) or non-finite gives a NaN row, so its loss is NaN;
+      levels: `gt_pyramid(gt)`, computed by the same launch (views into one buffer).
+    The poses are read when the kernel runs, so a captured CUDA graph rebuilds the labels of whatever they hold then."""
+    H, W = size
+    cabi.check_pose_label_args(H, W, sigma, n_bins)
+    if not isinstance(poses, torch.Tensor) or not poses.is_cuda or poses.dim() != 2:
+        raise cabi.CcvpeError("labels_from_poses: poses must be a float64 [B, 3] CUDA tensor; there is no CPU fallback")
+    B, dev = poses.shape[0], poses.device
+    gt = torch.empty(B, 1, H, W, dtype=torch.float32, device=dev)
+    pyramid = torch.empty(cabi.gt_pyramid_elems(B, H, W), dtype=torch.float32, device=dev)
+    bin_weights = torch.empty(B, n_bins, dtype=torch.float32, device=dev)
+    ori_vec = torch.empty(B, 2, dtype=torch.float32, device=dev)
+    with cabi.device_of(poses):
+        cabi.pose_labels(poses, sigma, n_bins, gt, pyramid, bin_weights, ori_vec)
+    return gt, bin_weights, ori_vec, _pyramid_levels(pyramid, B, H, W)
+
+
+def training_loss_from_poses(outputs, poses, sigma=4.0, weight_infoNCE=1e4, weight_ori=1e1):
+    """`training_loss_from_labels` on the labels of poses float64 [B, 3] (`labels_from_poses`, at the resolution of the
+    orientation output, with as many bins as the score volumes have orientation channels): same value and gradients, and
+    the label pyramid comes from the same launch."""
+    ori = outputs[2]
+    n_bins = outputs[3].shape[1] if outputs[3].dim() == 4 else -1
+    _require_bins(outputs, n_bins, "training_loss_from_poses", "score volume 1")
+    gt, bin_weights, ori_vec, levels = labels_from_poses(poses, tuple(ori.shape[-2:]), sigma, n_bins)
+    return _compact_label_loss(outputs, gt, levels, bin_weights, ori_vec, weight_infoNCE, weight_ori)

@@ -73,16 +73,26 @@ def synthetic_labels(batch: int, seed: int = 0, size: int = 512):
     gt [B, 1, size, size], a sigma-4 Gaussian at a random pixel, and each pair's orientation in degrees, a float64 [B]
     tensor in [0, 360).  `losses.orientation_labels(angles)` turns the angles into the bin weights and unit vectors that
     `losses.training_loss_from_labels` reads; `synthetic_ground_truth` expands the same draws into the dense maps."""
-    g = torch.Generator().manual_seed(20_000 + seed)
+    poses = synthetic_poses(batch, seed, size)
     ys = torch.arange(size, dtype=torch.float32).view(size, 1)
     xs = torch.arange(size, dtype=torch.float32).view(1, size)
     gt = torch.zeros(batch, 1, size, size)
-    angles = torch.zeros(batch, dtype=torch.float64)
+    for b in range(batch):
+        cy, cx = poses[b, :2].tolist()
+        gt[b, 0] = torch.exp(-((ys - cy) ** 2 + (xs - cx) ** 2) / (2.0 * 4.0 ** 2))
+    return gt, poses[:, 2].clone()
+
+
+def synthetic_poses(batch: int, seed: int = 0, size: int = 512):
+    """The poses `synthetic_labels` draws for the same seed (same random sequence): a float64 [B, 3] CPU tensor of rows
+    (row, col, angle_deg), the Gaussian's centre and the orientation in [0, 360).  `losses.training_loss_from_poses` builds
+    the labels from them on the device."""
+    g = torch.Generator().manual_seed(20_000 + seed)
+    poses = torch.zeros(batch, 3, dtype=torch.float64)
     for b in range(batch):
         cy, cx = (torch.rand(2, generator=g) * (size - 64) + 32).tolist()
-        gt[b, 0] = torch.exp(-((ys - cy) ** 2 + (xs - cx) ** 2) / (2.0 * 4.0 ** 2))
-        angles[b] = float(torch.rand(1, generator=g)) * 360.0
-    return gt, angles
+        poses[b] = torch.tensor([cy, cx, float(torch.rand(1, generator=g)) * 360.0], dtype=torch.float64)
+    return poses
 
 
 def synthetic_ground_truth(batch: int, seed: int = 0, size: int = 512, n_bins: int = 20):

@@ -365,6 +365,19 @@ int ccvpe_infonce_loss_binned(const float* scores, const float* pooled, const fl
 int ccvpe_orientation_loss_const(const float* ori, const float* ori_vec, const float* gt, int B, int64_t HW,
                                  float* loss, float* d_ori, float* workspace, void* stream);
 
+/* The compact labels of a batch of poses, in one launch.  poses: float64 [B, 3], rows (row, col, angle_deg), read when the
+ * kernel runs (a captured launch replays with whatever the buffer holds then).  Writes
+ *   gt [B, H, W] (16-byte aligned; H, W positive multiples of 64): gt[b, i, j] = float32(exp(-(((i - row)^2 + (j - col)^2)
+ *     / (2 * sigma^2)))), evaluated in float64 without contractions and rounded once (NumPy float64's formula); a
+ *     non-finite centre gives NaN where NumPy does;
+ *   pyramid: ccvpe_gt_pyramid(gt)'s six levels, in its layout;
+ *   bin_weights [B, n_bins] and ori_vec [B, 2]: VIGOR's 18-degree rule, bit-identical to losses.orientation_labels
+ *     (Python float arithmetic); an angle outside [0, 360) or non-finite gives NaN weights and vector.
+ * sigma > 0 and finite, 10 <= n_bins <= 32; otherwise, or on bad sizes or alignment, CCVPE_ERR_BAD_ARGUMENT.  No workspace,
+ * no allocation, no synchronisation. */
+int ccvpe_pose_labels(const double* poses, int B, int H, int W, double sigma, int n_bins, float* gt, float* pyramid,
+                      float* bin_weights, float* ori_vec, void* stream);
+
 /* Backward of the ground descriptor heads (models.py:57-97, 152-157); arguments as ccvpe_grd_descriptors plus the incoming
  * dg[l] fp32 [B, W*c[l]].  Outputs: dfeat fp32 [B, K, H, W] contiguous (NCHW), dw1[l] [c, K], db1[l] [c], dw2[l] [H],
  * db2[l] [1].  scratch: fp32, >= 2*n_heads*B*K*W elements. */

@@ -1,15 +1,21 @@
-"""Dense vs compact training labels for the CVM_VIGOR training step.
+"""Dense vs compact vs pose training labels for the CVM_VIGOR training step.
 
 Dense labels are the three maps per pair (gt, gt_with_ori [20, 512, 512], gt_orientation [2, 512, 512]) fed to
-`losses.training_loss`; compact labels are (gt, bin_weights [20], ori_vec [2]) fed to `losses.training_loss_from_labels`.
-Both give the same loss and gradients.  The two arms alternate within one run, so they see the same machine state.
+`losses.training_loss`; compact labels are (gt, bin_weights [20], ori_vec [2]) fed to `losses.training_loss_from_labels`;
+pose labels are the pair's (row, col, angle) fed to `losses.training_loss_from_poses`, which builds gt, its pyramid and
+the orientation labels on the device.  Dense and compact give the same loss and gradients; the pose arm evaluates the
+Gaussian in float64 rather than the host's float32, so its labels differ in the last bits.  All arms are drawn from the
+same seeds (same label statistics) and alternate within one run, so they see the same machine state.
 
-  (a) loss stage: forward + backward of the loss alone on CVM_VIGOR B=8 bf16 outputs, CUDA events over --iters
-      iterations per round (the 168 MB gt_with_ori of the dense arm does not fit the 126 MB L2)
+  (a) loss stage: forward + backward of the loss alone (the pose arm includes building its labels) on CVM_VIGOR B=8
+      bf16 outputs, CUDA events over --iters iterations per round (the 168 MB gt_with_ori of the dense arm does not fit
+      the 126 MB L2); and the pose-label launch alone at B=8 and B=64, graph-timed, cycling through enough output
+      buffers to write more than twice the L2 per cycle, with its share of the HBM peak from the bytes it writes
   (b) end to end: one `training.GraphedTrainStep` per arm fed from pinned host buffers, double buffered as in
       bench_train.py (images + labels copied every step); pairs/s, H2D bytes per step and the copy time of one step's
       inputs alone.  Under torchrun: one process per GPU, 8 pairs each (weak scaling), bucketed gradient all-reduce.
-  (c) host cost per pair of building the labels on one CPU core: the dense maps vs gt + orientation_labels.
+  (c) host cost per pair of building the labels on one CPU core: the dense maps vs gt + orientation_labels vs drawing
+      the pose alone.
 
     python scripts/bench_train_labels.py --out DIR            # one GPU
     torchrun --nproc-per-node 8 scripts/bench_train_labels.py --out DIR --skip-loss --skip-host
@@ -32,12 +38,16 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-from ccvpe_b200 import losses, models  # noqa: E402
+from ccvpe_b200 import cabi, losses, models  # noqa: E402
 from ccvpe_b200.ddp import GradientAllReducer  # noqa: E402
-from ccvpe_b200.synthetic import fill_deterministic, synthetic_ground_truth, synthetic_labels, synthetic_pair  # noqa: E402
+from ccvpe_b200.synthetic import (fill_deterministic, synthetic_ground_truth, synthetic_labels, synthetic_pair,  # noqa: E402
+                                  synthetic_poses)
 from ccvpe_b200.training import GraphedTrainStep  # noqa: E402
 
 GROUND = (320, 640)
+HBM_PEAK_GBS = 6553.9                   # BASELINE.md (MEASURED_PEAKS.json)
+L2_BYTES = 126e6
+ARMS = ("dense", "compact", "poses")
 
 
 def card():
@@ -62,6 +72,42 @@ def compact_labels(B, seed):
     return [gt, *losses.orientation_labels(angles)]
 
 
+def pose_labels(B, seed):
+    return [synthetic_poses(B, seed=seed)]
+
+
+def label_launch(B, dev, iters, n_bins=20, size=512):
+    """ccvpe_pose_labels alone, captured in a CUDA graph (the events time the kernels, not the enqueue)."""
+    poses = synthetic_poses(B, seed=3).to(dev)
+    written = 4 * (B * size * size + cabi.gt_pyramid_elems(B, size, size) + B * n_bins + 2 * B)
+    n_sets = max(3, -(-int(2 * L2_BYTES) // written))
+    sets = [(torch.empty(B, 1, size, size, device=dev), torch.empty(cabi.gt_pyramid_elems(B, size, size), device=dev),
+             torch.empty(B, n_bins, device=dev), torch.empty(B, 2, device=dev)) for _ in range(n_sets)]
+    for o in sets:
+        cabi.pose_labels(poses, 4.0, n_bins, *o)
+    torch.cuda.synchronize()
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        for i in range(iters):
+            cabi.pose_labels(poses, 4.0, n_bins, *sets[i % n_sets])
+    graph.replay()
+    torch.cuda.synchronize()
+    ms = []
+    for _ in range(5):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        graph.replay()
+        e1.record()
+        torch.cuda.synchronize()
+        ms.append(e0.elapsed_time(e1) / iters)
+    t = statistics.median(ms)
+    return {"batch": B, "us_per_launch_median": round(t * 1e3, 2), "us_per_launch_min": round(min(ms) * 1e3, 2),
+            "bytes_written": written, "bytes_read": 24 * B, "output_sets_cycled": n_sets,
+            "gb_per_s_written": round(written / t / 1e6, 1), "share_of_hbm_peak": round(written / t / 1e6 / HBM_PEAK_GBS, 3),
+            "note": "gt + pyramid + bin weights + vectors written once per launch; median of 5 graph replays of %d "
+                    "launches; share of the %.1f GB/s HBM peak from the bytes written" % (iters, HBM_PEAK_GBS)}
+
+
 def loss_stage(model, B, dev, rounds, iters):
     grd, sat = (t.to(dev) for t in synthetic_pair(B, GROUND, seed=5))
     with torch.no_grad():
@@ -70,7 +116,9 @@ def loss_stage(model, B, dev, rounds, iters):
     wrt = [leaves[0], leaves[2]] + leaves[3:9]
     dense = [t.to(dev) for t in dense_labels(B, 1)]
     compact = [t.to(dev) for t in compact_labels(B, 1)]
-    arms = {"dense": lambda: losses.training_loss(leaves, *dense), "compact": lambda: losses.training_loss_from_labels(leaves, *compact)}
+    poses = [t.to(dev) for t in pose_labels(B, 1)]
+    arms = {"dense": lambda: losses.training_loss(leaves, *dense), "compact": lambda: losses.training_loss_from_labels(leaves, *compact),
+            "poses": lambda: losses.training_loss_from_poses(leaves, *poses)}
     vals = {}
     for name, f in arms.items():
         for _ in range(5):
@@ -92,9 +140,11 @@ def loss_stage(model, B, dev, rounds, iters):
     res = {k: {"ms_median": round(statistics.median(v), 4), "ms_min": round(min(v), 4), "ms_max": round(max(v), 4)}
            for k, v in ms.items()}
     res.update(batch=B, precision="bf16", rounds=rounds, iters_per_round=iters, identical_loss_and_grad_sums=same,
-               label_bytes_on_device={"dense": nbytes(dense), "compact": nbytes(compact)},
-               note="forward + backward (torch.autograd.grad) of the loss alone on fixed CVM_VIGOR outputs; median over "
-                    "rounds of the mean per iteration; the arms alternate every round")
+               loss={k: v[0] for k, v in vals.items()},
+               label_bytes_copied={"dense": nbytes(dense), "compact": nbytes(compact), "poses": nbytes(poses)},
+               note="forward + backward (torch.autograd.grad) of the loss alone on fixed CVM_VIGOR outputs (the pose arm "
+                    "builds its labels too); median over rounds of the mean per iteration; the arms alternate every round; "
+                    "identical_loss_and_grad_sums compares dense and compact")
     return res
 
 
@@ -117,7 +167,8 @@ def e2e(model, B, dev, rank, world, rounds, steps):
     imgs = list(synthetic_pair(B, GROUND, seed=200 + rank))
     arms = {}
     for name, labels, fn in (("dense", dense_labels(B, 200 + rank), losses.training_loss),
-                             ("compact", compact_labels(B, 200 + rank), losses.training_loss_from_labels)):
+                             ("compact", compact_labels(B, 200 + rank), losses.training_loss_from_labels),
+                             ("poses", pose_labels(B, 200 + rank), losses.training_loss_from_poses)):
         host = [t.pin_memory() for t in imgs + labels]
         resident = [t.to(dev) for t in host]
         resident[0] = resident[0].contiguous(memory_format=torch.channels_last)
@@ -187,9 +238,9 @@ def e2e(model, B, dev, rank, world, rounds, steps):
         torch.cuda.synchronize()
         copy_ms[name] = c0.elapsed_time(c1) / 10
     if world > 1:
-        t = torch.tensor([statistics.median(ms["dense"]), statistics.median(ms["compact"])], dtype=torch.float64, device=dev)
+        t = torch.tensor([statistics.median(ms[k]) for k in ARMS], dtype=torch.float64, device=dev)
         torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
-        med = dict(zip(("dense", "compact"), t.tolist()))
+        med = dict(zip(ARMS, t.tolist()))
     else:
         med = {k: statistics.median(v) for k, v in ms.items()}
     res = {}
@@ -208,7 +259,8 @@ def e2e(model, B, dev, rank, world, rounds, steps):
 def host_cost(B, reps):
     torch.set_num_threads(1)
     arms = {"dense": lambda s: synthetic_ground_truth(B, seed=s),
-            "compact": lambda s: (lambda gt, a: (gt, losses.orientation_labels(a)))(*synthetic_labels(B, seed=s))}
+            "compact": lambda s: (lambda gt, a: (gt, losses.orientation_labels(a)))(*synthetic_labels(B, seed=s)),
+            "poses": lambda s: synthetic_poses(B, seed=s)}
     ms = {k: [] for k in arms}
     for r in range(reps):
         for name, f in arms.items():
@@ -217,8 +269,8 @@ def host_cost(B, reps):
             ms[name].append((time.perf_counter() - t0) * 1e3 / B)
     return {k: {"ms_per_pair_median": round(statistics.median(v), 3), "ms_per_pair_min": round(min(v), 3)} for k, v in ms.items()} | {
         "batch": B, "reps": reps, "threads": 1, "host_cores": os.cpu_count(),
-        "note": "synthetic_ground_truth (the Gaussian and the dense maps) vs synthetic_labels + orientation_labels, one "
-                "torch thread; both include drawing the Gaussian"}
+        "note": "synthetic_ground_truth (the Gaussian and the dense maps) vs synthetic_labels + orientation_labels vs "
+                "synthetic_poses (drawing the pose only: the labels are built on the device), one torch thread"}
 
 
 def main():
@@ -232,6 +284,7 @@ def main():
     ap.add_argument("--host-reps", type=int, default=5)
     ap.add_argument("--skip-loss", action="store_true")
     ap.add_argument("--skip-host", action="store_true")
+    ap.add_argument("--label-iters", type=int, default=200)
     args = ap.parse_args()
     if not torch.cuda.is_available():
         raise SystemExit("bench_train_labels.py needs a CUDA device")
@@ -248,6 +301,7 @@ def main():
     res = {"card": card(), "torch": torch.__version__}
     if rank == 0 and not args.skip_loss:
         res["a_loss_stage"] = loss_stage(model, args.batch, dev, args.loss_rounds, args.loss_iters)
+        res["a_pose_label_launch"] = [label_launch(b, dev, args.label_iters) for b in (args.batch, 64)]
     res["b_end_to_end"] = e2e(model, args.batch, dev, rank, world, args.e2e_rounds, args.e2e_steps)
     if rank == 0 and not args.skip_host:
         res["c_host_cost"] = host_cost(args.batch, args.host_reps)
