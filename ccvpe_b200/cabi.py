@@ -24,7 +24,7 @@ EXPORTED_SYMBOLS = (
     "ccvpe_abi_version", "ccvpe_last_error", "ccvpe_launch_count", "ccvpe_reset_launch_count",
     "ccvpe_grd_descriptor", "ccvpe_grd_descriptors", "ccvpe_igemm", "ccvpe_igemm_plan", "ccvpe_match_scratch_elems", "ccvpe_match_plan", "ccvpe_match_level",
     "ccvpe_softmax_scratch_elems", "ccvpe_softmax_heatmap", "ccvpe_ori_normalize",
-    "ccvpe_pose_scratch_bytes", "ccvpe_pose_decode", "ccvpe_bias_silu_nhwc", "ccvpe_dwconv_bias_silu_nhwc",
+    "ccvpe_pose_scratch_bytes", "ccvpe_pose_decode", "ccvpe_bias_silu_nhwc", "ccvpe_dwconv_bias_silu_nhwc", "ccvpe_dwconv_plan",
     "ccvpe_pointwise_silu_nhwc", "ccvpe_stem_conv_silu_nhwc", "ccvpe_se_gate_scale", "ccvpe_mbconv_project_nhwc",
     "ccvpe_wrap_columns_nhwc",
     "ccvpe_ingest_u8", "ccvpe_resize_u8", "ccvpe_affine_u8", "ccvpe_stem_conv_silu_u8_nhwc",
@@ -137,6 +137,8 @@ def load() -> C.CDLL:
     lib.ccvpe_dwconv_bias_silu_nhwc.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_void_p]
+    lib.ccvpe_dwconv_plan.restype = C.c_int
+    lib.ccvpe_dwconv_plan.argtypes = [C.c_int] * 6
     lib.ccvpe_pointwise_silu_nhwc.restype = C.c_int
     lib.ccvpe_pointwise_silu_nhwc.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                               C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
@@ -424,6 +426,17 @@ def dwconv_bias_silu_nhwc(x_pad: torch.Tensor, w: torch.Tensor, bias: torch.Tens
     _check(load().ccvpe_dwconv_bias_silu_nhwc(_ptr(x_pad), x_pad.stride(0), x_pad.stride(1), x_pad.stride(2), Hp, Wp,
                                               _ptr(w), _ptr(bias), _ptr(y), B, Cc, k, stride, _ptr(chan_sum), _stream()),
            "ccvpe_dwconv_bias_silu_nhwc")
+
+
+DWCONV_KERNELS = ("dwconv_bias_silu_kernel", "dwconv_tile_kernel")
+
+
+def dwconv_kernel_name(B: int, C: int, Hp: int, Wp: int, k: int, stride: int) -> str:
+    """Which kernel `dwconv_bias_silu_nhwc` launches for a [B, Hp, Wp, C] padded input (tests / bench attribution)."""
+    rc = load().ccvpe_dwconv_plan(B, C, Hp, Wp, k, stride)
+    if rc < 0:
+        _check(rc, "ccvpe_dwconv_plan")
+    return DWCONV_KERNELS[rc]
 
 
 def pad_k_blocks(w: torch.Tensor) -> torch.Tensor:

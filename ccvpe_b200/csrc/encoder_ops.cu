@@ -531,6 +531,21 @@ static bool dwt_plan(int K, int Ho, int Wo, int C, int B, DwTileParams* p) {
   return true;
 }
 
+// The depthwise dispatch, shared by the launch and by ccvpe_dwconv_plan so that the two cannot disagree: checks the shape,
+// then returns 1 for dwconv_tile_kernel (its plan in *tp), 0 for dwconv_bias_silu_kernel, < 0 on a bad argument.
+// Measured per layer (B=64, scripts/bench_dwconv.py): the tiled kernel wins wherever the window is 5x5 (1.2-1.5x) and for
+// the deep 3x3 layers (>= 240 channels); the shallow 3x3 layers (32 / 144 channels on large images) stay on the streaming
+// kernel.  CCVPE_DW_TILED = 0 / 2 forces streaming / tiled (development switch).
+static int dw_select(int B, int C, int Hp, int Wp, int K, int S, DwTileParams* tp) {
+  CCVPE_REQUIRE(B > 0 && C > 0 && C % 8 == 0 && C <= 2048, "ccvpe_dwconv_bias_silu_nhwc: bad shape B=%d C=%d", B, C);
+  CCVPE_REQUIRE((K == 3 || K == 5) && (S == 1 || S == 2) && Hp >= K && Wp >= K, "ccvpe_dwconv_bias_silu_nhwc: K=%d S=%d Hp=%d Wp=%d unsupported", K, S, Hp, Wp);
+  const int Ho = (Hp - K) / S + 1, Wo = (Wp - K) / S + 1;
+  static const int use_tiled = getenv("CCVPE_DW_TILED") ? atoi(getenv("CCVPE_DW_TILED")) : 1;
+  memset(tp, 0, sizeof(*tp));
+  if (S == 1 && (use_tiled == 2 || (use_tiled == 1 && (K == 5 || C >= 240))) && dwt_plan(K, Ho, Wo, C, B, tp)) return 1;
+  return 0;
+}
+
 // ---------------------------------------------------------------------------------------------------------------------
 // Encoder stem: see stem_tcgen05.cu (3x3 stride-2 convolution over the planar fp32 / uint8 image as an implicit GEMM on the
 // tensor cores + folded-BN bias + SiLU, written as bf16 channels-last into the interior of the first depthwise
@@ -832,37 +847,30 @@ extern "C" int ccvpe_dwconv_bias_silu_nhwc(const void* x, int64_t x_sb, int64_t 
                                            int64_t* chan_sum, void* stream) {
   using namespace ccvpe;
   CCVPE_REQUIRE(x && w && bias && y, "ccvpe_dwconv_bias_silu_nhwc: null pointer");
-  CCVPE_REQUIRE(B > 0 && C > 0 && C % 8 == 0 && C <= 2048, "ccvpe_dwconv_bias_silu_nhwc: bad shape B=%d C=%d", B, C);
-  CCVPE_REQUIRE((K == 3 || K == 5) && (S == 1 || S == 2) && Hp >= K && Wp >= K, "ccvpe_dwconv_bias_silu_nhwc: K=%d S=%d Hp=%d Wp=%d unsupported", K, S, Hp, Wp);
+  DwTileParams tp;
+  const int kernel = dw_select(B, C, Hp, Wp, K, S, &tp);
+  if (kernel < 0) return kernel;
   CCVPE_REQUIRE(aligned16(x) && aligned16(w) && aligned16(bias) && aligned16(y), "ccvpe_dwconv_bias_silu_nhwc: pointers must be 16-byte aligned");
   CCVPE_REQUIRE(x_sb % 8 == 0 && x_sh % 8 == 0 && x_sw % 8 == 0, "ccvpe_dwconv_bias_silu_nhwc: input strides must be multiples of 8");
   CCVPE_REQUIRE(x_sw > 0 && x_sw * 16 < (1LL << 31), "ccvpe_dwconv_bias_silu_nhwc: pixel stride out of range");
   const int Ho = (Hp - K) / S + 1, Wo = (Wp - K) / S + 1;
-  // Measured per layer (B=64, scripts/bench_dwconv.py): the tiled kernel wins wherever the window is 5x5 (1.2-1.5x) and
-  // for the deep 3x3 layers (>= 240 channels); the shallow 3x3 layers (32 / 144 channels on large images) stay on the
-  // streaming kernel.  CCVPE_DW_TILED = 0 / 2 forces streaming / tiled (development switch).
-  static const int use_tiled = getenv("CCVPE_DW_TILED") ? atoi(getenv("CCVPE_DW_TILED")) : 1;
-  if (S == 1 && (use_tiled == 2 || (use_tiled == 1 && (K == 5 || C >= 240)))) {
-    DwTileParams tp;
-    memset(&tp, 0, sizeof(tp));
-    if (dwt_plan(K, Ho, Wo, C, B, &tp)) {
-      tp.x = (const __nv_bfloat16*)x; tp.x_sb = x_sb; tp.x_sh = x_sh; tp.x_sw = x_sw; tp.Hp = Hp; tp.Wp = Wp;
-      tp.w = (const __nv_bfloat16*)w; tp.bias = (const __nv_bfloat16*)bias; tp.y = (__nv_bfloat16*)y;
-      tp.Ho = Ho; tp.Wo = Wo; tp.C = C;
-      tp.chan_sum = reinterpret_cast<long long*>(chan_sum);
-      const int smem = DWT_SCRATCH + 2 * tp.stage_bytes;
-      static thread_local uint64_t tiled_attr = 0;
-      if (first_use_on_device(tiled_attr)) {
-        cudaFuncSetAttribute(dwconv_tile_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, DWT_SCRATCH + 2 * DWT_STAGE_LIMIT);
-        cudaFuncSetAttribute(dwconv_tile_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, DWT_SCRATCH + 2 * DWT_STAGE_LIMIT);
-      }
-      const int max_grid = 2 * sm_count();
-      const int grid = tp.total_items < max_grid ? tp.total_items : max_grid;
-      if (K == 3) dwconv_tile_kernel<3><<<grid, DWT_THREADS, smem, (cudaStream_t)stream>>>(tp);
-      else dwconv_tile_kernel<5><<<grid, DWT_THREADS, smem, (cudaStream_t)stream>>>(tp);
-      CCVPE_LAUNCH_CHECK("dwconv_tile_kernel");
-      return CCVPE_OK;
+  if (kernel == 1) {
+    tp.x = (const __nv_bfloat16*)x; tp.x_sb = x_sb; tp.x_sh = x_sh; tp.x_sw = x_sw; tp.Hp = Hp; tp.Wp = Wp;
+    tp.w = (const __nv_bfloat16*)w; tp.bias = (const __nv_bfloat16*)bias; tp.y = (__nv_bfloat16*)y;
+    tp.Ho = Ho; tp.Wo = Wo; tp.C = C;
+    tp.chan_sum = reinterpret_cast<long long*>(chan_sum);
+    const int smem = DWT_SCRATCH + 2 * tp.stage_bytes;
+    static thread_local uint64_t tiled_attr = 0;
+    if (first_use_on_device(tiled_attr)) {
+      cudaFuncSetAttribute(dwconv_tile_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, DWT_SCRATCH + 2 * DWT_STAGE_LIMIT);
+      cudaFuncSetAttribute(dwconv_tile_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize, DWT_SCRATCH + 2 * DWT_STAGE_LIMIT);
     }
+    const int max_grid = 2 * sm_count();
+    const int grid = tp.total_items < max_grid ? tp.total_items : max_grid;
+    if (K == 3) dwconv_tile_kernel<3><<<grid, DWT_THREADS, smem, (cudaStream_t)stream>>>(tp);
+    else dwconv_tile_kernel<5><<<grid, DWT_THREADS, smem, (cudaStream_t)stream>>>(tp);
+    CCVPE_LAUNCH_CHECK("dwconv_tile_kernel");
+    return CCVPE_OK;
   }
   // V = channels per thread
   static const int force_v = getenv("CCVPE_DW_V") ? atoi(getenv("CCVPE_DW_V")) : 0;
@@ -919,4 +927,9 @@ extern "C" int ccvpe_dwconv_bias_silu_nhwc(const void* x, int64_t x_sb, int64_t 
 #undef CCVPE_DW
   CCVPE_LAUNCH_CHECK("dwconv_bias_silu_kernel");
   return CCVPE_OK;
+}
+
+extern "C" int ccvpe_dwconv_plan(int B, int C, int Hp, int Wp, int K, int S) {
+  ccvpe::DwTileParams tp;
+  return ccvpe::dw_select(B, C, Hp, Wp, K, S, &tp);
 }

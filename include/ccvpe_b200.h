@@ -181,6 +181,9 @@ int ccvpe_bias_silu_nhwc(const void* x, const void* bias, void* y, int64_t y_sb,
 int ccvpe_dwconv_bias_silu_nhwc(const void* x, int64_t x_sb, int64_t x_sh, int64_t x_sw, int Hp, int Wp,
                                 const void* w, const void* bias, void* y, int B, int C, int K, int S,
                                 int64_t* chan_sum, void* stream);
+/* which kernel ccvpe_dwconv_bias_silu_nhwc would launch for this layer (the launch makes the same choice, environment
+ * switches included): 0 = dwconv_bias_silu_kernel, 1 = dwconv_tile_kernel; < 0 = error. */
+int ccvpe_dwconv_plan(int B, int C, int Hp, int Wp, int K, int S);
 
 /* Encoder stem (reference efficientnet_pytorch/model.py:296-297 in eval mode, BN folded; circular variant: the reference's
  * models.py circular-padding patch of the ground encoder): 3x3 stride-2 conv over the fp32 NCHW image with the reference's

@@ -84,3 +84,84 @@ def check_against_golden(outputs, golden, tol, loose=None):
         s_ref, as_ref = float(golden[name + ".sum"]), float(golden[name + ".abssum"])
         assert abs(flat.astype(np.float64).sum() - s_ref) <= tol * max(as_ref, 1e-30), name + " checksum"
     return worst
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# per-element bounds and guarded replays of the plan checks (tests/test_gpu_plan_parity.py, tests/test_gpu_encoder_plan.py)
+# ---------------------------------------------------------------------------------------------------------------------
+RHO_BF16 = 2.0 ** -8        # bound on the relative error of one bf16 store (its unit roundoff is 2^-9)
+TINY = 2.0 ** -126          # smallest normal fp32 / bf16 magnitude
+
+
+def subnormal_floor(t1):
+    """Absolute allowance for flush-to-zero.  The tensor cores flush subnormal operands, products and partial sums: a term
+    a*w of an output loses at most TINY * (|a| + |w| + 2) <= 2 TINY (|a| + 1)(|w| + 1); `t1` is that sum over the output's
+    terms.  Without it, gradients that decay into the subnormal range (the orientation loss is a Gaussian blob, so its
+    data gradients are ~1e-40 far from the blob) fail the relative bound although they are zero to within 1e-38.  The
+    floor stays below 1e-30 for every shape here, far under any value the bound is meant to resolve."""
+    return 2 * TINY * t1
+
+
+def bound_check(got, ref, S, rho, tau, floor=0.0):
+    """Returns (worst |got - ref| / (rho |ref| + tau S + floor), worst (|got - ref| - rho |ref| - floor) / S = the tau this
+    tensor needs).  Where the bound is zero the element must be exact; a non-finite output where the reference is finite
+    fails."""
+    got, ref, S = got.to(torch.float64).reshape(-1), ref.to(torch.float64).reshape(-1), S.to(torch.float64).reshape(-1)
+    if torch.is_tensor(floor):
+        floor = floor.to(torch.float64).reshape(-1)
+    d = (got - ref).abs()
+    d = torch.where(torch.isfinite(d), d, torch.full_like(d, float("inf")))
+    bound = rho * ref.abs() + tau * S + floor
+    ratio = torch.where(bound > 0, d / bound.clamp_min(1e-300), torch.where(d > 0, float("inf"), 0.0))
+    excess = (d - rho * ref.abs() - floor).clamp_min(0.0)
+    need = torch.where(S > 0, excess / S.clamp_min(1e-300), torch.where(excess > 0, float("inf"), 0.0))
+    return (float(ratio.max()) if ratio.numel() else 0.0), (float(need.max()) if need.numel() else 0.0)
+
+
+def image_subset(B):
+    """Images whose outputs are checked for the per-image operators: all of them up to 8, else 0, 1, B/2 and B-1."""
+    return list(range(B)) if B <= 8 else sorted({0, 1, B // 2, B - 1})
+
+
+SENTINEL = {torch.bfloat16: (torch.int16, -1), torch.float32: (torch.int32, -1)}    # all-ones bits: a NaN no kernel writes
+
+
+def sentinel_bits(t):
+    ity, _ = SENTINEL[t.dtype]
+    return t.view(ity)
+
+
+def guarded(n, dtype, guard, dev):
+    """A sentinel-filled buffer of guard + n + guard elements; the output is buf[guard:guard + n]."""
+    buf = torch.empty(guard + n + guard, dtype=dtype, device=dev)
+    sentinel_bits(buf).fill_(SENTINEL[dtype][1])
+    return buf
+
+
+def guard_report(buf, n, guard, ref_out, written=None):
+    """Problems of a replay into `guarded(n, ...)`: writes into the guards, output elements left unwritten, and output
+    elements that differ from the plan's own output `ref_out`.  `written` (bool, shaped like ref_out): the elements the
+    launch must write; the others must still hold the sentinel.  None = every element."""
+    s = SENTINEL[buf.dtype][1]
+    bits = sentinel_bits(buf)
+    problems = []
+    if not bool((bits[:guard] == s).all()):
+        problems.append("wrote %d elements before the output" % int((bits[:guard] != s).sum()))
+    if not bool((bits[guard + n:] == s).all()):
+        problems.append("wrote %d elements past the output" % int((bits[guard + n:] != s).sum()))
+    inner = bits[guard:guard + n]
+    want = sentinel_bits(ref_out.reshape(-1))
+    if written is not None:
+        mask = written.reshape(-1)
+        if not bool((inner[~mask] == s).all()):
+            problems.append("wrote %d elements outside the ones it owns" % int((inner[~mask] != s).sum()))
+        inner, want = inner[mask], want[mask]
+    if bool((inner == s).any()):
+        problems.append("left %d output elements unwritten" % int((inner == s).sum()))
+    if not torch.equal(inner, want):
+        problems.append("replay differs from the plan's output in %d elements" % int((inner != want).sum()))
+    return problems
+
+
+def guard_len(row):
+    return (128 * row + 4096 + 511) // 512 * 512          # >= one 128-row tile; keeps the interior 1 KB aligned

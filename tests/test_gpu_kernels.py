@@ -11,8 +11,11 @@ from torch.nn import functional as F
 
 from ccvpe_b200 import cabi
 from ccvpe_b200.decoder import decode_pose
-from helpers import rel_err
+from helpers import RHO_BF16, bound_check, rel_err
 from oracle import ccvpe_oracle as orc
+from test_gpu_encoder_plan import (TAU, TAU_GATE, TAU_SUM, act_check, dwconv_reference, pointwise_reference,
+                                   project_reference, se_gate_reference, se_sum_conversions, se_sum_reference, stem_operand,
+                                   stem_reference)
 
 pytestmark = pytest.mark.gpu
 
@@ -532,7 +535,8 @@ def test_grd_descriptors_all_heads(cuda_device, B, H, W, cs, layout, dtype):
                                          (2, 64, 64, 32, 3, 1), (1, 40, 80, 144, 5, 1), (2, 20, 40, 672, 5, 1),
                                          (1, 50, 70, 8, 5, 1), (2, 10, 20, 1152, 3, 1)])
 def test_dwconv_bias_silu_nhwc(cuda_device, B, H, W, C, K, S):
-    """fused depthwise conv + bias + SiLU + SE channel sums over a pre-padded buffer vs torch (fp32 math on bf16 data)."""
+    """fused depthwise conv + bias + SiLU + SE channel sums over a pre-padded buffer vs the float64 reference of
+    test_gpu_encoder_plan.py, element by element (y: the activated bound; sums: the fixed-point sum bound)."""
     g = _gen(15)
     dev = cuda_device
     lo = (K - S) // 2 if S == 2 else (K - 1) // 2
@@ -551,29 +555,36 @@ def test_dwconv_bias_silu_nhwc(cuda_device, B, H, W, C, K, S):
     again = torch.zeros_like(sums)
     cabi.dwconv_bias_silu_nhwc(buf, w.reshape(C, K * K).t().contiguous().to(dev), bias.to(dev), y, K, S, again)
     assert torch.equal(sums, again)                      # fixed-point accumulation: order independent, bit-reproducible
-    sums = sums.double() / cabi.SE_SUM_SCALE
     torch.cuda.synchronize()
-    assert rel_err(y.float(), ref) < 1e-2
-    assert rel_err(sums, y.float().sum(dim=(1, 2))) < 1e-4
+    y, sums = y.cpu(), sums.cpu().double() / cabi.SE_SUM_SCALE
+    w_taps = w.reshape(C, K * K).t().contiguous()
+    a_ref, S_a, floor = dwconv_reference(x, w_taps, bias, K, S, lo, hi, False)
+    assert tuple(a_ref.shape) == tuple(ref.shape)
+    ratio = act_check(y, a_ref, S_a, floor, TAU["dwconv"])[0]
+    assert ratio <= 1.0, ratio
+    ref_s, S_s, floor_s = se_sum_reference(y, se_sum_conversions(*y.shape[1:3]))
+    ratio = bound_check(sums, ref_s, S_s, 0.0, TAU_SUM, floor_s)[0]
+    assert ratio <= 1.0, ratio
 
 
 @pytest.mark.parametrize("B,H,W,K,N,lo,hi", [(2, 20, 36, 16, 96, 0, 1), (1, 33, 17, 24, 144, 1, 1), (3, 16, 16, 40, 240, 2, 2),
                                             (2, 10, 20, 112, 672, 2, 2), (1, 16, 16, 192, 1152, 1, 1),
                                             (2, 10, 20, 320, 1280, 0, 0), (1, 5, 7, 80, 480, 1, 2)])
 def test_pointwise_silu_nhwc(cuda_device, B, H, W, K, N, lo, hi):
-    """tcgen05 1x1 conv + bias + SiLU written into the interior of a padded image vs torch (fp32 math on bf16 data);
-    the border of the image must be left untouched."""
+    """tcgen05 1x1 conv + bias + SiLU written into the interior of a padded image vs the float64 reference of
+    test_gpu_encoder_plan.py, element by element; the border of the image must be left untouched."""
     g = _gen(16)
     dev = cuda_device
     x = torch.randn(B, H, W, K, generator=g).to(torch.bfloat16)
     w = (torch.randn(N, K, generator=g) / math.sqrt(K) * 2.0).to(torch.bfloat16)
     bias = torch.randn(N, generator=g)
-    ref = F.silu(x.float() @ w.float().t() + bias)
     out = torch.full((B, H + lo + hi, W + lo + hi, N), 7.0, device=dev, dtype=torch.bfloat16)
-    cabi.pointwise_silu_nhwc(x.to(dev), cabi.pad_k_blocks(w.to(dev)), bias.to(dev), out, lo, hi)
+    w_nk = cabi.pad_k_blocks(w.to(dev))
+    cabi.pointwise_silu_nhwc(x.to(dev), w_nk, bias.to(dev), out, lo, hi)
     torch.cuda.synchronize()
-    got = out[:, lo:lo + H, lo:lo + W, :].float()
-    assert rel_err(got, ref) < 1e-2
+    got = out[:, lo:lo + H, lo:lo + W, :].cpu()
+    ratio = act_check(got, *pointwise_reference(x, w_nk.cpu(), bias), TAU["pointwise"])[0]
+    assert ratio <= 1.0, ratio
     border = out.clone()
     border[:, lo:lo + H, lo:lo + W, :] = 7.0
     assert bool((border == 7.0).all())
@@ -582,7 +593,8 @@ def test_pointwise_silu_nhwc(cuda_device, B, H, W, K, N, lo, hi):
 @pytest.mark.parametrize("B,H,W,circ,olo,ohi", [(2, 64, 96, False, 1, 1), (2, 40, 72, True, 1, 1), (1, 31, 45, False, 0, 2),
                                                (3, 16, 20, True, 2, 1)])
 def test_stem_conv_silu_nhwc(cuda_device, B, H, W, circ, olo, ohi):
-    """fused stem (3x3 s2 conv from the fp32 NCHW image + bias + SiLU -> padded bf16 NHWC, wrap columns) vs torch."""
+    """fused stem (3x3 s2 conv from the fp32 NCHW image + bias + SiLU -> padded bf16 NHWC, wrap columns) vs the float64
+    reference of test_gpu_encoder_plan.py, element by element."""
     g = _gen(17)
     dev = cuda_device
     x = torch.randn(B, 3, H, W, generator=g)
@@ -597,7 +609,10 @@ def test_stem_conv_silu_nhwc(cuda_device, B, H, W, circ, olo, ohi):
                              lo, hi, olo, ohi, circ)
     torch.cuda.synchronize()
     got = out.float().cpu()
-    assert rel_err(got[:, olo:olo + Ho, olo:olo + Wo, :], ref) < 1e-2
+    w_taps = w.permute(1, 2, 3, 0).reshape(27, 32)
+    ratio = act_check(got[:, olo:olo + Ho, olo:olo + Wo, :], *stem_reference(stem_operand(x), w_taps, bias, lo, hi, circ),
+                      TAU["stem"])[0]
+    assert ratio <= 1.0, ratio
     assert bool((got[:, :olo] == 0).all()) and bool((got[:, olo + Ho:] == 0).all())          # zero rows untouched
     if circ:
         if olo:
@@ -614,32 +629,34 @@ def test_stem_conv_silu_nhwc(cuda_device, B, H, W, circ, olo, ohi):
                                                  (2, 1152, 48, 320, True, 1), (3, 96, 4, 24, True, 1), (3, 32, 8, 16, True, 2),
                                                  (2, 48, 4, 8, True, 4)])
 def test_se_gate_scale(cuda_device, B, mid, R, cout, ws, rep):
-    """fused squeeze-excite gate + projection-weight scaling vs torch (fp32 math on bf16 parameters)."""
+    """fused squeeze-excite gate + projection-weight scaling vs the float64 reference of test_gpu_encoder_plan.py (from the
+    int64 sums as stored), element by element."""
     g = _gen(18)
     dev = cuda_device
     hw = 77
     sums_fixed = (torch.randn(B, mid, generator=g) * hw * 0.5 * cabi.SE_SUM_SCALE).round().to(torch.int64)
-    sums = (sums_fixed.double() / cabi.SE_SUM_SCALE).float()
     w_red = (torch.randn(R, mid, generator=g) / math.sqrt(mid)).to(torch.bfloat16)
     b_red = torch.randn(R, generator=g).to(torch.bfloat16)
     w_se = (torch.randn(mid, R, generator=g) / math.sqrt(R)).to(torch.bfloat16)
     b_se = torch.randn(mid, generator=g).to(torch.bfloat16)
     w_proj = torch.randn(cout, mid, generator=g).to(torch.bfloat16)
-    mean = sums / hw
-    h = F.silu(mean @ w_red.float().t() + b_red.float())
-    gate = torch.sigmoid(h @ w_se.float().t() + b_se.float())
-    ref1 = w_proj.float().unsqueeze(0) * gate.unsqueeze(1)
-    ref = torch.zeros(B, rep * cout, rep * mid)
+    diagonal = torch.zeros(B, rep * cout, rep * mid, dtype=torch.bool)
     for r in range(rep):
-        ref[:, r * cout:(r + 1) * cout, r * mid:(r + 1) * mid] = ref1
+        diagonal[:, r * cout:(r + 1) * cout, r * mid:(r + 1) * mid] = True
     wg = torch.full((B, rep * cout, rep * mid), 7.0, device=dev, dtype=torch.bfloat16)
     gate_ws = torch.empty(B, mid, device=dev, dtype=torch.float32) if ws else None
     cabi.se_gate_scale(sums_fixed.to(dev), 1.0 / hw, w_red.to(dev), b_red.to(dev), w_se.t().contiguous().to(dev), b_se.to(dev),
                        w_proj.to(dev), wg, gate_ws, rep)
     torch.cuda.synchronize()
-    assert rel_err(wg.float().cpu(), ref) < 1e-2
+    _, wg_ref = se_gate_reference(sums_fixed, hw, w_red, b_red, w_se.t(), b_se, w_proj)
+    S = w_proj.double().abs().unsqueeze(0).expand_as(wg_ref)
+    got = wg.cpu()
+    for r in range(rep):                            # every diagonal block element by element
+        blk = got[:, r * cout:(r + 1) * cout, r * mid:(r + 1) * mid]
+        ratio = bound_check(blk, wg_ref, S, RHO_BF16, TAU_GATE)[0]
+        assert ratio <= 1.0, (r, ratio)
     if rep > 1:                                     # off-diagonal blocks are exact zeros
-        assert bool((wg.float().cpu()[ref == 0] == 0).all())
+        assert bool((got[~diagonal] == 0).all())
 
 
 @pytest.mark.parametrize("B,HW,mid,cout,res,biased", [
@@ -653,22 +670,21 @@ def test_se_gate_scale(cuda_device, B, mid, R, cout, ws, rep):
     (160, 50, 96, 16, True, False),     # more work items than SMs: persistent loop + accumulator double buffering
 ])
 def test_mbconv_project_nhwc(cuda_device, B, HW, mid, cout, res, biased):
-    """batched per-image-weight projection GEMM (+ residual, + biased copy) on tcgen05 vs torch (fp32 math on bf16 data);
-    the biased copy must be exactly bf16(out) + bias as torch computes it."""
+    """batched per-image-weight projection GEMM (+ residual, + biased copy) on tcgen05 vs the float64 reference of
+    test_gpu_encoder_plan.py, element by element; the biased copy must be exactly bf16(out) + bias as torch computes it."""
     g = _gen(23)
     dev = cuda_device
     d = torch.randn(B, HW, mid, generator=g).to(torch.bfloat16)
     wg = (torch.randn(B, cout, mid, generator=g) / math.sqrt(mid)).to(torch.bfloat16)
     r = torch.randn(B, HW, cout, generator=g).to(torch.bfloat16) if res else None
     bias = torch.randn(cout, generator=g).to(torch.bfloat16)
-    ref = torch.bmm(d.float(), wg.float().transpose(1, 2))
-    if res:
-        ref = ref + r.float()
     out = torch.full((B, HW, cout), 7.0, device=dev, dtype=torch.bfloat16)
     out2 = torch.full((B, HW, cout), 7.0, device=dev, dtype=torch.bfloat16) if biased else None
     cabi.mbconv_project_nhwc(d.to(dev), wg.to(dev), r.to(dev) if res else None, out, bias.to(dev) if biased else None, out2)
     torch.cuda.synchronize()
-    assert rel_err(out.float().cpu(), ref) < 1e-2
+    ref, S, floor = project_reference(d, wg, r)
+    ratio = bound_check(out.cpu(), ref, S, RHO_BF16, TAU["project"], floor)[0]
+    assert ratio <= 1.0, ratio
     if biased:
         assert torch.equal(out2, out + bias.to(dev))
 
@@ -716,8 +732,9 @@ def test_ingest_u8_matches_torchvision_arithmetic(cuda_device, B, H, W, crop, nh
 @pytest.mark.parametrize("B,H,W,crop,circ,rolled", [(2, 32, 64, 64, True, True), (1, 20, 48, 30, False, True),
                                                      (2, 16, 24, 24, False, False)])
 def test_stem_conv_silu_u8_fused_ingest(cuda_device, B, H, W, crop, circ, rolled):
-    """Stem kernel reading uint8 images (ToTensor + Normalize + roll + crop in the loads) == the fp32 stem kernel on the
-    ingested image (the normalisation is one FMA instead of divide-subtract-divide: 1e-2 of max|ref| after bf16 rounding)."""
+    """Stem kernel reading uint8 images (ToTensor + Normalize + roll + crop in the loads) vs the float64 reference of
+    test_gpu_encoder_plan.py on the rolled, cropped, FMA-normalised operand, element by element; and within bf16 noise of
+    the fp32 stem kernel on the ingested image (the normalisation is one FMA instead of divide-subtract-divide)."""
     g = _gen(42)
     dev = cuda_device
     img = torch.randint(0, 256, (B, 3, H, W), generator=g, dtype=torch.uint8).to(dev)
@@ -733,6 +750,10 @@ def test_stem_conv_silu_u8_fused_ingest(cuda_device, B, H, W, crop, circ, rolled
     cabi.stem_conv_silu_u8_nhwc(img, w, bias, got, 0, 1, 1, 1, circ, crop_w=crop, shift=shifts)
     torch.cuda.synchronize()
     assert rel_err(got.float(), ref.float()) < 1e-2
+    v = stem_operand(img.cpu(), None if shifts is None else shifts.cpu(), crop)
+    a_ref, S, floor = stem_reference(v, w.cpu(), bias.cpu(), 0, 1, circ)
+    ratio = act_check(got[:, 1:1 + Ho, 1:1 + Wo].cpu(), a_ref, S, floor, TAU["stem"])[0]
+    assert ratio <= 1.0, ratio
 
 
 @pytest.mark.parametrize("B,C,N,Hout,Wout,backend", [

@@ -32,10 +32,10 @@ from torch.nn import functional as F
 from ccvpe_b200 import cabi
 from ccvpe_b200.decoder import PostEncoderPipeline
 from ccvpe_b200.training import PostEncoderTrainer
+from helpers import RHO_BF16, TINY, bound_check, guard_len, guard_report, guarded, image_subset, subnormal_floor
 from oracle import ccvpe_oracle as orc
 
 F64 = torch.float64
-RHO_BF16 = 2.0 ** -8
 
 #: tau per operator: at least 4x the worst (|got - ref| - rho |ref| - floor) / S measured on a B200 (1000 W power limit)
 #: over every configuration of this file, and never above 1e-4.  Measured worst values:
@@ -48,9 +48,6 @@ TAU = {"igemm": 1e-5, "wgrad": 1e-4, "match": 6e-5, "match_bwd": 1e-5}
 
 #: bf16 launches allowed to resolve to a CUDA-core kernel: {kernel-qualified tag: reason}
 SIMT_ALLOWED = {}
-
-SENTINEL = {torch.bfloat16: (torch.int16, -1), torch.float32: (torch.int32, -1)}    # all-ones bits: a NaN no kernel writes
-
 
 # ---------------------------------------------------------------------------------------------------------------
 # float64 references
@@ -100,18 +97,6 @@ def igemm_reference(a0, c0, a1, c1, geom, w_kn, N, bias=None, row_scale=None, ro
     if relu:
         y = y.clamp_min(0.0)
     return y, s, floor + 4 * TINY                    # (+ the fp32 epilogue's own flushes)
-
-
-TINY = 2.0 ** -126          # smallest normal fp32 / bf16 magnitude
-
-
-def subnormal_floor(t1):
-    """Absolute allowance for flush-to-zero.  The tensor cores flush subnormal operands, products and partial sums: a term
-    a*w of an output loses at most TINY * (|a| + |w| + 2) <= 2 TINY (|a| + 1)(|w| + 1); `t1` is that sum over the output's
-    terms.  Without it, gradients that decay into the subnormal range (the orientation loss is a Gaussian blob, so its
-    data gradients are ~1e-40 far from the blob) fail the relative bound although they are zero to within 1e-38.  The
-    floor stays below 1e-30 for every shape here, far under any value the bound is meant to resolve."""
-    return 2 * TINY * t1
 
 
 def output_as_mn(out, mode, N, ldo, B, Hout, Wout):
@@ -227,81 +212,29 @@ def match_bwd_reference(x, g, offset, shifts, mask, scores, ds, dscl, dmax, dxh)
     return dx, Sdx, dg, Sdg
 
 
-def bound_check(got, ref, S, rho, tau, floor=0.0):
-    """Returns (worst |got - ref| / (rho |ref| + tau S + floor), worst (|got - ref| - rho |ref| - floor) / S = the tau this
-    tensor needs).  Where the bound is zero the element must be exact; a non-finite output where the reference is finite
-    fails."""
-    got, ref, S = got.to(F64).reshape(-1), ref.to(F64).reshape(-1), S.to(F64).reshape(-1)
-    if torch.is_tensor(floor):
-        floor = floor.to(F64).reshape(-1)
-    d = (got - ref).abs()
-    d = torch.where(torch.isfinite(d), d, torch.full_like(d, float("inf")))
-    bound = rho * ref.abs() + tau * S + floor
-    ratio = torch.where(bound > 0, d / bound.clamp_min(1e-300), torch.where(d > 0, float("inf"), 0.0))
-    excess = (d - rho * ref.abs() - floor).clamp_min(0.0)
-    need = torch.where(S > 0, excess / S.clamp_min(1e-300), torch.where(excess > 0, float("inf"), 0.0))
-    return (float(ratio.max()) if ratio.numel() else 0.0), (float(need.max()) if need.numel() else 0.0)
-
-
 def _rho(t):
     return RHO_BF16 if t.dtype == torch.bfloat16 else 0.0
-
-
-def image_subset(B):
-    """Images whose outputs are checked for the per-image operators: all of them up to 8, else 0, 1, B/2 and B-1."""
-    return list(range(B)) if B <= 8 else sorted({0, 1, B // 2, B - 1})
 
 
 # ---------------------------------------------------------------------------------------------------------------
 # guarded replay
 # ---------------------------------------------------------------------------------------------------------------
-def _bits(t):
-    ity, _ = SENTINEL[t.dtype]
-    return t.view(ity)
-
-
-def _guarded(n, dtype, guard, dev):
-    buf = torch.empty(guard + n + guard, dtype=dtype, device=dev)
-    _bits(buf).fill_(SENTINEL[dtype][1])
-    return buf
-
-
-def _guard_report(buf, n, guard, ref_out):
-    s = SENTINEL[buf.dtype][1]
-    bits = _bits(buf)
-    problems = []
-    if not bool((bits[:guard] == s).all()):
-        problems.append("wrote %d elements before the output" % int((bits[:guard] != s).sum()))
-    if not bool((bits[guard + n:] == s).all()):
-        problems.append("wrote %d elements past the output" % int((bits[guard + n:] != s).sum()))
-    inner = bits[guard:guard + n]
-    if bool((inner == s).any()):
-        problems.append("left %d output elements unwritten" % int((inner == s).sum()))
-    if not torch.equal(inner, _bits(ref_out.reshape(-1))):
-        problems.append("replay differs from the plan's output in %d elements" % int((inner != _bits(ref_out.reshape(-1))).sum()))
-    return problems
-
-
-def _guard_len(row):
-    return (128 * row + 4096 + 511) // 512 * 512          # >= one 128-row tile; keeps the interior 1 KB aligned
-
-
 def replay_igemm(d, out):
     """Launches the plan's descriptor once more into a sentinel-guarded buffer; returns a list of problems."""
     n = out.numel()
-    guard = _guard_len(max(d.N, d.ldo))
-    buf = _guarded(n, out.dtype, guard, out.device)
+    guard = guard_len(max(d.N, d.ldo))
+    buf = guarded(n, out.dtype, guard, out.device)
     d2 = cabi.IgemmDesc.from_buffer_copy(d)
     d2.out = buf[guard:].data_ptr()
     _ORIG["cabi.igemm"](d2)
     torch.cuda.synchronize()
-    return _guard_report(buf, n, guard, out)
+    return guard_report(buf, n, guard, out)
 
 
 def replay_wgrad(d, out):
     n = out.numel()
-    guard = _guard_len(d.N)
-    buf = _guarded(n, out.dtype, guard, out.device)
+    guard = guard_len(d.N)
+    buf = guarded(n, out.dtype, guard, out.device)
     d2 = cabi.WgradDesc.from_buffer_copy(d)
     n_ws = cabi.wgrad_workspace_elems(d2)
     ws = torch.empty(n_ws, dtype=torch.float32, device=out.device)
@@ -309,7 +242,7 @@ def replay_wgrad(d, out):
     d2.out = buf[guard:].data_ptr()
     _ORIG["cabi.wgrad"](d2)
     torch.cuda.synchronize()
-    return _guard_report(buf, n, guard, out)
+    return guard_report(buf, n, guard, out)
 
 
 # ---------------------------------------------------------------------------------------------------------------
