@@ -122,11 +122,8 @@ def main(args):
     model = models.CVM_VIGOR("cuda", True)
     fill_deterministic(model.state_dict(), seed=0)          # identical replicas on every rank
     model = model.to(dev).set_precision(args.precision).train()
-    # PyTorch-side tuning of the (PyTorch) encoders: cuDNN autotuning, and optionally channels-last convolutions
+    # PyTorch-side tuning of the (PyTorch) encoders: cuDNN autotuning, and channels-last inputs (below)
     torch.backends.cudnn.benchmark = True
-    # (the model itself feeds its bf16-autocast encoders channels-last inputs; CCVPE_TRAIN_CL=1 additionally keeps the resident
-    # input buffers channels-last so that conversion is free)
-    enc_cl = os.environ.get("CCVPE_TRAIN_CL", "1") == "1"
     if args.backend == "simt":
         model.set_backend(cabi.BACKEND_SIMT)
     reducer = GradientAllReducer(model)
@@ -135,9 +132,9 @@ def main(args):
                            capturable=use_graph)
     host = [t.pin_memory() for t in _synthetic_batch(Bsz, 200 + rank)]
     resident = [t.to(dev) for t in host]
-    if enc_cl:
-        resident[0] = resident[0].contiguous(memory_format=torch.channels_last)
-        resident[1] = resident[1].contiguous(memory_format=torch.channels_last)
+    # the model feeds its bf16-autocast encoders channels-last inputs: resident channels-last buffers make that conversion free
+    resident[0] = resident[0].contiguous(memory_format=torch.channels_last)
+    resident[1] = resident[1].contiguous(memory_format=torch.channels_last)
 
     def eager_step(grd, sat, gt, gwo, gor):
         reducer.zero_grad()
@@ -337,7 +334,7 @@ def main(args):
             "config": {"workload": DESC, "workload_key": "train", "batch_per_gpu": Bsz, "global_batch": world * Bsz,
                        "parallelism": "data-parallel x%d (bucketed NCCL gradient all-reduce)" % world,
                        "backend": args.backend, "optimizer": "Adam(lr=1e-4, betas=(0.9, 0.999)), fused",
-                       "encoder_memory_format": "channels_last" if enc_cl else "contiguous", "cudnn_benchmark": True,
+                       "encoder_memory_format": "channels_last", "cudnn_benchmark": True,
                        "cuda_graph": bool(use_graph), **({"cuda_graph_note": graph_note} if graph_note else {}),
                        "precision_note": "fp32 master weights and optimizer; encoders fp32 autograd; decoder activations and GEMM "
                                          "operands in the stated dtype with fp32 accumulation",

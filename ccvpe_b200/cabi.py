@@ -439,14 +439,24 @@ def dwconv_kernel_name(B: int, C: int, Hp: int, Wp: int, k: int, stride: int) ->
     return DWCONV_KERNELS[rc]
 
 
+def w_nk_layout(per_tap_rows: torch.Tensor, splits: Sequence[int]) -> torch.Tensor:
+    """[N, taps, sum(splits)] weights -> bf16 [N, taps, sum(pad(split))], the tcgen05 backend's w_nk layout
+    (include/ccvpe_b200.h): every source's K range is zero padded to a multiple of its K-block width, 16 if c <= 16,
+    32 if c <= 32, else 64 (the kernels' tc_block_width)."""
+    N, taps, _ = per_tap_rows.shape
+    pads = [-(-c // kw) * kw for c, kw in ((c, 16 if c <= 16 else (32 if c <= 32 else 64)) for c in splits)]
+    out = torch.zeros((N, taps, sum(pads)), dtype=torch.bfloat16, device=per_tap_rows.device)
+    src = dst = 0
+    for c, cp in zip(splits, pads):
+        out[:, :, dst:dst + c] = per_tap_rows[:, :, src:src + c]
+        src += c
+        dst += cp
+    return out
+
+
 def pad_k_blocks(w: torch.Tensor) -> torch.Tensor:
-    """[N, K] weights -> bf16 [N, pad(K)] in the tcgen05 backend's K-block padded layout (include/ccvpe_b200.h: block width
-    16 if K <= 16, 32 if K < 64, else 64; zero filled)."""
-    N, K = w.shape
-    kw = 16 if K <= 16 else (32 if K < 64 else 64)
-    out = torch.zeros((N, -(-K // kw) * kw), dtype=torch.bfloat16, device=w.device)
-    out[:, :K] = w
-    return out.contiguous()
+    """[N, K] weights -> bf16 [N, pad(K)]: the one-source, one-tap case of `w_nk_layout`."""
+    return w_nk_layout(w.unsqueeze(1), [w.shape[1]]).squeeze(1)
 
 
 def pointwise_silu_nhwc(x: torch.Tensor, w_nk: torch.Tensor, bias: Optional[torch.Tensor], out: torch.Tensor,

@@ -396,9 +396,8 @@ static bool ring_plan(const ccvpe_igemm_desc& d, RingParams* p) {
     }
     p->n_steps = fits ? j : 0;
     // the plain bf16 channels-last convs with 2..4 K16 slices per tap (levels 2 and 3) take the unrolled issue path
-    static const bool unroll_off = getenv("CCVPE_RING_UNROLL") && atoi(getenv("CCVPE_RING_UNROLL")) == 0;   // development switch
     const bool plain = d.relu != 2 && d.out_mode == 0 && d.out_dtype == CCVPE_BF16 && !d.row_r1;            // epilogue variant 0
-    p->unrolled = (!unroll_off && plain && ring_stages_output(d) && p->n_steps >= 2 && p->n_steps <= 4) ? 1 : 0;
+    p->unrolled = (plain && ring_stages_output(d) && p->n_steps >= 2 && p->n_steps <= 4) ? 1 : 0;
   }
   p->tx_row = (p->nb0 * p->kw0 + p->nb1 * p->kw1) * RING_HALO_W * 2;
   p->tx_weights = 9 * (p->nb0 * p->kw0 + p->nb1 * p->kw1) * p->block_n * 2;

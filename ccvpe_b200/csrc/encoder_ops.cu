@@ -140,33 +140,24 @@ __device__ __forceinline__ float dw_tanh(float x) {
   return y;
 }
 
-// V = channels per thread (8: 16-byte vectors; 4: 8-byte vectors -- half the registers, twice the resident warps, which
-// is what the latency-bound 5x5 layers need).
-template <int V> struct DwVec;
-template <> struct DwVec<8> { using type = uint4; };
-template <> struct DwVec<4> { using type = uint2; };
-template <int V>
-__device__ __forceinline__ void dw_widen(const typename DwVec<V>::type& q, uint64_t (&f)[V / 2]);
-template <>
-__device__ __forceinline__ void dw_widen<8>(const uint4& q, uint64_t (&f)[4]) {
+__device__ __forceinline__ void dw_widen(const uint4& q, uint64_t (&f)[4]) {
   f[0] = bf16x2_to_f32x2(q.x);
   f[1] = bf16x2_to_f32x2(q.y);
   f[2] = bf16x2_to_f32x2(q.z);
   f[3] = bf16x2_to_f32x2(q.w);
 }
-template <>
-__device__ __forceinline__ void dw_widen<4>(const uint2& q, uint64_t (&f)[2]) {
-  f[0] = bf16x2_to_f32x2(q.x);
-  f[1] = bf16x2_to_f32x2(q.y);
-}
 
-template <int K, int S, int V>
-__global__ void __launch_bounds__(256, V == 8 ? 2 : 3)
+// (measured: 4 channels per thread gains nothing over 8, the loop is issue-bound)
+constexpr int DW_V = 8;                              // channels per thread: one 16-byte vector
+
+template <int K, int S>
+__global__ void __launch_bounds__(256, 2)
 dwconv_bias_silu_kernel(const __nv_bfloat16* __restrict__ x, int64_t x_sb, int64_t x_sh, int64_t x_sw,
                         const __nv_bfloat16* __restrict__ w, const __nv_bfloat16* __restrict__ bias,
                         __nv_bfloat16* __restrict__ y, int Ho, int Wo, int C, int CG, int strips_per_block,
                         long long* __restrict__ chan_sum) {
-  using vec_t = typename DwVec<V>::type;
+  constexpr int V = DW_V;
+  using vec_t = uint4;
   constexpr int P = V / 2;                           // fp32x2 pairs per thread
   constexpr int TW = 4;                              // outputs per thread along W
   constexpr int IW = (TW - 1) * S + K;               // input columns a strip touches
@@ -219,7 +210,7 @@ dwconv_bias_silu_kernel(const __nv_bfloat16* __restrict__ x, int64_t x_sb, int64
   for (int j = 0; j < V; ++j) csum[j] = 0.f;
   if (active) {
     uint64_t bv[P];
-    dw_widen<V>(*reinterpret_cast<const vec_t*>(bias + cg * V), bv);
+    dw_widen(*reinterpret_cast<const vec_t*>(bias + cg * V), bv);
 #pragma unroll
     for (int j = 0; j < P; ++j) {                       // bias pre-halved like the weights
       float lo, hi;
@@ -261,7 +252,7 @@ dwconv_bias_silu_kernel(const __nv_bfloat16* __restrict__ x, int64_t x_sb, int64
 #pragma unroll
           for (int t = 0; t < TW; ++t) {
             const int ix = t * S + kx;
-            if (t == TW - 1 || kx < S) dw_widen<V>(xin[ix], xf[ix]);   // first use of this input column
+            if (t == TW - 1 || kx < S) dw_widen(xin[ix], xf[ix]);      // first use of this input column
 #pragma unroll
             for (int j = 0; j < P; ++j) acc[t][j] = ffma2(xf[ix][j], wv[j], acc[t][j]);
           }
@@ -534,15 +525,14 @@ static bool dwt_plan(int K, int Ho, int Wo, int C, int B, DwTileParams* p) {
 // The depthwise dispatch, shared by the launch and by ccvpe_dwconv_plan so that the two cannot disagree: checks the shape,
 // then returns 1 for dwconv_tile_kernel (its plan in *tp), 0 for dwconv_bias_silu_kernel, < 0 on a bad argument.
 // Measured per layer (B=64, scripts/bench_dwconv.py): the tiled kernel wins wherever the window is 5x5 (1.2-1.5x) and for
-// the deep 3x3 layers (>= 240 channels); the shallow 3x3 layers (32 / 144 channels on large images) stay on the streaming
-// kernel.  CCVPE_DW_TILED = 0 / 2 forces streaming / tiled (development switch).
+// the deep 3x3 layers (>= 240 channels); the shallow 3x3 layers (32 / 144 channels on large images) and every stride-2
+// layer stay on the streaming kernel.
 static int dw_select(int B, int C, int Hp, int Wp, int K, int S, DwTileParams* tp) {
   CCVPE_REQUIRE(B > 0 && C > 0 && C % 8 == 0 && C <= 2048, "ccvpe_dwconv_bias_silu_nhwc: bad shape B=%d C=%d", B, C);
   CCVPE_REQUIRE((K == 3 || K == 5) && (S == 1 || S == 2) && Hp >= K && Wp >= K, "ccvpe_dwconv_bias_silu_nhwc: K=%d S=%d Hp=%d Wp=%d unsupported", K, S, Hp, Wp);
   const int Ho = (Hp - K) / S + 1, Wo = (Wp - K) / S + 1;
-  static const int use_tiled = getenv("CCVPE_DW_TILED") ? atoi(getenv("CCVPE_DW_TILED")) : 1;
   memset(tp, 0, sizeof(*tp));
-  if (S == 1 && (use_tiled == 2 || (use_tiled == 1 && (K == 5 || C >= 240))) && dwt_plan(K, Ho, Wo, C, B, tp)) return 1;
+  if (S == 1 && (K == 5 || C >= 240) && dwt_plan(K, Ho, Wo, C, B, tp)) return 1;
   return 0;
 }
 
@@ -872,9 +862,7 @@ extern "C" int ccvpe_dwconv_bias_silu_nhwc(const void* x, int64_t x_sb, int64_t 
     CCVPE_LAUNCH_CHECK("dwconv_tile_kernel");
     return CCVPE_OK;
   }
-  // V = channels per thread
-  static const int force_v = getenv("CCVPE_DW_V") ? atoi(getenv("CCVPE_DW_V")) : 0;
-  const int V = force_v ? force_v : 8;   // (measured: 4 channels per thread gains nothing, the loop is issue-bound)
+  constexpr int V = DW_V;
   const int G = C / V;
   // channel chunking: up to 256 channels a block takes them all; wider layers are cut into chunks of CG groups, CG the
   // largest divisor of G giving 64..128 channels (else 128 with a partial last chunk), which multiplies the number of
@@ -902,28 +890,20 @@ extern "C" int ccvpe_dwconv_bias_silu_nhwc(const void* x, int64_t x_sb, int64_t 
   CCVPE_REQUIRE(sm <= 96 * 1024, "ccvpe_dwconv_bias_silu_nhwc: K*K*C too large for shared memory");
   static thread_local uint64_t attr_set = 0;
   if (first_use_on_device(attr_set)) {
-#define CCVPE_DW_ATTR(KK, SS, VV) \
-  cudaFuncSetAttribute(dwconv_bias_silu_kernel<KK, SS, VV>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024)
-    CCVPE_DW_ATTR(3, 1, 8); CCVPE_DW_ATTR(3, 2, 8); CCVPE_DW_ATTR(5, 1, 8); CCVPE_DW_ATTR(5, 2, 8);
-    CCVPE_DW_ATTR(3, 1, 4); CCVPE_DW_ATTR(3, 2, 4); CCVPE_DW_ATTR(5, 1, 4); CCVPE_DW_ATTR(5, 2, 4);
+#define CCVPE_DW_ATTR(KK, SS) \
+  cudaFuncSetAttribute(dwconv_bias_silu_kernel<KK, SS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024)
+    CCVPE_DW_ATTR(3, 1); CCVPE_DW_ATTR(3, 2); CCVPE_DW_ATTR(5, 1); CCVPE_DW_ATTR(5, 2);
 #undef CCVPE_DW_ATTR
   }
   cudaStream_t st = (cudaStream_t)stream;
-#define CCVPE_DW(KK, SS, VV)                                                                                          \
-  dwconv_bias_silu_kernel<KK, SS, VV><<<grid, 256, sm, st>>>((const __nv_bfloat16*)x, x_sb, x_sh, x_sw,               \
-                                                             (const __nv_bfloat16*)w, (const __nv_bfloat16*)bias,     \
-                                                             (__nv_bfloat16*)y, Ho, Wo, C, CG, (int)spb, reinterpret_cast<long long*>(chan_sum))
-  if (V == 8) {
-    if (K == 3 && S == 1) CCVPE_DW(3, 1, 8);
-    else if (K == 3 && S == 2) CCVPE_DW(3, 2, 8);
-    else if (K == 5 && S == 1) CCVPE_DW(5, 1, 8);
-    else CCVPE_DW(5, 2, 8);
-  } else {
-    if (K == 3 && S == 1) CCVPE_DW(3, 1, 4);
-    else if (K == 3 && S == 2) CCVPE_DW(3, 2, 4);
-    else if (K == 5 && S == 1) CCVPE_DW(5, 1, 4);
-    else CCVPE_DW(5, 2, 4);
-  }
+#define CCVPE_DW(KK, SS)                                                                                              \
+  dwconv_bias_silu_kernel<KK, SS><<<grid, 256, sm, st>>>((const __nv_bfloat16*)x, x_sb, x_sh, x_sw,                   \
+                                                         (const __nv_bfloat16*)w, (const __nv_bfloat16*)bias,         \
+                                                         (__nv_bfloat16*)y, Ho, Wo, C, CG, (int)spb, reinterpret_cast<long long*>(chan_sum))
+  if (K == 3 && S == 1) CCVPE_DW(3, 1);
+  else if (K == 3 && S == 2) CCVPE_DW(3, 2);
+  else if (K == 5 && S == 1) CCVPE_DW(5, 1);
+  else CCVPE_DW(5, 2);
 #undef CCVPE_DW
   CCVPE_LAUNCH_CHECK("dwconv_bias_silu_kernel");
   return CCVPE_OK;

@@ -216,11 +216,6 @@ bool conv_ring_supported(const ccvpe_igemm_desc& d);
 
 }  // namespace ccvpe
 
-static bool ring_disabled() {
-  static const bool off = getenv("CCVPE_DISABLE_RING") != nullptr;
-  return off;
-}
-
 extern "C" int ccvpe_igemm_plan(const ccvpe_igemm_desc* desc) {
   using namespace ccvpe;
   CCVPE_REQUIRE(desc != nullptr, "ccvpe_igemm_plan: null descriptor");
@@ -230,7 +225,7 @@ extern "C" int ccvpe_igemm_plan(const ccvpe_igemm_desc* desc) {
     backend = (d.dtype == CCVPE_BF16 && d.w_nk && igemm_tcgen05_supported(d)) ? CCVPE_BACKEND_TCGEN05
                                                                                : CCVPE_BACKEND_SIMT;
   if (backend == CCVPE_BACKEND_SIMT) return 0;
-  if (backend == CCVPE_BACKEND_TCGEN05) return (!ring_disabled() && conv_ring_supported(d)) ? 2 : 1;
+  if (backend == CCVPE_BACKEND_TCGEN05) return conv_ring_supported(d) ? 2 : 1;
   return fail(CCVPE_ERR_BAD_ARGUMENT, "ccvpe_igemm_plan: unknown backend %d", d.backend);
 }
 
@@ -260,8 +255,8 @@ extern "C" int ccvpe_igemm(const ccvpe_igemm_desc* desc, void* stream) {
     backend = (d.dtype == CCVPE_BF16 && d.w_nk && igemm_tcgen05_supported(d)) ? CCVPE_BACKEND_TCGEN05
                                                                                : CCVPE_BACKEND_SIMT;
   if (backend == CCVPE_BACKEND_TCGEN05) {
-    // wide shallow 3x3 levels take the row-ring kernel (CCVPE_DISABLE_RING=1 forces the generic pipeline: A/B tests)
-    if (!ring_disabled() && conv_ring_supported(d)) return conv_ring_tcgen05(d, st);
+    // wide shallow 3x3 levels take the row-ring kernel
+    if (conv_ring_supported(d)) return conv_ring_tcgen05(d, st);
     return igemm_tcgen05(d, st, nullptr);
   }
   if (backend == CCVPE_BACKEND_SIMT) return igemm_simt(d, st);

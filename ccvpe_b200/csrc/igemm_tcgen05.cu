@@ -442,13 +442,6 @@ struct TcGeometry {
   int tw, th, tb;   // conv tile: tw x th pixels x tb images = 128 rows (cell: tw output columns x th (row, image) pairs)
 };
 
-// CCVPE_IGEMM_HALO: 0 = never, 1 = whenever the geometry allows, unset = the shallow 3x3 layers (N <= 160), which are bound by
-// TMA's per-box-row issue rate when every tap loads its own 128-row A box (9 x 128 rows per K block vs 180 for the halo box)
-static int halo_policy() {
-  static const int v = getenv("CCVPE_IGEMM_HALO") ? atoi(getenv("CCVPE_IGEMM_HALO")) : -1;
-  return v;
-}
-
 static bool tc_geometry(const ccvpe_igemm_desc& d, TcGeometry* g) {
   if (d.stride == 2 && d.kh == 2 && d.kw == 2 && d.pad == 0) {
     if (d.Hin != 2 * d.Hout || d.Win != 2 * d.Wout || d.c1 != 0 || !is_pow2(d.Wout)) return false;
@@ -470,7 +463,9 @@ static bool tc_geometry(const ccvpe_igemm_desc& d, TcGeometry* g) {
   }
   if (!is_pow2(d.Wout) || !is_pow2(d.Hout)) return false;
   g->halo = false;
-  if (d.Wout >= 8 && d.Hout >= 16 && halo_policy() != 0 && (halo_policy() == 1 || d.N <= 160)) {
+  // one halo A box per K block for the shallow 3x3 layers (N <= 160), which are bound by TMA's per-box-row issue rate
+  // when every tap loads its own 128-row A box (9 x 128 rows per K block vs 180 for the halo box)
+  if (d.Wout >= 8 && d.Hout >= 16 && d.N <= 160) {
     g->cell = false;
     g->halo = true;
     g->tw = 8;
@@ -582,9 +577,8 @@ int igemm_tcgen05(const ccvpe_igemm_desc& d, cudaStream_t st, const TcOutPad* ou
     // (one B tile of block_n box rows per tap) and the MMA issuer (~70 instructions per tap for 1-4 short MMAs) -- while
     // the tensor pipe idles.  Two CTAs per SM (the LIGHT instantiation: two producers, two issuers, staged epilogue)
     // double both; the shallower rings are what fits 2 x 104 KB.
-    static const int halo_light_env = getenv("CCVPE_HALO_LIGHT") ? atoi(getenv("CCVPE_HALO_LIGHT")) : 1;   // development switch
     const int hl_budget = light_budget - 2 * p.a_slot_bytes;
-    if (halo_light_env && p.tmem_cols <= 256 && block_n <= 96 && hl_budget / stage_bytes >= 3) {
+    if (p.tmem_cols <= 256 && block_n <= 96 && hl_budget / stage_bytes >= 3) {
       light = true;
       p.a_slots = 2;
       p.b_off = p.a_slots * p.a_slot_bytes;

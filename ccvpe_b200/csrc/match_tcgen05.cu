@@ -447,7 +447,7 @@ int match_tcgen05(const void* x, int B, int HW, int C, const float* g, int L, in
 
   static thread_local MatchTcParams p;
   memset(&p, 0, sizeof(p));
-  p.kw = tc_block_width_match(C);
+  p.kw = tc_block_width(C);
   p.nb = (C + p.kw - 1) / p.kw;
   p.C = C;
   p.HW = HW;

@@ -461,18 +461,10 @@ inline int encode_map(CUtensorMap* tm, const void* base, int rank, const uint64_
 
 // K-block width (bf16 channels) used for a source with c channels; one block is one swizzle row of 2*width bytes.
 // Narrow sources get narrow blocks so TMA neither over-fetches nor zero-fills most of the tile (include/ccvpe_b200.h
-// documents the same rule for the w_nk weight layout).
+// documents the same rule for the w_nk weight layout; ccvpe_b200/cabi.py:w_nk_layout builds it).
 // 33..63 channels take ONE 64-wide block rather than two 32-wide ones: the padded K extent (64), the shared-memory
 // footprint and the number of K16 MMA slices are the same, but TMA walks half as many box rows (its cost is per box row).
-inline int tc_block_width(int c) {
-  static const bool old_rule = getenv("CCVPE_KW_OLD") != nullptr;   // development switch: A/B against the round-1 rule
-  return c <= 16 ? 16 : (c < (old_rule ? 64 : 33) ? 32 : 64);
-}
-// the matching kernel (same rule; CCVPE_MATCH_KW_OLD restores two 32-wide blocks for 33..63 channels: development switch)
-inline int tc_block_width_match(int c) {
-  static const bool old_rule = getenv("CCVPE_MATCH_KW_OLD") != nullptr;
-  return c <= 16 ? 16 : (c < (old_rule ? 64 : 33) ? 32 : 64);
-}
+inline int tc_block_width(int c) { return c <= 16 ? 16 : (c <= 32 ? 32 : 64); }
 
 inline void fill_epi(EpiParams& e, const ccvpe_igemm_desc& d) {
   e.N = d.N;

@@ -17,8 +17,6 @@
 // per box row, which is what bounded the first version of this kernel).  K (pixels) is split over
 // CTAs when there are fewer tiles than SMs; partial tiles go to the workspace and are folded in a fixed order
 // (deterministic).  Warp 0 = TMA producer, warp 1 = MMA issuer + TMEM owner, warps 2-5 = epilogue.
-#include <cstdlib>
-
 #include "tcgen05_common.cuh"
 
 namespace ccvpe {
@@ -28,11 +26,9 @@ constexpr int WT_CT = 32;          // A-channel tile
 constexpr int WT_NT = 128;         // G-channel tile
 constexpr int WT_TAPS = 9;
 constexpr int WT_THREADS = 192;
-constexpr int WT_MAX_STAGES = 4;
-constexpr int WT_MAX_STAGES_HALO = 6;
+constexpr int WT_MAX_STAGES = 6;
 constexpr int WT_G_BYTES = WT_BK * WT_NT * 2;          // 16 KB: two [64 px x 64 n] SWIZZLE_128B boxes
-constexpr int WT_A_BYTES = WT_BK * WT_CT * 2;          // 4 KB per tap, SWIZZLE_64B
-constexpr int WT_STAGE_BYTES = WT_G_BYTES + WT_TAPS * WT_A_BYTES;   // 52 KB (one box per tap)
+constexpr int WT_A_BYTES = WT_BK * WT_CT * 2;          // 4 KB per k2 s2 tap, SWIZZLE_64B
 constexpr int WT_ROW_BYTES = WT_CT * 2;                // 64 B: one pixel of an A tile
 
 struct WgradTcParams {
@@ -42,7 +38,7 @@ struct WgradTcParams {
   int ksteps_total, ksteps_per_split;
   int c_tiles0;
   int stages;
-  int halo, stage_bytes, a_tx;         // halo mode: one (hb+2) x (wb+2) A box per stage; bytes TMA delivers for it
+  int stage_bytes, a_tx;               // 3x3: one (hb+2) x (wb+2) A box per stage; a_tx = bytes TMA delivers for it
   int k2s2, taps;                      // k2 s2 layers: 4 taps gathered through a 5-D map [c][dw][j][dh][(b, i)]
   float* dst;
 };
@@ -61,8 +57,8 @@ __device__ __forceinline__ uint64_t make_smem_desc_mn(uint32_t saddr, uint32_t l
 
 __global__ void __launch_bounds__(WT_THREADS, 1) wgrad_tcgen05_kernel(const __grid_constant__ WgradTcParams p) {
   extern __shared__ uint8_t smem_raw[];
-  __shared__ __align__(8) uint64_t bar_full[WT_MAX_STAGES_HALO];
-  __shared__ __align__(8) uint64_t bar_empty[WT_MAX_STAGES_HALO];
+  __shared__ __align__(8) uint64_t bar_full[WT_MAX_STAGES];
+  __shared__ __align__(8) uint64_t bar_empty[WT_MAX_STAGES];
   __shared__ __align__(8) uint64_t bar_acc;
   __shared__ uint32_t tmem_base_slot;
 
@@ -120,19 +116,15 @@ __global__ void __launch_bounds__(WT_THREADS, 1) wgrad_tcgen05_kernel(const __gr
       if (elect_one()) {
         const uint32_t full = smem_u32(&bar_full[stage]);
         const uint32_t dst = smem_base + (uint32_t)(stage * p.stage_bytes);
-        mbar_arrive_expect_tx(full, (uint32_t)(WT_G_BYTES + (p.halo ? p.a_tx : p.taps * WT_A_BYTES)));
+        mbar_arrive_expect_tx(full, (uint32_t)(WT_G_BYTES + (p.k2s2 ? p.taps * WT_A_BYTES : p.a_tx)));
         tma_load_2d(dst, &p.tm_g, full, n0, m0);
         tma_load_2d(dst + WT_G_BYTES / 2, &p.tm_g, full, n1, m0);
         if (p.k2s2) {
 #pragma unroll
           for (int tap = 0; tap < 4; ++tap)      // tap = dh * 2 + dw
             tma_load_5d(dst + WT_G_BYTES + tap * WT_A_BYTES, tma, full, c_start, tap & 1, w0, tap >> 1, h0);
-        } else if (p.halo) {
-          tma_load_4d(dst + WT_G_BYTES, tma, full, c_start, w0 - 1, h0 - 1, b);
         } else {
-#pragma unroll
-          for (int tap = 0; tap < WT_TAPS; ++tap)
-            tma_load_4d(dst + WT_G_BYTES + tap * WT_A_BYTES, tma, full, c_start, w0 + tap % 3 - 1, h0 + tap / 3 - 1, b);
+          tma_load_4d(dst + WT_G_BYTES, tma, full, c_start, w0 - 1, h0 - 1, b);
         }
       }
       __syncwarp();
@@ -144,8 +136,8 @@ __global__ void __launch_bounds__(WT_THREADS, 1) wgrad_tcgen05_kernel(const __gr
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     // D[128 n x 96 (kx, c)] (+)= G^T[128 n x 16 px] * [A_(ky,0) | A_(ky,1) | A_(ky,2)][16 px x 96]; both operands MN-major
-    // (idesc bits 15, 16).  The three kx taps of a ky row are three 32-channel atoms of ONE B operand: in the halo tile
-    // they are the same rows shifted by one pixel (LBO = 64 B: overlapping atoms), in the per-tap layout 4 KB apart.
+    // (idesc bits 15, 16).  The three kx taps of a ky row are three 32-channel atoms of ONE B operand: the same rows of
+    // the halo tile shifted by one pixel (LBO = 64 B: overlapping atoms).
     // One thread issues everything, at ~5 cycles per dependent instruction, so the per-MMA descriptor words are
     // precomputed: 12 MMAs per stage, two adds each.
     constexpr int NW = 3 * WT_CT;                          // 96 accumulator columns per MMA
@@ -158,11 +150,10 @@ __global__ void __launch_bounds__(WT_THREADS, 1) wgrad_tcgen05_kernel(const __gr
       const int hrow = (kk * 16) / p.wb, wcol = (kk * 16) - hrow * p.wb;   // the 16 pixels of K step kk: row hrow, from wcol
 #pragma unroll
       for (int ky = 0; ky < 3; ++ky)
-        a_off[kk][ky] = (uint32_t)(WT_G_BYTES + (p.halo ? ((hrow + ky) * pitch + wcol) * WT_ROW_BYTES
-                                                         : ky * 3 * WT_A_BYTES + kk * 1024)) >> 4;
+        a_off[kk][ky] = (uint32_t)(WT_G_BYTES + ((hrow + ky) * pitch + wcol) * WT_ROW_BYTES) >> 4;
     }
     const uint64_t gdesc0 = make_smem_desc_mn(smem_base, WT_G_BYTES / 2, 1024, 2);
-    const uint64_t adesc0 = make_smem_desc_mn(smem_base, p.halo ? WT_ROW_BYTES : WT_A_BYTES, 512, 4);
+    const uint64_t adesc0 = make_smem_desc_mn(smem_base, p.k2s2 ? WT_A_BYTES : WT_ROW_BYTES, 512, 4);
     // k2 s2: the two dw taps of a dh row are two atoms (4 KB apart) of one N = 64 MMA
     const uint32_t idesc2 = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(2 * WT_CT >> 3) << 17) |
                             ((uint32_t)(WT_NT >> 4) << 24);
@@ -304,11 +295,9 @@ int wgrad_tcgen05(const ccvpe_wgrad_desc& d, cudaStream_t st) {
   p.wb = pl.wb; p.hb = pl.hb; p.tiles_w = pl.tiles_w; p.tiles_h = pl.tiles_h;
   p.ksteps_total = pl.ksteps; p.ksteps_per_split = pl.ksteps_per_split;
   p.c_tiles0 = pl.c_tiles0;
-  static const bool halo_off = getenv("CCVPE_WGRAD_HALO") && atoi(getenv("CCVPE_WGRAD_HALO")) == 0;
-  p.halo = (halo_off || pl.k2s2) ? 0 : 1;
   p.a_tx = (pl.wb + 2) * (pl.hb + 2) * WT_ROW_BYTES;
-  p.stage_bytes = p.halo ? WT_G_BYTES + (p.a_tx + 1023) / 1024 * 1024 : WT_G_BYTES + p.taps * WT_A_BYTES;
-  p.stages = (p.halo || pl.k2s2) ? WT_MAX_STAGES_HALO : WT_MAX_STAGES;
+  p.stage_bytes = pl.k2s2 ? WT_G_BYTES + p.taps * WT_A_BYTES : WT_G_BYTES + (p.a_tx + 1023) / 1024 * 1024;
+  p.stages = WT_MAX_STAGES;
   while (p.stages * p.stage_bytes > 200 * 1024) --p.stages;
   const int64_t n_out = (int64_t)p.Q * d.N;
   if (pl.splits > 1) {
@@ -331,7 +320,7 @@ int wgrad_tcgen05(const ccvpe_wgrad_desc& d, cudaStream_t st) {
     const int c = s ? d.c1 : d.c0, ld = s ? d.ld1 : d.ld0;
     uint64_t dims[4] = {(uint64_t)c, (uint64_t)d.Win, (uint64_t)d.Hin, (uint64_t)d.B};
     uint64_t str[3] = {(uint64_t)ld * 2, (uint64_t)d.Win * ld * 2, (uint64_t)d.Hin * d.Win * ld * 2};
-    uint32_t box[4] = {WT_CT, (uint32_t)(pl.wb + (p.halo ? 2 : 0)), (uint32_t)(pl.hb + (p.halo ? 2 : 0)), 1};
+    uint32_t box[4] = {WT_CT, (uint32_t)(pl.wb + 2), (uint32_t)(pl.hb + 2), 1};
     if ((rc = encode_map(s ? &p.tm_a1 : &p.tm_a0, base, 4, dims, str, box, 32)) != CCVPE_OK) return rc;
   }
   {

@@ -30,20 +30,6 @@ def _cl(t: torch.Tensor, dtype: torch.dtype) -> torch.Tensor:
     return v.contiguous()
 
 
-def _nk(per_tap_rows: torch.Tensor, splits: Sequence[int]) -> torch.Tensor:
-    """[N, taps, K] -> [N, taps, sum(pad(split))] bf16: every source's K range zero padded to its K-block width (16 if
-    c <= 16, 32 if c < 64, else 64 -- the tcgen05 backend's w_nk layout, see include/ccvpe_b200.h)."""
-    N_, taps, _ = per_tap_rows.shape
-    pads = [-(-c // kw) * kw for c, kw in ((c, 16 if c <= 16 else (32 if c < 64 else 64)) for c in splits)]
-    out = torch.zeros((N_, taps, sum(pads)), dtype=torch.bfloat16, device=per_tap_rows.device)
-    src = dst = 0
-    for c, cp in zip(splits, pads):
-        out[:, :, dst:dst + c] = per_tap_rows[:, :, src:src + c]
-        src += c
-        dst += cp
-    return out.contiguous()
-
-
 _SIDE_STREAMS: Dict[int, "torch.cuda.Stream"] = {}
 
 
@@ -171,14 +157,11 @@ class PostEncoderPipeline:
         lw = params["sat_feature_to_descriptors.1.weight"].detach()
         D = lw.shape[0]
         tc = dtype == torch.bfloat16     # also build the K-major layout of the tcgen05 backend
-
-        nk = _nk
-
         w["cell"] = dict(w_kn=lw.view(D, ENCODER_CHANNELS, 2, 2).permute(2, 3, 1, 0).reshape(4, ENCODER_CHANNELS, D)
                          .to(dtype).contiguous(), bias=f32(params["sat_feature_to_descriptors.1.bias"]))
         if tc:
-            w["cell"]["w_nk"] = nk(lw.view(D, ENCODER_CHANNELS, 2, 2).permute(0, 2, 3, 1).reshape(D, 4, ENCODER_CHANNELS),
-                                   [ENCODER_CHANNELS])
+            w["cell"]["w_nk"] = cabi.w_nk_layout(
+                lw.view(D, ENCODER_CHANNELS, 2, 2).permute(0, 2, 3, 1).reshape(D, 4, ENCODER_CHANNELS), [ENCODER_CHANNELS])
 
         def deconv(name: str, lead: int, lead_pad: int):
             """ConvTranspose2d weight [Cin, Cout, 2, 2] -> GEMM B [1][K][4*Cout], N ordered (i, j, co).
@@ -196,7 +179,7 @@ class PostEncoderPipeline:
             out["w_kn"] = W.permute(0, 2, 3, 1).reshape(1, W.shape[0], 4 * cout).to(dtype).contiguous()
             if tc:
                 rows = W.permute(2, 3, 1, 0).reshape(4 * cout, 1, W.shape[0])
-                out["w_nk"] = nk(rows, [lead_pad, W.shape[0] - lead_pad] if lead > 0 else [W.shape[0]])
+                out["w_nk"] = cabi.w_nk_layout(rows, [lead_pad, W.shape[0] - lead_pad] if lead > 0 else [W.shape[0]])
             return out
 
         def conv(name: str, c0: int):
@@ -205,7 +188,7 @@ class PostEncoderPipeline:
                        bias=f32(params[name + ".bias"]), cout=W.shape[0])
             if tc:
                 rows = W.permute(0, 2, 3, 1).reshape(W.shape[0], 9, W.shape[1])
-                out["w_nk"] = nk(rows, [c0, W.shape[1] - c0] if c0 < W.shape[1] else [c0])
+                out["w_nk"] = cabi.w_nk_layout(rows, [c0, W.shape[1] - c0] if c0 < W.shape[1] else [c0])
             return out
 
         w["loc"], w["ori"] = [], []

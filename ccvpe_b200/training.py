@@ -21,7 +21,7 @@ from typing import Dict, List, Optional, Sequence, Tuple
 import torch
 
 from . import cabi
-from .decoder import SCORES_CL_PAD, Fork, PostEncoderPipeline, _cl, _nk
+from .decoder import SCORES_CL_PAD, Fork, PostEncoderPipeline, _cl
 from .specs import ENCODER_CHANNELS, SKIP_BLOCKS
 
 GRAD_PAD = 8      # incoming 1- / 2-channel gradients (logits, orientation field) are zero padded to 8 channels
@@ -52,7 +52,7 @@ class BackwardWeights:
             out = dict(w_kn=Wf.permute(2, 3, 0, 1).reshape(9, coutp, cin).to(dtype).contiguous(), bias=None, cout=cin,
                        k=coutp)
             if tc:
-                out["w_nk"] = _nk(Wf.permute(1, 2, 3, 0).reshape(cin, 9, coutp), [coutp])
+                out["w_nk"] = cabi.w_nk_layout(Wf.permute(1, 2, 3, 0).reshape(cin, 9, coutp), [coutp])
             return out
 
         def deconv_dgrad(name: str, lead: int, lead_pad: int) -> dict:
@@ -71,7 +71,7 @@ class BackwardWeights:
             n = W.shape[0]
             out = dict(w_kn=W.permute(2, 3, 1, 0).reshape(4, cout, n).to(dtype).contiguous(), bias=None, cout=n, k=cout)
             if tc:
-                out["w_nk"] = _nk(W.permute(0, 2, 3, 1).reshape(n, 4, cout), [cout])
+                out["w_nk"] = cabi.w_nk_layout(W.permute(0, 2, 3, 1).reshape(n, 4, cout), [cout])
             return out
 
         self.loc: List[dict] = []
@@ -89,7 +89,7 @@ class BackwardWeights:
         self.cell = dict(w_kn=Wc.permute(0, 2, 3, 1).reshape(1, D, 4 * ENCODER_CHANNELS).to(dtype).contiguous(), bias=None,
                          cout=ENCODER_CHANNELS)
         if tc:
-            self.cell["w_nk"] = _nk(Wc.permute(2, 3, 1, 0).reshape(4 * ENCODER_CHANNELS, 1, D), [D])
+            self.cell["w_nk"] = cabi.w_nk_layout(Wc.permute(2, 3, 1, 0).reshape(4 * ENCODER_CHANNELS, 1, D), [D])
 
 
 class PostEncoderTrainer:

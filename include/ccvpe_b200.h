@@ -91,7 +91,7 @@ typedef struct ccvpe_igemm_desc {
   /* weights, one of (depending on backend):
    *   w_kn : [taps][c0 + c1][N]                     (N contiguous)       -- SIMT backend
    *   w_nk : [N][taps][pad(c0) + pad(c1)]           (K contiguous, bf16) -- tcgen05 backend; pad(c) rounds c up to
-   *          a multiple of the source's K-block width kw(c) = 16 if c <= 16, 32 if c < 64, else 64 (zero filled)   */
+   *          a multiple of the source's K-block width kw(c) = 16 if c <= 16, 32 if c <= 32, else 64 (zero filled)  */
   const void* w_kn; const void* w_nk;
   const float* bias;             /* [N] fp32 or NULL                                                                */
   const float* row_scale;        /* [M] fp32 or NULL                                                                */
@@ -181,8 +181,8 @@ int ccvpe_bias_silu_nhwc(const void* x, const void* bias, void* y, int64_t y_sb,
 int ccvpe_dwconv_bias_silu_nhwc(const void* x, int64_t x_sb, int64_t x_sh, int64_t x_sw, int Hp, int Wp,
                                 const void* w, const void* bias, void* y, int B, int C, int K, int S,
                                 int64_t* chan_sum, void* stream);
-/* which kernel ccvpe_dwconv_bias_silu_nhwc would launch for this layer (the launch makes the same choice, environment
- * switches included): 0 = dwconv_bias_silu_kernel, 1 = dwconv_tile_kernel; < 0 = error. */
+/* which kernel ccvpe_dwconv_bias_silu_nhwc would launch for this layer (the launch makes the same choice):
+ * 0 = dwconv_bias_silu_kernel, 1 = dwconv_tile_kernel; < 0 = error. */
 int ccvpe_dwconv_plan(int B, int C, int Hp, int Wp, int K, int S);
 
 /* Encoder stem (reference efficientnet_pytorch/model.py:296-297 in eval mode, BN folded; circular variant: the reference's

@@ -12,18 +12,6 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from ccvpe_b200 import cabi  # noqa: E402
 
 
-def nk(rows, splits):
-    N_, taps, _ = rows.shape
-    pads = [-(-c // kw) * kw for c, kw in ((c, 16 if c <= 16 else (32 if c < 64 else 64)) for c in splits)]
-    out = torch.zeros((N_, taps, sum(pads)), dtype=torch.bfloat16, device=rows.device)
-    src = dst = 0
-    for c, cp in zip(splits, pads):
-        out[:, :, dst:dst + c] = rows[:, :, src:src + c]
-        src += c
-        dst += cp
-    return out.contiguous()
-
-
 def main():
     kind = sys.argv[1]
     dev = torch.device("cuda")
@@ -35,7 +23,7 @@ def main():
         a0 = torch.randn(B, H, H, c0, device=dev, dtype=bf)
         a1 = torch.randn(B, H, H, c1, device=dev, dtype=bf) if c1 else None
         W = torch.randn(cout, c0 + c1, 3, 3, device=dev) * 0.05
-        w_nk = nk(W.permute(0, 2, 3, 1).reshape(cout, 9, c0 + c1), [c0, c1] if c1 else [c0])
+        w_nk = cabi.w_nk_layout(W.permute(0, 2, 3, 1).reshape(cout, 9, c0 + c1), [c0, c1] if c1 else [c0])
         out = torch.empty(B, H, H, cout, device=dev, dtype=bf)
         bias = torch.randn(cout, device=dev)
         d.a0, d.a1, d.c0, d.c1, d.ld0, d.ld1 = a0.data_ptr(), (a1.data_ptr() if c1 else None), c0, c1, c0, c1
@@ -49,7 +37,7 @@ def main():
         reps = int(sys.argv[6]) if len(sys.argv) > 6 else 10
         a0 = torch.randn(B, H, H, C, device=dev, dtype=bf)
         W = torch.randn(C, cout, 2, 2, device=dev) * 0.05
-        w_nk = nk(W.permute(2, 3, 1, 0).reshape(4 * cout, 1, C), [C])
+        w_nk = cabi.w_nk_layout(W.permute(2, 3, 1, 0).reshape(4 * cout, 1, C), [C])
         out = torch.empty(B, 2 * H, 2 * H, cout, device=dev, dtype=bf)
         bias = torch.randn(4 * cout, device=dev)
         rs = torch.rand(B * H * H, device=dev)

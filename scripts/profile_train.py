@@ -15,9 +15,8 @@ red = GradientAllReducer(model)
 opt = torch.optim.Adam([p for p in model.parameters() if p.requires_grad], lr=1e-4, fused=True)
 B = 8
 batch = [t.to(dev) for t in synthetic_pair(B, (320, 640), seed=1)] + [t.to(dev) for t in synthetic_ground_truth(B, seed=1)]
-if os.environ.get("CCVPE_TRAIN_CL_INPUTS", "1") == "1":
-    batch[0] = batch[0].contiguous(memory_format=torch.channels_last)
-    batch[1] = batch[1].contiguous(memory_format=torch.channels_last)
+batch[0] = batch[0].contiguous(memory_format=torch.channels_last)
+batch[1] = batch[1].contiguous(memory_format=torch.channels_last)
 
 def step():
     red.zero_grad()

@@ -37,7 +37,6 @@ The CPU self-test at the end shows that the bounds pass a correctly rounded resu
 """
 import inspect
 import math
-import os
 import time
 
 import numpy as np
@@ -49,9 +48,6 @@ from ccvpe_b200 import cabi
 from ccvpe_b200.fast_encoder import FastEncoder
 from helpers import (RHO_BF16, TINY, bound_check, guard_len, guard_report, guarded, image_subset, sentinel_bits,
                      subnormal_floor)
-
-assert "CCVPE_DW_TILED" not in os.environ and "CCVPE_DW_V" not in os.environ, \
-    "the encoder plan check covers the default depthwise dispatch only"
 
 F64 = torch.float64
 

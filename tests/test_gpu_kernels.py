@@ -59,19 +59,6 @@ def test_grd_descriptor(cuda_device, B, H, W, c, layout, dtype):
 # ---------------------------------------------------------------------------------------------------------------
 # igemm helper
 # ---------------------------------------------------------------------------------------------------------------
-def _nk(rows, splits):
-    """[N, taps, K] -> tcgen05 weight layout [N, taps, sum(pad64(split))] bf16 (see include/ccvpe_b200.h)."""
-    N_, taps, _ = rows.shape
-    pads = [-(-c // kw) * kw for c, kw in ((c, 16 if c <= 16 else (32 if c < 64 else 64)) for c in splits)]
-    out = torch.zeros((N_, taps, sum(pads)), dtype=torch.bfloat16)
-    src = dst = 0
-    for c, cp in zip(splits, pads):
-        out[:, :, dst:dst + c] = rows[:, :, src:src + c]
-        src += c
-        dst += cp
-    return out.contiguous()
-
-
 def _igemm(dev, a0, a1, Hout, Wout, stride, k, pad, N, w_kn, bias, out, out_mode, ldo, relu=False, row_scale=None,
            row_r1=None, r1_w=None, backend=cabi.BACKEND_SIMT, w_nk=None):
     d = cabi.IgemmDesc()
@@ -108,7 +95,7 @@ def test_sat_cell_descriptors(cuda_device, B, D, dtype, tol, backend):
     bias = torch.randn(D, generator=g)
     ref = orc.sat_cell_descriptors(fs.to(dtype).float(), W.to(dtype).float(), bias)       # [B, D, 8, 8]
     w_kn = W.view(D, 1280, 2, 2).permute(2, 3, 1, 0).reshape(4, 1280, D).contiguous().to(cuda_device, dtype)
-    w_nk = _nk(W.view(D, 1280, 2, 2).permute(0, 2, 3, 1).reshape(D, 4, 1280), [1280]).to(cuda_device)
+    w_nk = cabi.w_nk_layout(W.view(D, 1280, 2, 2).permute(0, 2, 3, 1).reshape(D, 4, 1280), [1280]).to(cuda_device)
     out = torch.empty(B, 8, 8, D, device=cuda_device, dtype=dtype)
     _igemm(cuda_device, _cl(fs, dtype, cuda_device), None, 8, 8, 2, 2, 0, D, w_kn, bias.to(cuda_device), out, 0, D,
            backend=backend, w_nk=w_nk)
@@ -313,7 +300,7 @@ def test_deconv_fused_normalize_concat(cuda_device, B, C, H, cout, dtype, tol, b
     inv = (1.0 / xr.norm(dim=1).clamp_min(1e-12)).to(dev)
     w_kn = W[1:].permute(0, 2, 3, 1).reshape(1, C, 4 * cout).contiguous().to(dev, dtype)
     r1_w = W[0].permute(1, 2, 0).reshape(4 * cout).contiguous().to(dev)
-    w_nk = _nk(W[1:].permute(2, 3, 1, 0).reshape(4 * cout, 1, C), [C]).to(dev)
+    w_nk = cabi.w_nk_layout(W[1:].permute(2, 3, 1, 0).reshape(4 * cout, 1, C), [C]).to(dev)
     out = torch.empty(B, 2 * H, 2 * H, cout, device=dev, dtype=dtype)
     _igemm(dev, _cl(x, dtype, dev), None, H, H, 1, 1, 0, 4 * cout, w_kn, bias.repeat(4).to(dev), out, 1, cout,
            row_scale=inv.contiguous(), row_r1=mx[:, 0].contiguous().to(dev), r1_w=r1_w, backend=backend, w_nk=w_nk)
@@ -358,7 +345,7 @@ def test_conv3x3_two_sources(cuda_device, B, c0, c1, cout, H, relu, mode, dtype,
     if relu:
         ref = F.relu(ref)
     w_kn = W.permute(2, 3, 1, 0).reshape(9, c0 + c1, cout).contiguous().to(dev, dtype)
-    w_nk = _nk(W.permute(0, 2, 3, 1).reshape(cout, 9, c0 + c1), [c0, c1] if c1 else [c0]).to(dev)
+    w_nk = cabi.w_nk_layout(W.permute(0, 2, 3, 1).reshape(cout, 9, c0 + c1), [c0, c1] if c1 else [c0]).to(dev)
     if mode == 2:
         out = torch.empty(B, cout, H, H, device=dev)
         _igemm(dev, _cl(a0, dtype, dev), None, H, H, 1, 3, 1, cout, w_kn, bias.to(dev), out, 2, 0, relu=relu,
@@ -770,7 +757,7 @@ def test_conv_k2s2_general_shapes(cuda_device, B, C, N, Hout, Wout, backend):
     w = (torch.randn(N, C, 2, 2, generator=g) * 0.1).to(dt).float()
     ref = F.conv2d(x, w, stride=2)
     w_kn = w.permute(2, 3, 1, 0).reshape(4, C, N).contiguous().to(dev, dt)
-    w_nk = _nk(w.permute(0, 2, 3, 1).reshape(N, 4, C), [C]).to(dev)
+    w_nk = cabi.w_nk_layout(w.permute(0, 2, 3, 1).reshape(N, 4, C), [C]).to(dev)
     out = torch.empty(B, Hout, Wout, N, device=dev, dtype=dt)
     _igemm(dev, _cl(x, dt, dev), None, Hout, Wout, 2, 2, 0, N, w_kn, None, out, 0, N, backend=backend, w_nk=w_nk)
     assert rel_err(out.permute(0, 3, 1, 2).float(), ref) < BF16_TOL

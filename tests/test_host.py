@@ -72,13 +72,22 @@ def test_specs_match_reference_tables():
 
 
 def test_pad_k_blocks_layout_rule():
-    """w_nk K padding documented in include/ccvpe_b200.h: block width 16 if K <= 16, 32 if K < 64, else 64; zero filled."""
-    for K, padded in [(16, 16), (24, 32), (40, 64), (80, 128), (112, 128), (192, 192), (320, 320), (8, 16)]:
+    """w_nk K padding documented in include/ccvpe_b200.h and used by the kernels (tc_block_width): block width 16 if
+    K <= 16, 32 if K <= 32, else 64; zero filled.  Each source of a two-source layout is padded by its own width."""
+    for K, padded in [(16, 16), (24, 32), (40, 64), (80, 128), (112, 128), (192, 192), (320, 320), (8, 16),
+                      (32, 32), (33, 64), (63, 64), (64, 64)]:
         w = torch.arange(3 * K, dtype=torch.float32).reshape(3, K) + 1.0
         out = cabi.pad_k_blocks(w)
         assert out.dtype == torch.bfloat16 and tuple(out.shape) == (3, padded), (K, out.shape)
         assert torch.equal(out[:, :K].float(), w.to(torch.bfloat16).float())
         assert float(out[:, K:].abs().sum()) == 0.0
+    # two sources of 40 + 24 channels over 9 taps -> 64 + 32 per tap
+    rows = torch.arange(2 * 9 * 64, dtype=torch.float32).reshape(2, 9, 64) + 1.0
+    out = cabi.w_nk_layout(rows, [40, 24])
+    assert out.dtype == torch.bfloat16 and tuple(out.shape) == (2, 9, 96), out.shape
+    assert torch.equal(out[:, :, :40].float(), rows[:, :, :40].to(torch.bfloat16).float())
+    assert torch.equal(out[:, :, 64:88].float(), rows[:, :, 40:].to(torch.bfloat16).float())
+    assert float(out[:, :, 40:64].abs().sum()) == 0.0 and float(out[:, :, 88:].abs().sum()) == 0.0
 
 
 def test_cuda_graph_cache_is_dropped_when_weights_change():
