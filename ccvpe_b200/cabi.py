@@ -34,6 +34,7 @@ EXPORTED_SYMBOLS = (
     "ccvpe_match_bwd_scratch_elems", "ccvpe_match_level_bwd", "ccvpe_loss_workspace_elems", "ccvpe_infonce_loss",
     "ccvpe_cross_entropy_loss", "ccvpe_orientation_loss", "ccvpe_grd_descriptors_bwd",
     "ccvpe_gt_pyramid", "ccvpe_infonce_loss_binned", "ccvpe_orientation_loss_const", "ccvpe_pose_labels",
+    "ccvpe_pose_hypotheses_smem_bytes", "ccvpe_pose_hypotheses",
 )
 
 
@@ -130,6 +131,10 @@ def load() -> C.CDLL:
     lib.ccvpe_pose_decode.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_void_p]
+    lib.ccvpe_pose_hypotheses_smem_bytes.restype = C.c_int64
+    lib.ccvpe_pose_hypotheses_smem_bytes.argtypes = [C.c_int, C.c_int]
+    lib.ccvpe_pose_hypotheses.restype = C.c_int
+    lib.ccvpe_pose_hypotheses.argtypes = [C.c_void_p, C.c_void_p] + [C.c_int] * 5 + [C.c_void_p] * 9
     lib.ccvpe_bias_silu_nhwc.restype = C.c_int
     lib.ccvpe_bias_silu_nhwc.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64,
                                          C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
@@ -396,6 +401,48 @@ def pose_decode(heatmap: torch.Tensor, ori: torch.Tensor, idx, rc, cs, angle, va
     H, W = heatmap.shape[-2:]
     _check(load().ccvpe_pose_decode(_ptr(heatmap), _ptr(ori), B, H, W, _ptr(idx), _ptr(rc), _ptr(cs), _ptr(angle),
                                     _ptr(valid), _ptr(scratch), _stream()), "ccvpe_pose_decode")
+
+
+#: the hypothesis counts and disc radii (pixels) `pose_hypotheses` accepts
+HYPOTHESES_K = (1, 64)
+HYPOTHESES_RADIUS = (0, 32767)
+
+
+def pose_hypotheses(heatmap: torch.Tensor, ori: torch.Tensor, k: int, radius: int, idx, rc, value, mass, cs, angle,
+                    valid, count):
+    """The k strongest mutually exclusive modes of each heatmap (include/ccvpe_b200.h, ccvpe_pose_hypotheses), in one
+    launch.  heatmap fp32 [B, 1, H, W], ori fp32 [B, 2, H, W]; outputs idx int64 [B, k], rc int32 [B, k, 2], value and
+    mass fp32 [B, k], cs fp32 [B, k, 2], angle float64 [B, k], valid uint8 [B, k], count int32 [B].  All contiguous, on the
+    current device; every argument is checked before the launch."""
+    if not (_is_int(k) and HYPOTHESES_K[0] <= k <= HYPOTHESES_K[1]):
+        raise CcvpeError("pose_hypotheses: k must be an int in [%d, %d], got %r" % (*HYPOTHESES_K, k))
+    if not (_is_int(radius) and HYPOTHESES_RADIUS[0] <= radius <= HYPOTHESES_RADIUS[1]):
+        raise CcvpeError("pose_hypotheses: radius must be an int in [%d, %d] (pixels), got %r"
+                         % (*HYPOTHESES_RADIUS, radius))
+    _require_f32("heatmap", heatmap, (None, 1, None, None))
+    B, _, H, W = heatmap.shape
+    if min(B, H, W) <= 0 or B > 65535:
+        raise CcvpeError("pose_hypotheses: heatmap must be [B, 1, H, W] with 0 < B <= 65535 and H, W > 0, got %s"
+                         % (tuple(heatmap.shape),))
+    if load().ccvpe_pose_hypotheses_smem_bytes(H, W) < 0:
+        raise CcvpeError("pose_hypotheses: a %dx%d map does not fit the shared memory of one 8-CTA cluster (a band of "
+                         "ceil(H/8) + 2 rows per CTA)" % (H, W))
+    _require_f32("ori", ori, (B, 2, H, W))
+    for name, t, dt, shape in (("idx", idx, torch.int64, (B, k)), ("rc", rc, torch.int32, (B, k, 2)),
+                               ("value", value, torch.float32, (B, k)), ("mass", mass, torch.float32, (B, k)),
+                               ("cs", cs, torch.float32, (B, k, 2)), ("angle", angle, torch.float64, (B, k)),
+                               ("valid", valid, torch.uint8, (B, k)), ("count", count, torch.int32, (B,))):
+        if not isinstance(t, torch.Tensor) or t.dtype != dt or tuple(t.shape) != shape or not t.is_contiguous():
+            raise CcvpeError("pose_hypotheses: %s must be a contiguous %s tensor of shape %s, got %s %s"
+                             % (name, dt, shape, getattr(t, "dtype", type(t).__name__), tuple(getattr(t, "shape", ()))))
+    tensors = (heatmap, ori, idx, rc, value, mass, cs, angle, valid, count)
+    for name, t in zip(("heatmap", "ori", "idx", "rc", "value", "mass", "cs", "angle", "valid", "count"), tensors):
+        if t.data_ptr() % t.element_size():
+            raise CcvpeError("pose_hypotheses: %s is misaligned for its dtype" % name)
+    _require_cuda(*tensors)
+    _check(load().ccvpe_pose_hypotheses(_ptr(heatmap), _ptr(ori), B, H, W, k, radius, _ptr(idx), _ptr(rc), _ptr(value),
+                                        _ptr(mass), _ptr(cs), _ptr(angle), _ptr(valid), _ptr(count), _stream()),
+           "ccvpe_pose_hypotheses")
 
 
 def _check_se_sum(chan_sum: Optional[torch.Tensor]):

@@ -125,6 +125,27 @@ __device__ __forceinline__ uint64_t ffma2(uint64_t a, uint64_t b, uint64_t c) {
   return d;
 }
 
+// a13's orientation rule at a decoded pixel (reference train_VIGOR.py:290-326), evaluated in float64: valid when
+// |cos| <= 1 && |sin| <= 1, then degrees(acos(cos)), or for sin < 0 Python's `degrees(-acos(cos)) % 360`; NaN when not
+// valid.  pose_finish_kernel and pose_hypotheses_kernel both call it, so a single hypothesis equals decode_pose bit for bit.
+__device__ __forceinline__ double pose_angle_deg(float c, float s, bool& ok) {
+  ok = fabsf(c) <= 1.f && fabsf(s) <= 1.f;
+  double a = __longlong_as_double(0x7ff8000000000000LL);
+  if (ok) {
+    const double rad2deg = 180.0 / 3.141592653589793238462643383279502884;
+    double ac = acos((double)c);
+    if (s < 0.f) {
+      double r = fmod(-ac * rad2deg, 360.0);  // python's float % : result takes the sign of the divisor
+      if (r < 0.0) r += 360.0;
+      if (r == 0.0) r = 0.0;
+      a = r;
+    } else {
+      a = ac * rad2deg;
+    }
+  }
+  return a;
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

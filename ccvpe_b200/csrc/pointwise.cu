@@ -294,22 +294,9 @@ __global__ void pose_finish_kernel(const ArgPartial* __restrict__ partial, int s
   float c = ori[((int64_t)b * 2 + 0) * n + vi], s = ori[((int64_t)b * 2 + 1) * n + vi];
   cs[2 * b + 0] = c;
   cs[2 * b + 1] = s;
-  bool ok = fabsf(c) <= 1.f && fabsf(s) <= 1.f;
+  bool ok;
+  angle[b] = pose_angle_deg(c, s, ok);
   valid[b] = ok ? 1 : 0;
-  double a = __longlong_as_double(0x7ff8000000000000LL);
-  if (ok) {
-    const double rad2deg = 180.0 / 3.141592653589793238462643383279502884;
-    double ac = acos((double)c);
-    if (s < 0.f) {
-      double r = fmod(-ac * rad2deg, 360.0);  // python's float % : result takes the sign of the divisor
-      if (r < 0.0) r += 360.0;
-      if (r == 0.0) r = 0.0;
-      a = r;
-    } else {
-      a = ac * rad2deg;
-    }
-  }
-  angle[b] = a;
 }
 
 }  // namespace ccvpe

@@ -419,3 +419,34 @@ def decode_pose(heatmap: torch.Tensor, ori: torch.Tensor) -> Dict[str, torch.Ten
     with cabi.device_of(heatmap):
         cabi.pose_decode(heatmap, ori, out["idx"], out["rc"], out["cs"], out["angle"], out["valid"], scratch)
     return out
+
+
+@torch.no_grad()
+def decode_hypotheses(heatmap: torch.Tensor, ori: torch.Tensor, k: int, radius: int) -> Dict[str, torch.Tensor]:
+    """The k strongest mutually exclusive location modes of each heatmap, in one launch (include/ccvpe_b200.h,
+    ccvpe_pose_hypotheses).  A mode is a pixel >= its 8 neighbours; modes are taken highest first (ties: smaller flat
+    index), each one claims the disc of `radius` pixels around it, and a mode inside an earlier disc is skipped.
+
+    heatmap [B,1,H,W] fp32, ori [B,2,H,W] fp32 (CUDA).  Returns CUDA tensors: decode_pose's keys per hypothesis -- idx
+    int64[B,k], rc int32[B,k,2], cs float32[B,k,2], angle float64[B,k], valid uint8[B,k] -- plus value float32[B,k] (the
+    heatmap at the mode), mass float32[B,k] (the heatmap summed over the part of its disc no earlier hypothesis claimed;
+    mass[:, 0] is a confidence) and count int32[B].  Slots t >= count[b] hold idx -1 and NaN.  A heatmap holding a NaN
+    has count 0.  With k = 1, idx / rc / cs / angle / valid equal decode_pose's on every NaN-free map."""
+    if not heatmap.is_cuda:
+        raise cabi.CcvpeError("decode_hypotheses needs CUDA tensors; there is no CPU fallback")
+    heatmap = heatmap.contiguous().float()
+    ori = ori.contiguous().float()
+    B = heatmap.shape[0]
+    dev = heatmap.device
+    out = dict(idx=torch.empty((B, k), dtype=torch.int64, device=dev),
+               rc=torch.empty((B, k, 2), dtype=torch.int32, device=dev),
+               cs=torch.empty((B, k, 2), dtype=torch.float32, device=dev),
+               angle=torch.empty((B, k), dtype=torch.float64, device=dev),
+               valid=torch.empty((B, k), dtype=torch.uint8, device=dev),
+               value=torch.empty((B, k), dtype=torch.float32, device=dev),
+               mass=torch.empty((B, k), dtype=torch.float32, device=dev),
+               count=torch.empty(B, dtype=torch.int32, device=dev))
+    with cabi.device_of(heatmap):
+        cabi.pose_hypotheses(heatmap, ori, k, radius, out["idx"], out["rc"], out["value"], out["mass"], out["cs"],
+                             out["angle"], out["valid"], out["count"])
+    return out

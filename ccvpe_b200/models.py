@@ -9,6 +9,8 @@ called, and there is no PyTorch fallback for the decoder.
 Extras over the reference (all optional, defaults reproduce the reference's fp32 behaviour):
   * `set_precision("bf16")`  -- encoders in bf16 channels-last, decoder kernels on tcgen05 tensor cores;
   * `decode_pose(heatmap, ori)` -- the scripts' NumPy argmax/orientation decode as a CUDA kernel;
+  * `decode_hypotheses(heatmap, ori, k, radius)` -- the k strongest heatmap modes with their probability mass and
+    orientation (confidence, alternative locations);
   * `localize(grd, sat)`     -- forward + decode in one call, returns only the small pose tensors;
   * `resize_u8(img, size)`   -- the reference's bilinear `transforms.Resize` of native-size uint8 images, on the device;
   * `affine_u8(img, matrices, size)`, `rotate_u8(img, angles)` -- Pillow's bilinear affine transform / rotation (+ crop) of
@@ -25,7 +27,7 @@ import torch
 from torch import nn
 
 from . import cabi
-from .decoder import Fork, PostEncoderPipeline, decode_pose
+from .decoder import Fork, PostEncoderPipeline, decode_hypotheses, decode_pose
 from .efficientnet import EfficientNetB0
 from .fast_encoder import FastEncoder
 from .specs import KITTI, OXFORD, SKIP_BLOCKS, SKIP_CHANNELS, VIGOR, VariantSpec
@@ -306,6 +308,10 @@ class _CVMBase(nn.Module):
     @staticmethod
     def decode_pose(heatmap, ori):
         return decode_pose(heatmap, ori)
+
+    @staticmethod
+    def decode_hypotheses(heatmap, ori, k, radius):
+        return decode_hypotheses(heatmap, ori, k, radius)
 
     @torch.no_grad()
     def localize(self, grd, sat):

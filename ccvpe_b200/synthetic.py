@@ -104,3 +104,22 @@ def synthetic_ground_truth(batch: int, seed: int = 0, size: int = 512, n_bins: i
     gt_with_ori = gt * bin_weights[:, :, None, None]
     gt_orientation = ori_vec[:, :, None, None].expand(batch, 2, size, size).contiguous()
     return gt, gt_with_ori, gt_orientation
+
+
+def synthetic_mixture(batch: int, n_modes: int, H: int = 512, W: int = 512, seed: int = 0):
+    """Multi-modal heatmaps, fp32 [B, 1, H, W] CPU, each summing to 1 like a softmax output: a mixture of `n_modes`
+    isotropic Gaussians with random centres (anywhere in the map, edges included), widths sigma in [2, 12) and weights.
+    The peaks are the planted location modes; the tails between them add many shallow ones."""
+    g = torch.Generator().manual_seed(30_000 + seed)
+    ys = torch.arange(H, dtype=torch.float64).view(H, 1)
+    xs = torch.arange(W, dtype=torch.float64).view(1, W)
+    out = torch.zeros(batch, 1, H, W)
+    for b in range(batch):
+        m = torch.zeros(H, W, dtype=torch.float64)
+        for _ in range(n_modes):
+            cy, cx = float(torch.rand(1, generator=g)) * (H - 1), float(torch.rand(1, generator=g)) * (W - 1)
+            sigma = 2.0 + 10.0 * float(torch.rand(1, generator=g))
+            w = 0.2 + float(torch.rand(1, generator=g))
+            m += w * torch.exp(-(ys - cy) ** 2 / (2 * sigma ** 2)) * torch.exp(-(xs - cx) ** 2 / (2 * sigma ** 2))
+        out[b, 0] = (m / m.sum()).float()
+    return out

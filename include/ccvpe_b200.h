@@ -159,6 +159,32 @@ int ccvpe_pose_decode(const float* heatmap, const float* ori, int B, int H, int 
                       int64_t* idx, int32_t* rc, float* cs, double* angle_deg, uint8_t* valid,
                       void* scratch, void* stream);
 
+/* a13  pose hypotheses -- the k strongest mutually exclusive location modes of each heatmap, in one launch.
+ * heatmap fp32 [B, H*W]; ori fp32 planar [B, 2, H*W]; 1 <= k <= 64; 0 <= radius <= 32767.  For each pair:
+ *   candidates: the pixels whose value is >= every in-bounds 8-neighbour (fixed from the original map), ordered by value,
+ *     highest first, ties to the smaller flat index i*W + j (NumPy's first occurrence; -0 and +0 are equal values);
+ *   greedy claim: the first candidate not yet claimed becomes the next hypothesis and claims every pixel of its disc
+ *     (i - i0)^2 + (j - j0)^2 <= radius^2 (integer arithmetic); stop after k hypotheses or when the candidates run out.
+ * Hypothesis t < count[b], at slot [b, t]:
+ *   idx = i0*W + j0;  rc = (i0, j0);  value = heatmap[b, idx];
+ *   mass = the sum of the heatmap over the pixels of its disc that no earlier hypothesis claimed, accumulated in float64
+ *     in a fixed order and rounded once to float32 (the masses partition the claimed probability: their sum is <= 1 for a
+ *     softmax heatmap);
+ *   cs, angle_deg, valid: ccvpe_pose_decode's rule at idx.
+ * Slots t >= count[b]: idx = -1, rc = (-1, -1), value = mass = cs = angle_deg = NaN, valid = 0.
+ * A heatmap holding any NaN has no neighbourhood order: count = 0.  +-inf compare as ordinary values (an all -inf map
+ * gives idx 0, as ccvpe_pose_decode).  With k = 1 idx, rc, cs, angle_deg and valid equal ccvpe_pose_decode's on every
+ * NaN-free map (its first-occurrence maximum is always a mode).
+ * Outputs: idx [B, k], rc [B, k, 2], value / mass [B, k], cs [B, k, 2], angle_deg [B, k], valid [B, k], count [B], each
+ * naturally aligned.  One 8-CTA cluster per pair holds the map in shared memory, a band of ceil(H/8) rows (+ 2 halo rows)
+ * per CTA: ccvpe_pose_hypotheses_smem_bytes(H, W) is that per-CTA need, or -1 where it does not fit (a 512x512 map needs
+ * 143 376 bytes); such maps, like every other bad argument, are refused with CCVPE_ERR_BAD_ARGUMENT before any launch.
+ * Reads the heatmap once; no workspace, no allocation, no synchronisation; deterministic; graph-capturable. */
+int64_t ccvpe_pose_hypotheses_smem_bytes(int H, int W);
+int ccvpe_pose_hypotheses(const float* heatmap, const float* ori, int B, int H, int W, int k, int radius,
+                          int64_t* idx, int32_t* rc, float* value, float* mass, float* cs, double* angle_deg,
+                          uint8_t* valid, int32_t* count, void* stream);
+
 /* ---------------------------------------------------------------------------------------------------------------
  * Encoder glue (SURVEY section 8(f)-2, first step; the encoders themselves stay cuDNN/cuBLAS through PyTorch):
  *   y[b,h,w,c] = SiLU(x[b,h,w,c] + bias[c]);   chan_sum[b,c] += sum_{h,w} y[b,h,w,c]   (optional, caller zeroes it)
