@@ -34,7 +34,7 @@ EXPORTED_SYMBOLS = (
     "ccvpe_match_bwd_scratch_elems", "ccvpe_match_level_bwd", "ccvpe_loss_workspace_elems", "ccvpe_infonce_loss",
     "ccvpe_cross_entropy_loss", "ccvpe_orientation_loss", "ccvpe_grd_descriptors_bwd",
     "ccvpe_gt_pyramid", "ccvpe_infonce_loss_binned", "ccvpe_orientation_loss_const", "ccvpe_pose_labels",
-    "ccvpe_pose_hypotheses_smem_bytes", "ccvpe_pose_hypotheses",
+    "ccvpe_pose_hypotheses_smem_bytes", "ccvpe_pose_hypotheses", "ccvpe_track_scratch_bytes", "ccvpe_track_step",
 )
 
 
@@ -135,6 +135,10 @@ def load() -> C.CDLL:
     lib.ccvpe_pose_hypotheses_smem_bytes.argtypes = [C.c_int, C.c_int]
     lib.ccvpe_pose_hypotheses.restype = C.c_int
     lib.ccvpe_pose_hypotheses.argtypes = [C.c_void_p, C.c_void_p] + [C.c_int] * 5 + [C.c_void_p] * 9
+    lib.ccvpe_track_scratch_bytes.restype = C.c_int64
+    lib.ccvpe_track_scratch_bytes.argtypes = [C.c_int, C.c_int, C.c_int]
+    lib.ccvpe_track_step.restype = C.c_int
+    lib.ccvpe_track_step.argtypes = [C.c_void_p] * 3 + [C.c_int] * 3 + [C.c_float] * 2 + [C.c_void_p] * 4
     lib.ccvpe_bias_silu_nhwc.restype = C.c_int
     lib.ccvpe_bias_silu_nhwc.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64,
                                          C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
@@ -443,6 +447,53 @@ def pose_hypotheses(heatmap: torch.Tensor, ori: torch.Tensor, k: int, radius: in
     _check(load().ccvpe_pose_hypotheses(_ptr(heatmap), _ptr(ori), B, H, W, k, radius, _ptr(idx), _ptr(rc), _ptr(value),
                                         _ptr(mass), _ptr(cs), _ptr(angle), _ptr(valid), _ptr(count), _stream()),
            "ccvpe_pose_hypotheses")
+
+
+#: the process-noise widths (pixels) and uniform-mix weights `track_step` accepts, and its largest map side
+TRACK_SIGMA = (0.0, 32.0)
+TRACK_EPSILON = (0.0, 1.0)
+TRACK_MAX_DIM = 4096
+
+
+def track_scratch_bytes(B: int, H: int, W: int) -> int:
+    return int(load().ccvpe_track_scratch_bytes(B, H, W))
+
+
+def track_step(belief: torch.Tensor, heatmap: torch.Tensor, motion: torch.Tensor, sigma: float, epsilon: float,
+               evidence: torch.Tensor, reset: torch.Tensor, scratch: torch.Tensor):
+    """One step of the sequential location filter (include/ccvpe_b200.h, ccvpe_track_step), updating `belief` in place.
+    belief and heatmap fp32 [B, 1, H, W] (heatmap's storage must not overlap belief's), motion float64 [B, 6] (read when
+    the kernels run), evidence float64 [B], reset uint8 [B], scratch uint8 [>= track_scratch_bytes(B, H, W)].  All
+    contiguous, on the current device; sigma in TRACK_SIGMA pixels, epsilon in TRACK_EPSILON; every argument is checked
+    before the launch."""
+    for name, v, (lo, hi) in (("sigma", sigma, TRACK_SIGMA), ("epsilon", epsilon, TRACK_EPSILON)):
+        if not (isinstance(v, numbers.Real) and not isinstance(v, bool) and lo <= v <= hi):
+            raise CcvpeError("track_step: %s must be a number in [%g, %g], got %r" % (name, lo, hi, v))
+    _require_f32("belief", belief, (None, 1, None, None))
+    B, _, H, W = belief.shape
+    if not (1 <= B <= 65535 and 1 <= H <= TRACK_MAX_DIM and 1 <= W <= TRACK_MAX_DIM):
+        raise CcvpeError("track_step: belief must be [B, 1, H, W] with 1 <= B <= 65535 and 1 <= H, W <= %d, got %s"
+                         % (TRACK_MAX_DIM, tuple(belief.shape)))
+    _require_f32("heatmap", heatmap, (B, 1, H, W))
+    for name, t, dt, shape in (("motion", motion, torch.float64, (B, 6)), ("evidence", evidence, torch.float64, (B,)),
+                               ("reset", reset, torch.uint8, (B,))):
+        if not isinstance(t, torch.Tensor) or t.dtype != dt or tuple(t.shape) != shape or not t.is_contiguous():
+            raise CcvpeError("track_step: %s must be a contiguous %s tensor of shape %s, got %s %s"
+                             % (name, dt, shape, getattr(t, "dtype", type(t).__name__), tuple(getattr(t, "shape", ()))))
+    need = track_scratch_bytes(B, H, W)
+    if not isinstance(scratch, torch.Tensor) or scratch.dtype != torch.uint8 or scratch.dim() != 1 \
+            or not scratch.is_contiguous() or scratch.numel() < need:
+        raise CcvpeError("track_step: scratch must be a contiguous uint8 tensor of at least %d bytes" % need)
+    tensors = (belief, heatmap, motion, evidence, reset, scratch)
+    for name, t, align in zip(("belief", "heatmap", "motion", "evidence", "reset", "scratch"), tensors, (4, 4, 8, 8, 1, 8)):
+        if t.data_ptr() % align:
+            raise CcvpeError("track_step: %s is misaligned (needs %d bytes)" % (name, align))
+    b0, h0, nbytes = belief.data_ptr(), heatmap.data_ptr(), belief.numel() * 4
+    if b0 < h0 + nbytes and h0 < b0 + nbytes:
+        raise CcvpeError("track_step: heatmap overlaps belief; the step writes belief while it reads heatmap")
+    _require_cuda(*tensors)
+    _check(load().ccvpe_track_step(_ptr(belief), _ptr(heatmap), _ptr(motion), B, H, W, float(sigma), float(epsilon),
+                                   _ptr(evidence), _ptr(reset), _ptr(scratch), _stream()), "ccvpe_track_step")
 
 
 def _check_se_sum(chan_sum: Optional[torch.Tensor]):

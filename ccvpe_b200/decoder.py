@@ -450,3 +450,27 @@ def decode_hypotheses(heatmap: torch.Tensor, ori: torch.Tensor, k: int, radius: 
         cabi.pose_hypotheses(heatmap, ori, k, radius, out["idx"], out["rc"], out["value"], out["mass"], out["cs"],
                              out["angle"], out["valid"], out["count"])
     return out
+
+
+@torch.no_grad()
+def track_step(belief: torch.Tensor, heatmap: torch.Tensor, motion: torch.Tensor, sigma: float,
+               epsilon: float = 0.0) -> Dict[str, torch.Tensor]:
+    """One step of the sequential location filter (include/ccvpe_b200.h, ccvpe_track_step): warps `belief` by `motion`,
+    blurs it with a Gaussian of `sigma` pixels, mixes in `epsilon` of the uniform distribution, multiplies by this frame's
+    heatmap and renormalises, updating `belief` in place.
+
+    belief fp32 [B,1,H,W] contiguous (CUDA; start a track with a copy of the first heatmap), heatmap [B,1,H,W] fp32,
+    motion float64 [B,6] on the device: the affine data (`models.track_motion`) mapping a pixel centre of this frame's
+    crop to a coordinate of the previous frame's.  Returns CUDA tensors evidence float64[B] (the sum Z of prior * heatmap:
+    the predictive likelihood of the frame) and reset uint8[B] (1 where Z was not a positive finite number and the belief
+    restarted as a copy of the heatmap).  Decode the belief with decode_pose / decode_hypotheses."""
+    if not belief.is_cuda:
+        raise cabi.CcvpeError("track_step needs CUDA tensors; there is no CPU fallback")
+    heatmap = heatmap.contiguous().float()
+    B, _, H, W = belief.shape
+    dev = belief.device
+    out = dict(evidence=torch.empty(B, dtype=torch.float64, device=dev), reset=torch.empty(B, dtype=torch.uint8, device=dev))
+    scratch = torch.empty(max(cabi.track_scratch_bytes(B, H, W), 0), dtype=torch.uint8, device=dev)
+    with cabi.device_of(belief):
+        cabi.track_step(belief, heatmap, motion, sigma, epsilon, out["evidence"], out["reset"], scratch)
+    return out

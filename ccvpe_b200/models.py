@@ -11,6 +11,8 @@ Extras over the reference (all optional, defaults reproduce the reference's fp32
   * `decode_pose(heatmap, ori)` -- the scripts' NumPy argmax/orientation decode as a CUDA kernel;
   * `decode_hypotheses(heatmap, ori, k, radius)` -- the k strongest heatmap modes with their probability mass and
     orientation (confidence, alternative locations);
+  * `track_step(belief, heatmap, motion, sigma, epsilon)` -- fuses each frame's heatmap with the motion-propagated
+    location belief of the previous frame (a recursive Bayes filter over the crop's pixels; `track_motion` builds motion);
   * `localize(grd, sat)`     -- forward + decode in one call, returns only the small pose tensors;
   * `resize_u8(img, size)`   -- the reference's bilinear `transforms.Resize` of native-size uint8 images, on the device;
   * `affine_u8(img, matrices, size)`, `rotate_u8(img, angles)` -- Pillow's bilinear affine transform / rotation (+ crop) of
@@ -27,7 +29,7 @@ import torch
 from torch import nn
 
 from . import cabi
-from .decoder import Fork, PostEncoderPipeline, decode_hypotheses, decode_pose
+from .decoder import Fork, PostEncoderPipeline, decode_hypotheses, decode_pose, track_step
 from .efficientnet import EfficientNetB0
 from .fast_encoder import FastEncoder
 from .specs import KITTI, OXFORD, SKIP_BLOCKS, SKIP_CHANNELS, VIGOR, VariantSpec
@@ -58,6 +60,25 @@ def rotate_matrix(angle, size, center=None, translate=None):
     m[2] += center[0]
     m[5] += center[1]
     return [float(v) for v in m]
+
+
+def track_motion(prev_crop, new_crop, shift=(0.0, 0.0)):
+    """The motion matrix of `track_step` for one track, as a list of 6 floats in the AFFINE data convention:
+    M(q) = A_prev^-1(A_new(q) - shift), which maps a pixel-centre coordinate q of the new crop to the coordinate of the
+    previous crop where the same vehicle position was.  prev_crop / new_crop: the affine data (6 numbers) with which each
+    frame's aerial crop was cut from the map (for a translation-only crop at (left, top), `[1, 0, left, 0, 1, top]`; for a
+    rotated crop, `rotate_matrix(...)`).  shift = (dx, dy): the vehicle's displacement in map pixels since the previous
+    frame.  Python float arithmetic; a translation-only pair gives an exact result."""
+    p0, p1, p2, p3, p4, p5 = [float(v) for v in prev_crop]
+    n0, n1, n2, n3, n4, n5 = [float(v) for v in new_crop]
+    sx, sy = [float(v) for v in shift]
+    det = p0 * p4 - p1 * p3
+    if det == 0.0 or not math.isfinite(det):
+        raise ValueError("track_motion: prev_crop is not invertible (det %r)" % det)
+    i0, i1, i3, i4 = p4 / det, -p1 / det, -p3 / det, p0 / det     # the inverse of prev_crop's linear part
+    tx, ty = (n2 - sx) - p2, (n5 - sy) - p5
+    return [i0 * n0 + i1 * n3, i0 * n1 + i1 * n4, i0 * tx + i1 * ty,
+            i3 * n0 + i4 * n3, i3 * n1 + i4 * n4, i3 * tx + i4 * ty]
 
 
 class _Permute(nn.Module):
@@ -312,6 +333,10 @@ class _CVMBase(nn.Module):
     @staticmethod
     def decode_hypotheses(heatmap, ori, k, radius):
         return decode_hypotheses(heatmap, ori, k, radius)
+
+    @staticmethod
+    def track_step(belief, heatmap, motion, sigma, epsilon=0.0):
+        return track_step(belief, heatmap, motion, sigma, epsilon)
 
     @torch.no_grad()
     def localize(self, grd, sat):

@@ -9,6 +9,7 @@ which makes end-to-end argmax comparisons meaningless -- SURVEY.md section 7.3-4
 """
 from __future__ import annotations
 
+import math
 import zlib
 from typing import Dict
 
@@ -123,3 +124,61 @@ def synthetic_mixture(batch: int, n_modes: int, H: int = 512, W: int = 512, seed
             m += w * torch.exp(-(ys - cy) ** 2 / (2 * sigma ** 2)) * torch.exp(-(xs - cx) ** 2 / (2 * sigma ** 2))
         out[b, 0] = (m / m.sum()).float()
     return out
+
+
+def synthetic_track(n_frames: int, batch: int = 1, H: int = 512, W: int = 512, seed: int = 0, sigma: float = 4.0):
+    """A seeded sequence of heatmaps along a known trajectory, for the sequential location filter (`track_step`).
+
+    Each of `batch` vehicles drives through a map at 3-6 map pixels per frame with a slowly turning heading.  Every frame's
+    aerial crop is cut at an integer offset that puts the vehicle within 40 pixels of the crop's centre (a noisy position
+    prior), with the translation-only crop data [1, 0, left, 0, 1, top].  The heatmap holds two isotropic Gaussians of
+    width `sigma`: the true mode at the vehicle's position (peak 1) and a distractor at a random place at least
+    min(100, max(H, W) / 4) pixels away (peak 1.5 on frames where it is stronger, about one in three from frame 1 on,
+    else 0.5), plus a floor of 1e-6, normalised to sum 1.
+
+    Returns a dict of CPU tensors: heatmap fp32 [T, B, 1, H, W]; motion float64 [T, B, 6], the true motion of each frame
+    from the previous one (`models.track_motion`; frame 0: identity); truth float64 [T, B, 2] and distractor float64
+    [T, B, 2], the (row, col) of both modes in crop pixels; strong bool [T, B], where the distractor has the higher peak."""
+    from .models import track_motion
+
+    rng = torch.Generator().manual_seed(40_000 + seed)
+    rand = lambda: float(torch.rand(1, generator=rng))
+    ys = torch.arange(H, dtype=torch.float64).view(H, 1)
+    xs = torch.arange(W, dtype=torch.float64).view(1, W)
+    heat = torch.empty(n_frames, batch, 1, H, W)
+    motion = torch.zeros(n_frames, batch, 6, dtype=torch.float64)
+    truth = torch.empty(n_frames, batch, 2, dtype=torch.float64)
+    distractor = torch.empty(n_frames, batch, 2, dtype=torch.float64)
+    strong = torch.zeros(n_frames, batch, dtype=torch.bool)
+
+    def bump(cy, cx):
+        return torch.exp(-((ys - cy) ** 2 + (xs - cx) ** 2) / (2 * sigma ** 2))
+
+    far = min(100.0, max(H, W) / 4)                          # reachable from any vehicle position
+    for b in range(batch):
+        pos = [10_000.0 * rand(), 10_000.0 * rand()]              # (x, y) in map pixels
+        heading = 2 * math.pi * rand()
+        prev_crop = None
+        for t in range(n_frames):
+            if t:
+                heading += 0.2 * (rand() - 0.5)
+                speed = 3.0 + 3.0 * rand()
+                step = (speed * math.cos(heading), speed * math.sin(heading))
+                pos = [pos[0] + step[0], pos[1] + step[1]]
+            left = math.floor(pos[0] - W / 2 + 80 * (rand() - 0.5))
+            top = math.floor(pos[1] - H / 2 + 80 * (rand() - 0.5))
+            crop = [1.0, 0.0, float(left), 0.0, 1.0, float(top)]
+            motion[t, b] = torch.tensor(track_motion(prev_crop, crop, step) if t else [1.0, 0.0, 0.0, 0.0, 1.0, 0.0],
+                                        dtype=torch.float64)
+            prev_crop = crop
+            cy, cx = pos[1] - top, pos[0] - left
+            while True:
+                dy, dx = rand() * (H - 1), rand() * (W - 1)
+                if (dy - cy) ** 2 + (dx - cx) ** 2 >= far ** 2:
+                    break
+            strong[t, b] = t > 0 and rand() < 1 / 3
+            m = bump(cy, cx) + (1.5 if strong[t, b] else 0.5) * bump(dy, dx) + 1e-6
+            heat[t, b, 0] = (m / m.sum()).float()
+            truth[t, b] = torch.tensor([cy, cx], dtype=torch.float64)
+            distractor[t, b] = torch.tensor([dy, dx], dtype=torch.float64)
+    return dict(heatmap=heat, motion=motion, truth=truth, distractor=distractor, strong=strong)

@@ -185,6 +185,34 @@ int ccvpe_pose_hypotheses(const float* heatmap, const float* ori, int B, int H, 
                           int64_t* idx, int32_t* rc, float* value, float* mass, float* cs, double* angle_deg,
                           uint8_t* valid, int32_t* count, void* stream);
 
+/* Sequential location filter -- one Bayes-filter step per frame, fusing each heatmap with the motion-propagated belief of
+ * the previous frame.  belief fp32 [B, H*W] (updated in place: one location distribution per track, on the pixel grid of
+ * the track's current aerial crop); heatmap fp32 [B, H*W] (this frame's model output, must not overlap belief); motion
+ * float64 [B, 6] on the device, read when the kernels run (a captured step replays with whatever it then holds);
+ * 0 <= sigma <= 32 (pixels); 0 <= epsilon <= 1; 1 <= B <= 65535; 1 <= H, W <= 4096.  Per track:
+ *   1. predict: motion a[0..5] maps a pixel centre of the new grid to a coordinate of the previous one (the convention of
+ *      ccvpe_affine_u8 / Pillow's AFFINE data).  For new pixel (i, j), in float64 with every operation rounded:
+ *        u = ((a0*(j+0.5) + a1*(i+0.5)) + a2) - 0.5,   v = ((a3*(j+0.5) + a4*(i+0.5)) + a5) - 0.5;
+ *      p = |a0*a4 - a1*a3| * bilinear(old belief at (v, u)) with the weights of (u - floor u, v - floor v), each tap outside
+ *      the grid contributing 0 (zero padding: probability leaving the crop is lost); a coordinate whose 4 taps all lie
+ *      outside (NaN, inf or huge ones included) gives p = 0;
+ *   2. process noise: p convolved with the separable Gaussian w_d ~ exp(-d^2 / (2 sigma^2)), |d| <= r = ceil(3 sigma),
+ *      normalised to sum 1 (float64, rounded to float32), zero padded; rows first, then columns; sigma = 0 is the identity;
+ *   3. mix: prior = (1 - epsilon) * p + epsilon / (H*W)   (float64, no renormalisation first);
+ *   4. update: q = prior * heatmap (float64), Z = sum q in float64 in a fixed order; evidence[b] = Z.
+ *      Z > 0 and finite: belief = q / Z (q rounded to float32 first), reset[b] = 0;
+ *      otherwise (disjoint supports with epsilon = 0, a NaN or inf in the heatmap, a NaN belief): belief = a bitwise copy
+ *      of the heatmap, reset[b] = 1.
+ * Each blur output is w_0 s_j + sum_{d=1..r} w_d (s_{j-d} + s_{j+d}), accumulated in float32 in that order.  Where q is
+ * below float32's normal range, its rounding is absolute (2^-150 / Z in the belief).  Values of prior * heatmap beyond float32's
+ * range are not supported.  scratch: >= ccvpe_track_scratch_bytes(B, H, W) bytes (-1 for a refused shape), 8-byte
+ * aligned.  belief and heatmap 4-byte, motion and evidence 8-byte aligned.  Every bad argument is refused with
+ * CCVPE_ERR_BAD_ARGUMENT before any launch.  Three launches, no allocation, no host synchronisation or copy;
+ * deterministic; graph-capturable. */
+int64_t ccvpe_track_scratch_bytes(int B, int H, int W);
+int ccvpe_track_step(float* belief, const float* heatmap, const double* motion, int B, int H, int W, float sigma,
+                     float epsilon, double* evidence, uint8_t* reset, void* scratch, void* stream);
+
 /* ---------------------------------------------------------------------------------------------------------------
  * Encoder glue (SURVEY section 8(f)-2, first step; the encoders themselves stay cuDNN/cuBLAS through PyTorch):
  *   y[b,h,w,c] = SiLU(x[b,h,w,c] + bias[c]);   chan_sum[b,c] += sum_{h,w} y[b,h,w,c]   (optional, caller zeroes it)
